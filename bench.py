@@ -69,7 +69,12 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-eager-baseline", action="store_true")
     ap.add_argument("--no-strong", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned to DIR/<name>.npy (float32), to compare two builds")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def measured_peaks():
@@ -118,6 +123,22 @@ class ClockSampler:
         busy = [s for s, p in zip(sm, pw) if p > 300] or sm
         return {"sm_mhz": float(np.median(busy)) if busy else None, "sm_max_mhz": max(mx) if mx else None,
                 "power_w_max": max(pw) if pw else None, "samples": len(sm), "reasons": sorted(reasons)}
+
+
+DUMP_MAX_BYTES = 60 * 10**6     # array data; with the .npy headers a dump stays under 64 MB
+
+
+def dump_outputs(d: Path, arrays: dict) -> None:
+    """Writes every tensor of `arrays` to d/<name>.npy as float32. Above DUMP_MAX_BYTES in all, each array keeps the same
+    fraction of its rows, drawn with a fixed seed and kept in order, so runs with the same arguments stay comparable."""
+    d.mkdir(parents=True, exist_ok=True)
+    total = sum(a.numel() * 4 for a in arrays.values())
+    frac = min(1.0, DUMP_MAX_BYTES / max(total, 1))
+    for name, a in arrays.items():
+        a = a.detach().float().cpu().numpy()
+        if frac < 1.0:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], int(a.shape[0] * frac), replace=False))]
+        np.save(d / f"{name}.npy", a)
 
 
 def episode_offsets(n_episodes: int, seed: int) -> np.ndarray:
@@ -383,19 +404,22 @@ def main():
     rows = [int(episode_offsets(args.episodes, seed=1 + r)[-1]) for r in range(world)]
 
     def step_device():
-        r, g, rs, gs = eng.label(ob, off, F)
+        """(reward, rtg, reward_stacked, rtg_stacked) of this rank, then with N>1 the gathered [rows, 2] (None off rank 0)"""
+        out = eng.label(ob, off, F)
         if world > 1:
-            gather_rows(torch.stack([r, g], dim=1), rows, dst=0)      # the path's only collective
-        return r
+            return (*out, gather_rows(torch.stack(out[:2], dim=1), rows, dst=0))      # the path's only collective
+        return out
 
     def timed(fn, k):
+        """(milliseconds for k calls of fn, what the last call returned)"""
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(k):
-            fn()
+            last = None                 # free the previous step's outputs before the next step, as if they were not kept
+            last = fn()
         e1.record()
         torch.cuda.synchronize()
         if world > 1:
@@ -403,7 +427,7 @@ def main():
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms)
+        return float(ms), last
 
     for _ in range(args.warmup):
         step_device()
@@ -411,9 +435,15 @@ def main():
     if rank == 0:
         sampler.start()
     l0 = eng.launch_count
-    total_ms = timed(step_device, args.steps)
+    total_ms, last = timed(step_device, args.steps)
     launches = eng.launch_count - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        arrays = dict(zip(("reward", "rtg", "reward_stacked", "rtg_stacked"), last))
+        if world > 1:
+            arrays.update(reward_all_ranks=last[4][:, 0], rtg_all_ranks=last[4][:, 1])
+        dump_outputs(Path(args.dump_outputs), arrays)
+    del last
     ms_per_step = total_ms / args.steps
     total_frames = sum(rows)
     value = total_frames / (ms_per_step * 1e-3)
@@ -453,7 +483,7 @@ def main():
 
     # ---- end to end through the host-buffer entry point (C ABI), then through the drop-in itself ----
     e2e = entry = None
-    r_dev = step_device().cpu().numpy()
+    r_dev = step_device()[0].cpu().numpy()
     if not args.no_e2e:
         pinned = True
         try:

@@ -9,6 +9,7 @@ from __future__ import annotations
 
 import importlib
 import importlib.util
+import os
 import sys
 import types
 from pathlib import Path
@@ -67,7 +68,7 @@ def install(use_shims: bool = True):
 
 
 def reference_available() -> bool:
-    return (REFERENCE / "arp_dt" / "label_reward.py").exists()
+    return os.path.exists(REFERENCE / "arp_dt" / "label_reward.py")     # False, not an error, where it is unreadable
 
 
 def import_reference():

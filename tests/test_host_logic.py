@@ -68,6 +68,30 @@ def test_instruction_strings_equal_reference():
     from arp_dt.assets.procgen_instruct import PROCGEN_POS_NEG_INSTRUCT
     for k, v in instructions.POS_NEG.items():
         assert PROCGEN_POS_NEG_INSTRUCT[k] == v
+    # the stored table that test_instruction_strings_match_golden checks everywhere is the reference's too
+    import json
+    from oracle.make_golden_instructions import GOLDEN, reference_table
+    gold = json.loads(GOLDEN.read_text())
+    assert {k: gold[k] for k in ("clip_instruct", "clip_special_instruct", "pos_neg")} == reference_table()
+
+
+def test_instruction_strings_match_golden():
+    """Every lookup of tests/golden/instructions.json (oracle/make_golden_instructions.py): 7 envs x 7 instruction types,
+    the refusals included, and every positive / negative prompt list."""
+    import json
+    from oracle.make_golden_instructions import ENVS, GOLDEN, INSTS, RAISES
+    gold = json.loads(GOLDEN.read_text())
+    assert list(gold["clip_instruct"]) == list(ENVS) and list(gold["clip_special_instruct"]) == list(ENVS)
+    for env in ENVS:
+        assert instructions.get_clip_instruct(env) == gold["clip_instruct"][env], env
+        assert list(gold["clip_special_instruct"][env]) == list(INSTS)
+        for inst, want in gold["clip_special_instruct"][env].items():
+            if want == RAISES:
+                with pytest.raises(ValueError):
+                    instructions.get_clip_special_instruct(env, inst)
+            else:
+                assert instructions.get_clip_special_instruct(env, inst) == want, (env, inst)
+    assert instructions.POS_NEG == gold["pos_neg"]
 
 
 def test_model_type_dispatch():
