@@ -24,6 +24,8 @@ DT_F32, DT_BF16, DT_F16 = 0, 1, 2
 ACT_NONE, ACT_QUICKGELU, ACT_RELU = 0, 1, 2
 PREC_BF16, PREC_F32, PREC_F32RESID = 0, 1, 2   # PREC_BF16 = the 16-bit tensor-core path (name is historical)
 PREC_16BIT = PREC_BF16
+#: precision names of the Python entry points ("bf16" / "fp16" name the 16-bit path whatever the operand format)
+PRECISIONS = {"16bit": PREC_16BIT, "bf16": PREC_16BIT, "fp16": PREC_16BIT, "fp32resid": PREC_F32RESID, "fp32": PREC_F32}
 MAX_TEXT = 16
 
 #: every symbol include/arp_b200.h declares (tests check the library exports exactly these)
@@ -54,6 +56,13 @@ class ArpError(RuntimeError):
 
 
 _lib = None
+
+
+def precision_enum(name: str) -> int:
+    """The PREC_* value of a precision name; ValueError naming the valid ones otherwise."""
+    if name not in PRECISIONS:
+        raise ValueError(f"precision must be one of {sorted(PRECISIONS)}, got {name!r}")
+    return PRECISIONS[name]
 
 
 def lib_path() -> Path:

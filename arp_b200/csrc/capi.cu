@@ -1,6 +1,7 @@
 // C-ABI implementation of include/arp_b200.h: handle, weight packing, TMA descriptors and the
-// stream-ordered pipeline   decode -> patch-embed GEMM -> ln_pre -> 12 x [QKV (ln_1 folded), attention, out-proj (+= x),
-// row moments, c_fc (ln_2 folded, QuickGELU), c_proj (+= x), row moments] -> reward head -> per-episode return-to-go scan.
+// stream-ordered pipeline   decode -> patch-embed GEMM -> ln_pre -> 12 x [QKV (ln_1 folded), attention, out-proj (+= x,
+// row moments), c_fc (ln_2 folded, QuickGELU), c_proj (+= x, row moments)] (the last block for the class-token row only)
+// -> reward head -> per-episode return-to-go scan.
 // Host logic only; every kernel lives in the .cuh next to this file.
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -117,24 +118,9 @@ struct ArpHandle {
   // epilogues from per-row moments — no LayerNorm kernels, no normalised copy, no fp32 read-modify-write.
   // false (ARP_PREC_F32RESID): fp32 x, standalone LayerNorm kernels writing a 16-bit copy (round 1's pipeline).
   bool resid16 = true;
-  // Row statistics of the 16-bit stream. false (default): the residual GEMMs add in registers and emit the statistics
-  // themselves (gemm_tcgen05.cuh G2_RESID_STATS; one rounding per update, no LayerNorm-class kernel inside the blocks).
-  // true (ARP_FUSED_STATS=0, measurement switch): x is updated by 16-bit TMA reduce-add and row_moments_kernel re-reads it.
-  // Measured on B200 (profiles/r02_stats_ab.json): isolated, c_proj 751 -> 731 us and out_proj 212 -> 255 us at 1024
-  // frames against 2 x 52 us of statistics kernels saved; inside the power-capped step the two forms are within 1 %.
-  bool stats_kernel = false;
   // Snake order: consecutive kernels of a chunk walk the rows in opposite directions, so each starts on what its
-  // predecessor wrote last (the tail of a 150-600 MB activation is still in the 126 MB L2). ARP_SNAKE=0 disables.
-  bool snake = true;
+  // predecessor wrote last (the tail of a 150-600 MB activation is still in the 126 MB L2). Flipped at every launch.
   int dir = 0;
-  // Last-layer pruning: every head reads only the class-token row of the last resblock's output (ln_post(x[:,0]),
-  // adapter taps = CLS rows), so that block computes K/V for all tokens but Q, attention, out_proj and the MLP for
-  // the class-token row only — same result, 2.4 of 35.1 GFLOP per frame less. ARP_PRUNE_LAST=0 disables.
-  // arp_encode_taps_chw: the chunk's input is a caller-preprocessed fp32 image batch instead of dataset bytes, and the
-  // class-token row of every block's output is copied out (fp32 [n, layers*W]) — the frozen-CLIP side of fine-tuning
-  const float* cur_chw = nullptr;
-  float* cur_taps32 = nullptr;
-  bool prune_last = true;
   bool f32 = false;   // cfg.precision == ARP_PREC_F32: verification path (fp32_path.cuh); GEMM weights are stored as fp32
   int tokens = 0, grid = 0, kp = 0;  // 197, 14, 768
   bool adapter = false, goal = false;
@@ -171,7 +157,6 @@ struct ArpHandle {
     bf16 *xn = nullptr, *qkv = nullptr, *attn = nullptr, *hid = nullptr;
     bf16 *taps = nullptr, *featb = nullptr, *hid2 = nullptr;
     float *featf = nullptr, *mlp = nullptr;
-    bool cls_compact = false;                                    // the heads read xcls (stride 1) instead of x (stride tokens)
     float* xcls = nullptr;                                       // [B, W] class-token residual rows (last-layer pruning)
     bf16 *xncls = nullptr, *qcls = nullptr, *acls = nullptr, *hcls = nullptr;   // [B,W] x3, [B,4W]
     // fp32 verification path
@@ -565,9 +550,6 @@ extern "C" int arp_create(const ArpConfig* cfg, ArpHandle** out) {
   if (cudaSetDevice(cfg->device) != cudaSuccess) { h->err = "cudaSetDevice failed"; return bail(ARP_ERR_CUDA); }
   h->f32 = cfg->precision == ARP_PREC_F32;
   h->resid16 = cfg->precision == ARP_PREC_BF16;
-  if (const char* e = getenv("ARP_SNAKE")) h->snake = atoi(e) != 0;            // measurement switches, both exact:
-  if (const char* e = getenv("ARP_PRUNE_LAST")) h->prune_last = atoi(e) != 0;  // kernel order / last-block pruning
-  if (const char* e = getenv("ARP_FUSED_STATS")) h->stats_kernel = atoi(e) == 0;
   h->grid = DEC_OUT / cfg->patch;
   h->tokens = h->grid * h->grid + 1;
   h->kp = 3 * cfg->patch * cfg->patch;
@@ -890,7 +872,7 @@ static int launch_gemm(ArpHandle* h, const bf16* a, int64_t a_rows_alloc, const 
   memset(&g, 0, sizeof(g));
   g.M = (int)M; g.N = N; g.K = K; g.out = out; g.ldo = ldo; g.bias = bias;
   g.rowtab = rowtab; g.period = period > 0 ? period : 1;
-  g.reverse = h->snake ? (h->dir ^= 1) : 0;
+  g.reverse = h->dir ^= 1;
   const bool reduce = resid != nullptr;
   if (fold) {
     if (out_f32 || act == ACT_RELU || reduce || rowtab || !fold->stats || !fold->svec || !fold->cvec)
@@ -982,8 +964,7 @@ static int launch_ln_bf16(ArpHandle* h, const float* x, const float* g, const fl
                           cudaStream_t st) {
   if (M <= 0) return ARP_OK;
   ProfScope prof(h, PC_LAYERNORM, 0.0, (double)M * 768 * 6, st);
-  layernorm_f32_bf16_kernel<768><<<(unsigned)((M + 7) / 8), 256, 0, st>>>(x, g, b, y, (int)M, 1e-5f,
-                                                                         h->snake ? (h->dir ^= 1) : 0);
+  layernorm_f32_bf16_kernel<768><<<(unsigned)((M + 7) / 8), 256, 0, st>>>(x, g, b, y, (int)M, 1e-5f, h->dir ^= 1);
   h->launches++;
   ARP_CUDA(h, cudaGetLastError());
   return ARP_OK;
@@ -993,7 +974,7 @@ static int launch_ln_bf16(ArpHandle* h, const float* x, const float* g, const fl
 static int launch_row_moments(ArpHandle* h, const bf16* x, float2* stats, int64_t M, cudaStream_t st) {
   if (M <= 0) return ARP_OK;
   ProfScope prof(h, PC_LAYERNORM, 0.0, (double)M * (768 * 2 + 8), st);
-  row_moments_kernel<768><<<(unsigned)((M + 7) / 8), 256, 0, st>>>(x, stats, (int)M, 1e-5f, h->snake ? (h->dir ^= 1) : 0);
+  row_moments_kernel<768><<<(unsigned)((M + 7) / 8), 256, 0, st>>>(x, stats, (int)M, 1e-5f, h->dir ^= 1);
   h->launches++;
   ARP_CUDA(h, cudaGetLastError());
   return ARP_OK;
@@ -1016,7 +997,7 @@ static int launch_attention(ArpHandle* h, const bf16* qkv, bf16* out, int B, int
   ARP_TRY(get_tmap(h, qkv, rows, 3 * W, 3 * W, 16, &tq16));            // 16-row boxes: query tile 1 spread over the quarters
   ARP_TRY(get_tmap_attn_out(h, out, (uint64_t)B, (uint64_t)tokens, (uint64_t)W, &to16, 16));
   const int grid = std::min(B * h->cfg.heads, kNumSMs);
-  const int rev = h->snake ? (h->dir ^= 1) : 0;
+  const int rev = h->dir ^= 1;
   if (tokens == 197)
     attention_tc_kernel<197><<<grid, ATC_THREADS, AtcCfg<197>::SMEM_BYTES, st>>>(*tq, *tkv, *to, *tq16, *to16, B, h->cfg.heads, W, scale_log2e, rev);
   else
@@ -1029,12 +1010,16 @@ static int launch_attention(ArpHandle* h, const bf16* qkv, bf16* out, int B, int
 // ------------------------------------------------------------------------------------------------
 // the encoder: n frames (n <= max_batch) -> residual stream x after the last block (+ CLS taps)
 // ------------------------------------------------------------------------------------------------
-static int encode_chunk_f32(ArpHandle* h, const uint8_t* ob, int64_t n, int64_t stride, cudaStream_t st);
+static int encode_chunk_f32(ArpHandle* h, const uint8_t* ob, int64_t n, int64_t stride, cudaStream_t st,
+                            const float* chw, float* taps32);
 
-// The last resblock for the class-token row only (see ArpHandle::prune_last). K and V of every token are already in
-// ws.qkv (columns [W, 3W)); XT = type of the residual stream `x` the class-token rows are gathered from.
+// The last resblock for the class-token row only: every head reads just the class-token row of the last block's output
+// (ln_post(x[:,0]), adapter taps = class-token rows), so that block computes K/V for all tokens but Q, attention,
+// out_proj and the MLP for the class-token row only — same result, 2.4 of 35.1 GFLOP per frame less. K and V of every
+// token are already in ws.qkv (columns [W, 3W)); XT = type of the residual stream `x` the class-token rows are gathered
+// from. The heads read the result from ws.xcls.
 template <typename XT>
-static int last_block_cls(ArpHandle* h, const LayerW& L, const XT* x, int64_t n, cudaStream_t st) {
+static int last_block_cls(ArpHandle* h, const LayerW& L, const XT* x, int64_t n, cudaStream_t st, float* taps32) {
   const ArpConfig& c = h->cfg;
   ArpHandle::Work& ws = h->ws;
   const int W = c.width;
@@ -1066,33 +1051,34 @@ static int last_block_cls(ArpHandle* h, const LayerW& L, const XT* x, int64_t n,
     gather_cls_bf16_kernel<768, float><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(ws.xcls, ws.taps, (int)n, 1, c.layers * W, l * W);
     h->launches++;
   }
-  if (h->cur_taps32) {
-    gather_cls_rows_f32_kernel<768, float><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(ws.xcls, h->cur_taps32, (int)n, 1,
+  if (taps32) {
+    gather_cls_rows_f32_kernel<768, float><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(ws.xcls, taps32, (int)n, 1,
                                                                                  c.layers * W, l * W);
     h->launches++;
   }
-  ws.cls_compact = true;
   return ARP_OK;
 }
 
-// class-token taps of block l's output: 16-bit for the adapter head, fp32 for arp_encode_taps_chw
+// class-token taps of block l's output: 16-bit for the adapter head, fp32 into taps32 for arp_encode_taps_chw
 template <typename XT>
-static void gather_taps(ArpHandle* h, const XT* x, int64_t n, int l, cudaStream_t st) {
+static void gather_taps(ArpHandle* h, const XT* x, int64_t n, int l, cudaStream_t st, float* taps32) {
   const ArpConfig& c = h->cfg;
   if (h->adapter) {
     gather_cls_bf16_kernel<768, XT><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(x, h->ws.taps, (int)n, h->tokens,
                                                                           c.layers * c.width, l * c.width);
     h->launches++;
   }
-  if (h->cur_taps32) {
-    gather_cls_rows_f32_kernel<768, XT><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(x, h->cur_taps32, (int)n, h->tokens,
+  if (taps32) {
+    gather_cls_rows_f32_kernel<768, XT><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(x, taps32, (int)n, h->tokens,
                                                                               c.layers * c.width, l * c.width);
     h->launches++;
   }
 }
 
-// Default path: 16-bit residual stream, LayerNorm folded into the consumer GEMMs (ArpHandle::resid16).
-static int encode_blocks_r16(ArpHandle* h, int64_t n, cudaStream_t st) {
+// Default path: 16-bit residual stream, LayerNorm folded into the consumer GEMMs (ArpHandle::resid16). The residual
+// GEMMs add in registers and emit the next LayerNorm's row statistics themselves (gemm_tcgen05.cuh G2_RESID_STATS): one
+// rounding per update and no LayerNorm-class kernel inside the blocks.
+static int encode_blocks_r16(ArpHandle* h, int64_t n, cudaStream_t st, float* taps32) {
   const ArpConfig& c = h->cfg;
   ArpHandle::Work& ws = h->ws;
   const int W = c.width;
@@ -1103,47 +1089,39 @@ static int encode_blocks_r16(ArpHandle* h, int64_t n, cudaStream_t st) {
                                                                           ws.stats, (int)M, 1e-5f);
     h->launches++;
   }
-  // format of ws.stats: 1 = (rstd, -mean*rstd) per row (statistics kernels), 2*W/256 = partial (mean, M2) per 128 columns
-  // (written by the residual GEMM's epilogue)
+  // format of ws.stats: 1 = (rstd, -mean*rstd) per row (layernorm_pre_r16_kernel), 2*W/256 = partial (mean, M2) per 128
+  // columns (written by the residual GEMM's epilogue)
   int parts = 1;
-  const int gemm_parts = 2 * W / 256;
   for (int l = 0; l < c.layers; ++l) {
     const LayerW& L = h->layers[l];
-    if (l == c.layers - 1 && h->prune_last) {
+    if (l == c.layers - 1) {
       // K and V of every token: rows [W, 3W) of in_proj, written at column W of the qkv buffer
       const LnFoldArgs f_kv{ws.stats, L.s_qkv + W, L.c_qkv + W, parts};
       ARP_TRY(launch_gemm(h, ws.x16, Mcap, L.w_qkv_fold + (size_t)W * W, ws.qkv + W, false, ACT_NONE, M, 2 * W, W, 3 * W,
                           nullptr, nullptr, 0, nullptr, 0, st, &f_kv));
-      ARP_TRY(last_block_cls(h, L, ws.x16, n, st));
+      ARP_TRY(last_block_cls(h, L, ws.x16, n, st, taps32));
       break;
     }
     const LnFoldArgs f_qkv{ws.stats, L.s_qkv, L.c_qkv, parts};
     ARP_TRY(launch_gemm(h, ws.x16, Mcap, L.w_qkv_fold, ws.qkv, false, ACT_NONE, M, 3 * W, W, 3 * W, nullptr, nullptr, 0,
                         nullptr, 0, st, &f_qkv));
-    parts = h->stats_kernel ? 1 : gemm_parts;
+    parts = 2 * W / 256;
     const LnFoldArgs f_fc{ws.stats, L.s_fc, L.c_fc, parts};
     ARP_TRY(launch_attention(h, ws.qkv, ws.attn, (int)n, h->tokens, st, Mcap));
     // x += out_proj(attn) in place; the epilogue also leaves ln_2's row statistics in ws.stats
     ARP_TRY(launch_gemm(h, ws.attn, Mcap, L.w_out, ws.x16, false, ACT_NONE, M, W, W, W, L.b_out, ws.x16, W, nullptr, 0, st,
-                        nullptr, h->stats_kernel ? nullptr : ws.stats));
-    if (h->stats_kernel) ARP_TRY(launch_row_moments(h, ws.x16, ws.stats, M, st));
+                        nullptr, ws.stats));
     ARP_TRY(launch_gemm(h, ws.x16, Mcap, L.w_fc_fold, ws.hid, false, ACT_QUICKGELU, M, 4 * W, W, 4 * W, nullptr, nullptr,
                         0, nullptr, 0, st, &f_fc));
     ARP_TRY(launch_gemm(h, ws.hid, Mcap, L.w_proj, ws.x16, false, ACT_NONE, M, W, 4 * W, W, L.b_proj, ws.x16, W, nullptr,
-                        0, st, nullptr, h->stats_kernel ? nullptr : ws.stats));   // ... and the next block's ln_1 statistics
-    if (h->stats_kernel && l + 1 < c.layers) ARP_TRY(launch_row_moments(h, ws.x16, ws.stats, M, st));
-    gather_taps(h, ws.x16, n, l, st);
-  }
-  if (!ws.cls_compact) {   // prune_last off: hand the heads compact fp32 class-token rows all the same
-    gather_cls_rows_f32_kernel<768, bf16><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(ws.x16, ws.xcls, (int)n, h->tokens, W, 0);
-    h->launches++;
-    ws.cls_compact = true;
+                        0, st, nullptr, ws.stats));   // ... and the next block's ln_1 statistics
+    gather_taps(h, ws.x16, n, l, st, taps32);
   }
   return ARP_OK;
 }
 
 // ARP_PREC_F32RESID: fp32 residual stream, standalone LayerNorm kernels writing the 16-bit GEMM operand.
-static int encode_blocks_r32(ArpHandle* h, int64_t n, cudaStream_t st) {
+static int encode_blocks_r32(ArpHandle* h, int64_t n, cudaStream_t st, float* taps32) {
   const ArpConfig& c = h->cfg;
   ArpHandle::Work& ws = h->ws;
   const int W = c.width;
@@ -1156,10 +1134,10 @@ static int encode_blocks_r32(ArpHandle* h, int64_t n, cudaStream_t st) {
   for (int l = 0; l < c.layers; ++l) {
     const LayerW& L = h->layers[l];
     ARP_TRY(launch_ln_bf16(h, ws.x, L.ln1_g, L.ln1_b, ws.xn, M, st));
-    if (l == c.layers - 1 && h->prune_last) {
+    if (l == c.layers - 1) {
       ARP_TRY(launch_gemm(h, ws.xn, Mcap, L.w_qkv + (size_t)W * W, ws.qkv + W, false, ACT_NONE, M, 2 * W, W, 3 * W,
                           L.b_qkv + W, nullptr, 0, nullptr, 0, st));
-      ARP_TRY(last_block_cls(h, L, ws.x, n, st));
+      ARP_TRY(last_block_cls(h, L, ws.x, n, st, taps32));
       break;
     }
     ARP_TRY(launch_gemm(h, ws.xn, Mcap, L.w_qkv, ws.qkv, false, ACT_NONE, M, 3 * W, W, 3 * W, L.b_qkv, nullptr, 0,
@@ -1170,22 +1148,26 @@ static int encode_blocks_r32(ArpHandle* h, int64_t n, cudaStream_t st) {
     ARP_TRY(launch_gemm(h, ws.xn, Mcap, L.w_fc, ws.hid, false, ACT_QUICKGELU, M, 4 * W, W, 4 * W, L.b_fc, nullptr, 0,
                         nullptr, 0, st));
     ARP_TRY(launch_gemm(h, ws.hid, Mcap, L.w_proj, ws.x, true, ACT_NONE, M, W, 4 * W, W, L.b_proj, ws.x, W, nullptr, 0, st));
-    gather_taps(h, ws.x, n, l, st);
+    gather_taps(h, ws.x, n, l, st, taps32);
   }
   return ARP_OK;
 }
 
-static int encode_chunk(ArpHandle* h, const uint8_t* ob, int64_t n, int64_t stride, cudaStream_t st) {
-  if (h->f32) return encode_chunk_f32(h, ob, n, stride, st);
+// Input: n dataset frames at ob (row pitch `stride`), or, when chw is set, a caller-preprocessed fp32 image batch
+// [n, 3, 224, 224]. taps32 (optional, arp_encode_taps_chw): fp32 [n, layers*W] receives the class-token row of every
+// block's output — the frozen-CLIP side of fine-tuning.
+static int encode_chunk(ArpHandle* h, const uint8_t* ob, int64_t n, int64_t stride, cudaStream_t st,
+                        const float* chw = nullptr, float* taps32 = nullptr) {
+  if (h->f32) return encode_chunk_f32(h, ob, n, stride, st, chw, taps32);
   const ArpConfig& c = h->cfg;
   ArpHandle::Work& ws = h->ws;
   const int W = c.width;
   const int64_t M = n * h->tokens;
   const int64_t Mcap = (int64_t)c.max_batch * h->tokens;
   bf16* patches = ws.hid;  // aliases the MLP hidden buffer (dead until layer 0's c_fc)
-  if (h->cur_chw) {
+  if (chw) {
     ProfScope prof(h, PC_DECODE, 0.0, (double)n * (3.0 * DEC_OUT * DEC_OUT * 4 + (double)h->tokens * h->kp * 2), st);
-    patchify_chw_bf16_kernel<<<kNumSMs * 8, 256, 0, st>>>(h->cur_chw, patches, (int)n, c.patch, h->grid, h->tokens);
+    patchify_chw_bf16_kernel<<<kNumSMs * 8, 256, 0, st>>>(chw, patches, (int)n, c.patch, h->grid, h->tokens);
     h->launches++;
   } else {
     ARP_TRY(launch_decode(h, ob, n, stride, patches, DEC_OUT_PATCH_BF16, st));
@@ -1193,8 +1175,7 @@ static int encode_chunk(ArpHandle* h, const uint8_t* ob, int64_t n, int64_t stri
   // patch embed (+ positional embedding, + class embedding on the all-zero row 0 of each frame), fp32 out
   ARP_TRY(launch_gemm(h, patches, Mcap, h->conv1, ws.x, true, ACT_NONE, M, W, h->kp, W, nullptr, nullptr, 0,
                       h->rowtab, h->tokens, st));
-  ws.cls_compact = false;
-  ARP_TRY(h->resid16 ? encode_blocks_r16(h, n, st) : encode_blocks_r32(h, n, st));
+  ARP_TRY(h->resid16 ? encode_blocks_r16(h, n, st, taps32) : encode_blocks_r32(h, n, st, taps32));
   ARP_CUDA(h, cudaGetLastError());
   return ARP_OK;
 }
@@ -1216,17 +1197,17 @@ static int launch_sgemm(ArpHandle* h, const float* a, int lda, const void* w, fl
   return ARP_OK;
 }
 
-static int encode_chunk_f32(ArpHandle* h, const uint8_t* ob, int64_t n, int64_t stride, cudaStream_t st) {
+// The verification path computes every row of every block: the heads read the class-token rows from ws.x.
+static int encode_chunk_f32(ArpHandle* h, const uint8_t* ob, int64_t n, int64_t stride, cudaStream_t st,
+                            const float* chw, float* taps32) {
   const ArpConfig& c = h->cfg;
   ArpHandle::Work& ws = h->ws;
-  ws.cls_compact = false;   // the verification path computes every row of every block
   const int W = c.width;
   const int64_t M = n * h->tokens;
   if (h->tokens != 197 && h->tokens != 50) return fail(h, ARP_ERR_INVALID, "unsupported token count %d", h->tokens);
   float* patches = ws.hid32;   // dead until layer 0's c_fc
-  if (!h->cur_chw) ARP_TRY(launch_decode(h, ob, n, stride, ws.chw32, DEC_OUT_CHW_F32, st));
-  im2col_f32_kernel<<<kNumSMs * 8, 256, 0, st>>>(h->cur_chw ? h->cur_chw : ws.chw32, patches, (int)n, c.patch, h->grid,
-                                                 h->tokens);
+  if (!chw) ARP_TRY(launch_decode(h, ob, n, stride, ws.chw32, DEC_OUT_CHW_F32, st));
+  im2col_f32_kernel<<<kNumSMs * 8, 256, 0, st>>>(chw ? chw : ws.chw32, patches, (int)n, c.patch, h->grid, h->tokens);
   h->launches++;
   ARP_TRY(launch_sgemm(h, patches, h->kp, h->conv1, ws.x, W, F32_ACT_NONE, M, W, h->kp, nullptr, nullptr, 0, h->rowtab,
                        h->tokens, st));
@@ -1261,8 +1242,8 @@ static int encode_chunk_f32(ArpHandle* h, const uint8_t* ob, int64_t n, int64_t 
                                                                         c.layers * W, l * W);
       h->launches++;
     }
-    if (h->cur_taps32) {
-      gather_cls_rows_f32_kernel<768, float><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(ws.x, h->cur_taps32, (int)n, h->tokens,
+    if (taps32) {
+      gather_cls_rows_f32_kernel<768, float><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(ws.x, taps32, (int)n, h->tokens,
                                                                         c.layers * W, l * W);
       h->launches++;
     }
@@ -1278,8 +1259,8 @@ static int head_chunk(ArpHandle* h, int64_t n, float* reward_out, float* logits_
   ArpHandle::Work& ws = h->ws;
   const bool need_text = reward_out || logits_out;
   if (need_text && !h->goal && !h->text) return fail(h, ARP_ERR_STATE, "arp_set_text has not been called");
-  const float* xsrc = ws.cls_compact ? ws.xcls : ws.x;     // class-token rows: compact after last-layer pruning
-  const int xtok = ws.cls_compact ? 1 : h->tokens;
+  const float* xsrc = h->f32 ? ws.x : ws.xcls;     // class-token rows: compact after the tensor-core paths' pruned last block
+  const int xtok = h->f32 ? h->tokens : 1;
   if (!h->adapter) {
     ProfScope prof(h, PC_HEAD, 2.0 * (double)n * 768 * 512, (double)n * 768 * 4 + 768.0 * 512 * 4, st);
     clip_head_kernel<768, 512><<<(unsigned)((n + HEAD_FR - 1) / HEAD_FR), 256, HEAD_SMEM_BYTES, st>>>(
@@ -1429,17 +1410,12 @@ extern "C" int arp_encode_taps_chw(ArpHandle* h, const float* chw_dev, int64_t T
   ARP_TRY(finalize_weights(h, st));
   const int64_t B = h->cfg.max_batch;
   const size_t img = (size_t)3 * DEC_OUT * DEC_OUT, tw = (size_t)h->cfg.layers * h->cfg.width;
-  int rc = ARP_OK;
-  for (int64_t t0 = 0; t0 < T && rc == ARP_OK; t0 += B) {
+  for (int64_t t0 = 0; t0 < T; t0 += B) {
     const int64_t n = std::min(B, T - t0);
-    h->cur_chw = chw_dev + t0 * img;
-    h->cur_taps32 = taps_dev ? taps_dev + t0 * tw : nullptr;
-    rc = encode_chunk(h, nullptr, n, 0, st);
-    if (rc == ARP_OK && feat_dev) rc = head_chunk(h, n, nullptr, nullptr, feat_dev + t0 * h->feat_dim, st);
+    ARP_TRY(encode_chunk(h, nullptr, n, 0, st, chw_dev + t0 * img, taps_dev ? taps_dev + t0 * tw : nullptr));
+    if (feat_dev) ARP_TRY(head_chunk(h, n, nullptr, nullptr, feat_dev + t0 * h->feat_dim, st));
   }
-  h->cur_chw = nullptr;
-  h->cur_taps32 = nullptr;
-  return rc;
+  return ARP_OK;
 }
 
 static int scan_launch(ArpHandle* h, const float* reward, int64_t T, const int64_t* ep_off, int n_eps, int F,

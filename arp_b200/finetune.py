@@ -23,7 +23,7 @@ import torch
 import torch.nn.functional as F
 from torch import nn
 
-from . import text_tower
+from . import capi, text_tower
 from .weights import ARCH
 
 _MEAN = (0.48145466, 0.4578275, 0.40821073)
@@ -57,11 +57,12 @@ class FrozenClip(nn.Module):
     is a no-op and the optimizer never sees CLIP), and evaluates the vision tower through the native library."""
 
     def __init__(self, state_dict: dict, arch: str = "ViT-B/16", max_batch: int = 256, precision: str = "16bit"):
+        prec = capi.precision_enum(precision)
         super().__init__()
         self.arch = arch
         self.patch, self.vision_width, self.vision_layers, self.embed_dim, self.text_width, self.text_layers = ARCH[arch][:6]
         self._sd = {k: v.detach().clone() for k, v in state_dict.items() if torch.is_tensor(v)}
-        self._max_batch, self._precision = int(max_batch), precision
+        self._max_batch, self._precision = int(max_batch), prec
         self._engine = None
         self._engine_stale = True
         self._text_cache: dict = {}
@@ -105,18 +106,15 @@ class FrozenClip(nn.Module):
 
     # -- frozen forward passes ----------------------------------------------------------------------------------
     def _get_engine(self, device: torch.device):
-        from . import capi
         if device.type != "cuda":
             raise RuntimeError("the frozen CLIP tower runs in libarp_b200.so on a B200: move the module and its "
                                "inputs to a CUDA device (there is no CPU fallback)")
         idx = device.index if device.index is not None else torch.cuda.current_device()
         if self._engine is None or self._engine.cfg.device != idx:
-            prec = {"16bit": capi.PREC_16BIT, "bf16": capi.PREC_16BIT, "fp16": capi.PREC_16BIT, "fp32resid": capi.PREC_F32RESID,
-                    "fp32": capi.PREC_F32}[self._precision]
             self._engine = capi.Engine(device=idx, patch=self.patch, in_h=224, in_w=224, preprocess=capi.PRE_BILINEAR,
                                        head=capi.HEAD_CLIP, max_batch=self._max_batch, layers=self.vision_layers,
                                        width=self.vision_width, heads=self.vision_width // 64,
-                                       embed_dim=self.embed_dim, precision=prec)
+                                       embed_dim=self.embed_dim, precision=self._precision)
             self._engine_stale = True
         if self._engine_stale:
             missing = self._engine.load_state_dict({k: v for k, v in self._sd.items() if k.startswith("visual.")})

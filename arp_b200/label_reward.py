@@ -112,10 +112,6 @@ def _resolve_clip_weights(clip_state_dict, arch: str) -> dict:
             "label_reward.py:126)") from e
 
 
-PRECISIONS = {"16bit": capi.PREC_16BIT, "bf16": capi.PREC_16BIT, "fp16": capi.PREC_16BIT,
-              "fp32resid": capi.PREC_F32RESID, "fp32": capi.PREC_F32}
-
-
 # One native handle is kept alive between label_reward() calls of a process (key = its whole configuration): creating it
 # (4 GB of workspace, the pinned staging ring) and tearing it down cost ~0.25 s, a tenth of a 70k-frame labeling pass.
 # Weights and the instruction embedding are uploaded again on every call. release_cached_engine() frees it.
@@ -148,8 +144,7 @@ class RewardLabeler:
                  clip_state_dict=None, arch: str = "ViT-B/16", use_crop: bool = False, reduce: str = "first",
                  max_batch: int = 1024, device: int | None = None, precision: str = "16bit", tokenizer=None):
         head, pre = _head_for(model_type)
-        if precision not in PRECISIONS:
-            raise ValueError(f"precision must be one of {sorted(PRECISIONS)}, got {precision!r}")
+        prec = capi.precision_enum(precision)
         adapter = head in (capi.HEAD_ADAPTER, capi.HEAD_ADAPTER_ENSEMBLE, capi.HEAD_ADAPTER_GOAL)
         if adapter:
             assert model_ckpt_dir is not None, "specify model_ckpt_dir"  # label_reward.py:174
@@ -160,7 +155,7 @@ class RewardLabeler:
         self.engine = _cached_engine(device=device, patch=patch, in_h=int(frame_hw[0]), in_w=int(frame_hw[1]),
                                      use_crop=bool(use_crop), preprocess=pre, head=head,
                                      reduce=capi.REDUCE_MEAN if reduce == "mean" else capi.REDUCE_FIRST,
-                                     max_batch=int(max_batch), precision=PRECISIONS[precision])
+                                     max_batch=int(max_batch), precision=prec)
         dev = self.engine.device
         if adapter:
             sd = load_checkpoint(model_ckpt_dir) if not isinstance(model_ckpt_dir, dict) else model_ckpt_dir
@@ -494,7 +489,7 @@ def main():
     parser.add_argument("--arch", type=str, default="ViT-B/16")
     parser.add_argument("--reduce", type=str, default="first", choices=["first", "mean"])
     parser.add_argument("--max_batch", type=int, default=1024)
-    parser.add_argument("--precision", type=str, default="16bit", choices=sorted(PRECISIONS))
+    parser.add_argument("--precision", type=str, default="16bit", choices=sorted(capi.PRECISIONS))
     parser.add_argument("--tokenizer", type=str, default=None, choices=["clip", "standin"])
     args = parser.parse_args()
 

@@ -37,13 +37,14 @@ class OnlineClip:
 
     def __init__(self, vl_type: str = "clip", *, vl_checkpoint=None, clip_state_dict=None, arch: str = "ViT-B/16",
                  device: int | None = None, max_batch: int = 2, precision: str = "16bit", tokenizer=None):
+        self._precision = capi.precision_enum(precision)
         if vl_type not in ("clip", "clip_goal_conditioned", "clip_ft", "clip_ft_goal_conditioned"):
             raise ValueError(vl_type)                                         # rollout_procgen.py:145
         self.vl_type, self.arch = vl_type, arch
         self.adapter = vl_type.startswith("clip_ft")
         self.goal = vl_type.endswith("goal_conditioned")
         self.device_index = int(os.environ.get("LOCAL_RANK", "0")) if device is None else device
-        self.max_batch, self.precision = max_batch, precision
+        self.max_batch = max_batch
         self._tokenize = resolve_tokenizer(tokenizer)   # refuses the stand-in unless opted in (tokenizer.py)
         if self.adapter:
             assert vl_checkpoint, "You have to specifiy vl_checkpoint."     # main_procgen.py:585
@@ -70,7 +71,7 @@ class OnlineClip:
             # clip.load's preprocess for every vl_type (main_procgen.py:570,572): PIL bicubic, not the adapter's bilinear
             e = capi.Engine(device=self.device_index, patch=32 if self.arch.endswith("/32") else 16, in_h=h, in_w=w,
                             preprocess=capi.PRE_PIL_BICUBIC, head=self._head(), max_batch=self.max_batch,
-                            precision={"fp32": capi.PREC_F32, "fp32resid": capi.PREC_F32RESID}.get(self.precision, capi.PREC_16BIT))
+                            precision=self._precision)
             missing = e.load_state_dict(self.sd, strict=False)
             if missing:
                 raise RuntimeError(f"checkpoint lacks {len(missing)} tensors, e.g. {missing[:3]}")

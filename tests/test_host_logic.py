@@ -262,3 +262,43 @@ def test_label_reward_refuses_without_a_tokenizer(tmp_path, monkeypatch):
     monkeypatch.setattr(capi, "Engine", FakeEngine)
     with pytest.raises(tk.TokenizerUnavailable):
         RewardLabeler("clip", "the goal is to collect the coin.", (64, 64), clip_state_dict={"visual.proj": torch.zeros(1)})
+
+
+def test_precision_names_are_one_table(monkeypatch):
+    """label_reward, OnlineClip and FrozenClip accept exactly the names of capi.PRECISIONS and hand the engine the same
+    enum for each; an unknown name is refused with ValueError when the object is built, before the library is used."""
+    from arp_b200 import capi, label_reward
+    from arp_b200.finetune import FrozenClip
+    from arp_b200.online import OnlineClip
+    from arp_b200.weights import random_clip_state_dict
+    assert sorted(capi.PRECISIONS) == ["16bit", "bf16", "fp16", "fp32", "fp32resid"]
+    built = []
+
+    class FakeEngine:                                       # no GPU here: record what the engine would be built with
+        device, goal = torch.device("cpu"), True
+        def __init__(self, **kw):
+            self.kw = kw
+            built.append(kw)
+        def load_state_dict(self, sd, strict=False): return []
+        def close(self): pass
+
+    def no_library():
+        raise AssertionError("the native library was used")
+    monkeypatch.setattr(capi, "Engine", FakeEngine)
+    monkeypatch.setattr(capi, "load_library", no_library)
+    monkeypatch.setattr(label_reward, "_ENGINE_CACHE", {})   # the labeler's handle cache: start and leave it untouched
+    sd = random_clip_state_dict("ViT-B/32", 0, device="cpu", with_text=False)
+    entry_points = {
+        "label_reward": lambda p: label_reward.RewardLabeler("clip_goal_conditioned", None, (64, 64), clip_state_dict=sd,
+                                                             arch="ViT-B/32", precision=p).engine,
+        "online": lambda p: OnlineClip("clip", clip_state_dict=sd, arch="ViT-B/32", precision=p)._engine(64, 64),
+        "finetune": lambda p: FrozenClip(sd, arch="ViT-B/32", precision=p)._get_engine(torch.device("cuda", 0)),
+    }
+    for name, make in entry_points.items():
+        for p, enum in capi.PRECISIONS.items():
+            assert make(p).kw["precision"] == enum, (name, p)
+        n = len(built)
+        for bad in ("bf32", "FP32", "fp16 ", "", None):
+            with pytest.raises(ValueError, match="precision must be one of"):
+                make(bad)
+        assert len(built) == n, name
