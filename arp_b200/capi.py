@@ -26,7 +26,9 @@ PREC_BF16, PREC_F32, PREC_F32RESID = 0, 1, 2   # PREC_BF16 = the 16-bit tensor-c
 PREC_16BIT = PREC_BF16
 #: precision names of the Python entry points ("bf16" / "fp16" name the 16-bit path whatever the operand format)
 PRECISIONS = {"16bit": PREC_16BIT, "bf16": PREC_16BIT, "fp16": PREC_16BIT, "fp32resid": PREC_F32RESID, "fp32": PREC_F32}
-MAX_TEXT = 16
+MAX_TEXT = 16            # texts of one instruction set (one text group)
+MAX_TEXT_GROUPS = 16     # instruction sets of one set_text_groups call
+MAX_TEXT_TOTAL = 64      # texts of all groups together
 
 #: every symbol include/arp_b200.h declares (tests check the library exports exactly these)
 EXPORTS = (
@@ -35,6 +37,7 @@ EXPORTS = (
     "arp_scan_only", "arp_gemm_bf16", "arp_layernorm_bf16", "arp_attention", "arp_launch_count",
     "arp_profile_begin", "arp_profile_end", "arp_online_reward", "arp_preprocess_rtgs",
     "arp_quantile_f32", "arp_encode_taps_chw", "arp_operand_dtype", "arp_ln_gemm", "arp_resid_gemm_stats", "arp_label_file", "arp_wants_weight",
+    "arp_set_text_groups", "arp_text_groups",
 )
 PROFILE_CLASSES = ("gemm", "attention", "layernorm", "decode", "head", "scan", "other")
 
@@ -90,6 +93,8 @@ def load_library() -> C.CDLL:
     lib.arp_set_weight.argtypes = [vp, C.c_char_p, vp, i32, C.POINTER(i64), i32, vp]
     lib.arp_missing_weights.argtypes = [vp, C.c_char_p, i64]
     lib.arp_set_text.argtypes = [vp, vp, i32, i32, f32, vp]
+    lib.arp_set_text_groups.argtypes = [vp, vp, i32, i32, vp, i32, f32, vp]
+    lib.arp_text_groups.argtypes = [vp]
     lib.arp_label.argtypes = [vp, vp, i64, i64, vp, i32, i32, vp, vp, vp, vp, vp]
     lib.arp_label_host.argtypes = [vp, vp, i64, i64, vp, i32, i32, vp, vp, vp, vp]
     lib.arp_label_file.argtypes = [vp, i32, i64, i64, i64, vp, i32, i32, vp, vp, vp, vp]
@@ -154,6 +159,7 @@ class Engine:
         self.goal = head in (HEAD_CLIP_GOAL, HEAD_ADAPTER_GOAL)
         self.feat_dim = (layers + 1) * embed_dim if self.adapter else embed_dim
         self.n_text = 0
+        self._grouped = False            # set_text_groups was called last: outputs carry a leading group axis
 
     # -- lifetime ---------------------------------------------------------------------------------
     def close(self):
@@ -232,6 +238,36 @@ class Engine:
                                            _stream_ptr(self.device)))
         torch.cuda.current_stream(self.device).synchronize()
         self.n_text = t.shape[0]
+        self._grouped = False
+
+    def set_text_groups(self, embs: "list[torch.Tensor]", logit_scale_exp: float):
+        """G instruction sets at once: embs[g] is group g's [n_g, dim] embedding, as set_text takes it. From now on label,
+        label_host, label_file and compute_reward score every group in one encoder pass and return arrays with a leading
+        group axis [G, ...] (also for G = 1); group g equals what the same call returns after set_text(embs[g]).
+        set_text goes back to one group and the plain shapes."""
+        rows = [e.detach().to(self.device, torch.float32) for e in embs]
+        assert rows and all(r.dim() == 2 for r in rows)
+        t = torch.cat(rows).contiguous()
+        off = np.concatenate([[0], np.cumsum([r.shape[0] for r in rows])]).astype(np.int32)
+        self._check(self._lib.arp_set_text_groups(self._h, _ptr(t), t.shape[0], t.shape[1], C.c_void_p(off.ctypes.data),
+                                                  len(rows), float(logit_scale_exp), _stream_ptr(self.device)))
+        torch.cuda.current_stream(self.device).synchronize()
+        self.n_text = t.shape[0]
+        self._grouped = True
+
+    @property
+    def n_groups(self) -> int:
+        """G of the text currently set (1 after set_text)."""
+        return int(self._lib.arp_text_groups(self._h))
+
+    def _lead(self) -> tuple:
+        """leading shape of the per-frame outputs: (G,) after set_text_groups, () after set_text"""
+        return (self.n_groups,) if self._grouped else ()
+
+    def _host_outputs(self, T: int, num_frames: int):
+        lead = self._lead()
+        return (np.empty(lead + (T,), np.float32), np.empty(lead + (T,), np.float32),
+                np.empty(lead + (T, num_frames), np.float32), np.empty(lead + (T, num_frames), np.float32))
 
     # -- hot path ---------------------------------------------------------------------------------
     @staticmethod
@@ -246,20 +282,23 @@ class Engine:
         return T, ob.data_ptr(), frame
 
     def label(self, ob: torch.Tensor, ep_offsets: torch.Tensor, num_frames: int):
-        """Device tensors in, device tensors out: (reward[T], rtg[T], reward_stacked[T,F], rtg_stacked[T,F])."""
+        """Device tensors in, device tensors out: (reward[T], rtg[T], reward_stacked[T,F], rtg_stacked[T,F]), each with a
+        leading group axis [G, ...] after set_text_groups."""
         T, p, stride = self._frames_view(ob)
         off = ep_offsets.to(self.device, torch.int64).contiguous()
         n_eps = off.numel() - 1
-        r = torch.empty(T, device=self.device, dtype=torch.float32)
-        g = torch.empty(T, device=self.device, dtype=torch.float32)
-        rs = torch.empty(T, num_frames, device=self.device, dtype=torch.float32)
-        gs = torch.empty(T, num_frames, device=self.device, dtype=torch.float32)
+        lead = self._lead()
+        r = torch.empty(lead + (T,), device=self.device, dtype=torch.float32)
+        g = torch.empty(lead + (T,), device=self.device, dtype=torch.float32)
+        rs = torch.empty(lead + (T, num_frames), device=self.device, dtype=torch.float32)
+        gs = torch.empty(lead + (T, num_frames), device=self.device, dtype=torch.float32)
         self._check(self._lib.arp_label(self._h, C.c_void_p(p), T, stride, _ptr(off), n_eps, num_frames, _ptr(r),
                                         _ptr(g), _ptr(rs), _ptr(gs), _stream_ptr(self.device)))
         return r, g, rs, gs
 
     def label_host(self, ob: "np.ndarray | torch.Tensor", ep_offsets: np.ndarray, num_frames: int, out=None):
-        """Host buffers in/out (numpy or CPU torch, ideally pinned). Blocks until the results are on the host."""
+        """Host buffers in/out (numpy or CPU torch, ideally pinned). Blocks until the results are on the host. Shapes as for
+        label (a leading group axis after set_text_groups); `out`, when given, must have them."""
         if isinstance(ob, np.ndarray):
             assert ob.dtype == np.uint8 and ob.flags.c_contiguous and ob.ndim in (4, 5)
             base, shape = ob.ctypes.data, ob.shape
@@ -274,8 +313,7 @@ class Engine:
             p, stride = base, frame
         off = np.ascontiguousarray(ep_offsets, dtype=np.int64)
         if out is None:
-            out = (np.empty(T, np.float32), np.empty(T, np.float32), np.empty((T, num_frames), np.float32),
-                   np.empty((T, num_frames), np.float32))
+            out = self._host_outputs(T, num_frames)
 
         def hp(a):
             return C.c_void_p(a.ctypes.data if isinstance(a, np.ndarray) else a.data_ptr())
@@ -290,8 +328,7 @@ class Engine:
         """arp_label_file: like label_host, the scored frame of row t read from `fd` at file_offset + t*row_stride_bytes."""
         off = np.ascontiguousarray(ep_offsets, dtype=np.int64)
         if out is None:
-            out = (np.empty(T, np.float32), np.empty(T, np.float32), np.empty((T, num_frames), np.float32),
-                   np.empty((T, num_frames), np.float32))
+            out = self._host_outputs(T, num_frames)
         hp = lambda a: C.c_void_p(a.ctypes.data)  # noqa: E731
         self._check(self._lib.arp_label_file(self._h, int(fd), int(file_offset), int(T), int(row_stride_bytes),
                                              C.c_void_p(off.ctypes.data), off.size - 1, num_frames, hp(out[0]), hp(out[1]),
@@ -299,8 +336,9 @@ class Engine:
         return out
 
     def compute_reward(self, ob: torch.Tensor, want_logits: bool = False):
+        """reward [T] (or [G, T] after set_text_groups); logits [T, n_text] over the texts of all groups."""
         T, p, stride = self._frames_view(ob)
-        r = torch.empty(T, device=self.device, dtype=torch.float32)
+        r = torch.empty(self._lead() + (T,), device=self.device, dtype=torch.float32)
         lg = torch.empty(T, max(self.n_text, 1), device=self.device, dtype=torch.float32) if want_logits else None
         self._check(self._lib.arp_compute_reward(self._h, C.c_void_p(p), T, stride, _ptr(r), _ptr(lg),
                                                  _stream_ptr(self.device)))

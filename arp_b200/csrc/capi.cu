@@ -35,6 +35,8 @@
 #include "scan.cuh"
 
 using namespace arp;
+static_assert(ARP_MAX_TEXT == HEAD_MAX_TEXT && ARP_MAX_TEXT_GROUPS == HEAD_MAX_GROUPS &&
+              ARP_MAX_TEXT_TOTAL == HEAD_MAX_TEXT_TOTAL, "text limits of include/arp_b200.h and head.cuh disagree");
 typedef arp::op_t bf16;   // the operand format (common.cuh: bf16 by default, fp16 with -DARP_OP_FP16=1)
 #define ARP_OP_DTYPE (ARP_OP_FP16 ? ARP_F16 : ARP_BF16)   // ... as an ArpDType of include/arp_b200.h
 
@@ -138,9 +140,11 @@ struct ArpHandle {
   bool finalized = false;
   std::map<std::string, WeightSlot> slots;
 
-  // text
-  float* text = nullptr;
-  int n_text = 0, text_dim = 0;
+  // text: n_text rows = n_groups instruction sets concatenated, group g = rows [group_off[g], group_off[g+1])
+  float* text = nullptr;             // [HEAD_MAX_TEXT_TOTAL, feat_dim]
+  int* group_off = nullptr;          // device int32 [n_groups + 1]
+  int group_off_host[HEAD_MAX_GROUPS + 1] = {};
+  int n_text = 0, text_dim = 0, n_groups = 1;
   float logit_scale = 0.f;
 
   // decode tables
@@ -762,21 +766,54 @@ static int finalize_weights(ArpHandle* h, cudaStream_t st) {
   return ARP_OK;
 }
 
-extern "C" int arp_set_text(ArpHandle* h, const float* text_emb_dev, int32_t n_text, int32_t dim,
-                            float logit_scale_exp, void* stream) {
-  if (!h || !text_emb_dev) return fail(h, ARP_ERR_INVALID, "null argument");
-  if (n_text < 1 || n_text > HEAD_MAX_TEXT) return fail(h, ARP_ERR_INVALID, "n_text must be in [1,%d]", HEAD_MAX_TEXT);
+// arp_set_text is the one-group case of arp_set_text_groups; only the grouped entry point refuses goal heads
+static int set_text_rows(ArpHandle* h, const float* text_emb_dev, int32_t n_text_total, int32_t dim,
+                         const int32_t* group_offsets_host, int32_t n_groups, float logit_scale_exp, cudaStream_t st) {
+  if (!h || !text_emb_dev || !group_offsets_host) return fail(h, ARP_ERR_INVALID, "null argument");
+  if (n_groups < 1 || n_groups > HEAD_MAX_GROUPS)
+    return fail(h, ARP_ERR_INVALID, "n_groups must be in [1,%d], got %d", HEAD_MAX_GROUPS, n_groups);
+  if (n_text_total < 1 || n_text_total > HEAD_MAX_TEXT_TOTAL)
+    return fail(h, ARP_ERR_INVALID, "n_text_total must be in [1,%d], got %d", HEAD_MAX_TEXT_TOTAL, n_text_total);
+  if (group_offsets_host[0] != 0 || group_offsets_host[n_groups] != n_text_total)
+    return fail(h, ARP_ERR_INVALID, "group offsets must run from 0 to n_text_total=%d", n_text_total);
+  for (int g = 0; g < n_groups; ++g) {
+    const int n = group_offsets_host[g + 1] - group_offsets_host[g];
+    if (n < 1 || n > HEAD_MAX_TEXT)
+      return fail(h, ARP_ERR_INVALID, "group %d has %d texts, must be in [1,%d]", g, n, HEAD_MAX_TEXT);
+  }
   if (dim != h->feat_dim) return fail(h, ARP_ERR_INVALID, "text dim %d, head expects %d", dim, h->feat_dim);
   ARP_CUDA(h, cudaSetDevice(h->cfg.device));
-  if (!h->text) ARP_TRY(dev_alloc(h, &h->text, (size_t)HEAD_MAX_TEXT * h->feat_dim));
-  ARP_CUDA(h, cudaMemcpyAsync(h->text, text_emb_dev, (size_t)n_text * dim * 4, cudaMemcpyDeviceToDevice,
-                              static_cast<cudaStream_t>(stream)));
-  h->n_text = n_text;
+  if (!h->text) ARP_TRY(dev_alloc(h, &h->text, (size_t)HEAD_MAX_TEXT_TOTAL * h->feat_dim));
+  if (!h->group_off) ARP_TRY(dev_alloc(h, &h->group_off, (size_t)HEAD_MAX_GROUPS + 1));
+  // the handle keeps the host copy: the H2D source stays valid whenever the copy runs
+  std::copy(group_offsets_host, group_offsets_host + n_groups + 1, h->group_off_host);
+  ARP_CUDA(h, cudaMemcpyAsync(h->text, text_emb_dev, (size_t)n_text_total * dim * 4, cudaMemcpyDeviceToDevice, st));
+  ARP_CUDA(h, cudaMemcpyAsync(h->group_off, h->group_off_host, (size_t)(n_groups + 1) * 4, cudaMemcpyHostToDevice, st));
+  h->n_text = n_text_total;
+  h->n_groups = n_groups;
   h->text_dim = dim;
   h->logit_scale = logit_scale_exp;
   h->online_epoch++;
   return ARP_OK;
 }
+
+extern "C" int arp_set_text_groups(ArpHandle* h, const float* text_emb_dev, int32_t n_text_total, int32_t dim,
+                                   const int32_t* group_offsets_host, int32_t n_groups, float logit_scale_exp,
+                                   void* stream) {
+  if (h && h->goal) return fail(h, ARP_ERR_INVALID, "goal-conditioned heads take no text");
+  return set_text_rows(h, text_emb_dev, n_text_total, dim, group_offsets_host, n_groups, logit_scale_exp,
+                       static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int arp_set_text(ArpHandle* h, const float* text_emb_dev, int32_t n_text, int32_t dim, float logit_scale_exp,
+                            void* stream) {
+  if (h && (n_text < 1 || n_text > HEAD_MAX_TEXT))
+    return fail(h, ARP_ERR_INVALID, "n_text must be in [1,%d]", HEAD_MAX_TEXT);
+  const int32_t off[2] = {0, n_text};
+  return set_text_rows(h, text_emb_dev, n_text, dim, off, 1, logit_scale_exp, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int arp_text_groups(const ArpHandle* h) { return h ? h->n_groups : 0; }
 
 // ------------------------------------------------------------------------------------------------
 // launch helpers
@@ -1252,8 +1289,9 @@ static int encode_chunk_f32(ArpHandle* h, const uint8_t* ob, int64_t n, int64_t 
   return ARP_OK;
 }
 
-// heads. reward_out [n] / logits_out [n, n_text] / feat_out [n, feat_dim] may each be null.
-static int head_chunk(ArpHandle* h, int64_t n, float* reward_out, float* logits_out, float* feat_out,
+// heads. reward_out [n_groups, ld] (this chunk's column 0; ld = the call's T) / logits_out [n, n_text] /
+// feat_out [n, feat_dim] may each be null.
+static int head_chunk(ArpHandle* h, int64_t n, float* reward_out, int64_t ld, float* logits_out, float* feat_out,
                       cudaStream_t st) {
   const ArpConfig& c = h->cfg;
   ArpHandle::Work& ws = h->ws;
@@ -1265,15 +1303,16 @@ static int head_chunk(ArpHandle* h, int64_t n, float* reward_out, float* logits_
     ProfScope prof(h, PC_HEAD, 2.0 * (double)n * 768 * 512, (double)n * 768 * 4 + 768.0 * 512 * 4, st);
     clip_head_kernel<768, 512><<<(unsigned)((n + HEAD_FR - 1) / HEAD_FR), 256, HEAD_SMEM_BYTES, st>>>(
         xsrc, xtok, h->ln_post_g, h->ln_post_b, 1e-5f, h->proj, (need_text && !h->goal) ? h->text : nullptr,
-        h->n_text, h->logit_scale, c.reduce, feat_out, c.embed_dim, 0, logits_out, h->goal ? nullptr : reward_out, (int)n);
+        h->n_text, h->group_off, h->n_groups, h->logit_scale, c.reduce, feat_out, c.embed_dim, 0, logits_out,
+        h->goal ? nullptr : reward_out, ld, (int)n);
     h->launches++;
   } else {
     const int D = h->feat_dim, Dmid = c.layers * c.embed_dim, Din = c.layers * c.width;
     const int64_t B = c.max_batch;
     // final CLIP feature -> last 512 columns of feat (un-normalised, clip_multiscale_adapter.py:136,145)
     clip_head_kernel<768, 512><<<(unsigned)((n + HEAD_FR - 1) / HEAD_FR), 256, HEAD_SMEM_BYTES, st>>>(
-        xsrc, xtok, h->ln_post_g, h->ln_post_b, 1e-5f, h->proj, nullptr, 0, 0.f, 0, ws.featf, D, Dmid, nullptr, nullptr,
-        (int)n);
+        xsrc, xtok, h->ln_post_g, h->ln_post_b, 1e-5f, h->proj, nullptr, 0, nullptr, 0, 0.f, 0, ws.featf, D, Dmid,
+        nullptr, nullptr, 0, (int)n);
     h->launches++;
     if (h->f32) {
       ARP_TRY(launch_sgemm(h, ws.taps32, Din, h->inter_w, ws.featf, D, F32_ACT_NONE, n, Dmid, Din, nullptr, nullptr, 0,
@@ -1297,8 +1336,8 @@ static int head_chunk(ArpHandle* h, int64_t n, float* reward_out, float* logits_
     const bool ens = c.head == ARP_HEAD_ADAPTER_ENSEMBLE;
     adapter_head_kernel<13, 512><<<(unsigned)n, 13 * 32, 0, st>>>(
         ws.featf, ws.mlp, h->res_sigmoid, (need_text && !h->goal) ? h->text : nullptr,
-        (need_text && !h->goal) ? h->n_text : 0, h->logit_scale, ens ? 1 : 0, c.reduce, logits_out,
-        h->goal ? nullptr : reward_out, feat_out);
+        (need_text && !h->goal) ? h->n_text : 0, h->group_off, (need_text && !h->goal) ? h->n_groups : 0,
+        h->logit_scale, ens ? 1 : 0, c.reduce, logits_out, h->goal ? nullptr : reward_out, ld, feat_out);
     h->launches++;
   }
   ARP_CUDA(h, cudaGetLastError());
@@ -1335,15 +1374,15 @@ static int ensure_scratch(ArpHandle* h, int slot, size_t bytes) {
 
 // temporaries of one label call, carved from scratch slot 0
 struct LabelTmp {
-  float* r = nullptr;            // [T] rewards when the caller did not ask for them
-  float* g = nullptr;            // [T] return-to-go, likewise
+  float* r = nullptr;            // [n_groups, T] rewards when the caller did not ask for them
+  float* g = nullptr;            // [n_groups, T] return-to-go, likewise
   long long* frame_goal = nullptr;  // [T] goal-conditioned heads: index of the episode's last frame
   float* feats = nullptr;        // [T, feat_dim] goal-conditioned heads
 };
 
 static int carve_label_tmp(ArpHandle* h, int64_t T, LabelTmp* t) {
   auto al = [](size_t b) { return (b + 255) & ~static_cast<size_t>(255); };
-  const size_t b_r = al((size_t)T * 4), b_goal = h->goal ? al((size_t)T * 8) : 0;
+  const size_t b_r = al((size_t)h->n_groups * T * 4), b_goal = h->goal ? al((size_t)T * 8) : 0;
   const size_t b_feat = h->goal ? al((size_t)T * h->feat_dim * 4) : 0;
   ARP_TRY(ensure_scratch(h, 0, 2 * b_r + b_goal + b_feat + 256));
   uint8_t* p = reinterpret_cast<uint8_t*>(h->scratch[0]);
@@ -1376,7 +1415,7 @@ extern "C" int arp_compute_reward(ArpHandle* h, const uint8_t* ob_dev, int64_t T
   for (int64_t t0 = 0; t0 < T; t0 += B) {
     const int64_t n = std::min(B, T - t0);
     ARP_TRY(encode_chunk(h, ob_dev + t0 * row_stride_bytes, n, row_stride_bytes, st));
-    ARP_TRY(head_chunk(h, n, reward_dev ? reward_dev + t0 : nullptr,
+    ARP_TRY(head_chunk(h, n, reward_dev ? reward_dev + t0 : nullptr, T,
                        logits_dev ? logits_dev + t0 * h->n_text : nullptr, nullptr, st));
   }
   return ARP_OK;
@@ -1391,7 +1430,7 @@ extern "C" int arp_encode_image(ArpHandle* h, const uint8_t* ob_dev, int64_t T, 
   for (int64_t t0 = 0; t0 < T; t0 += B) {
     const int64_t n = std::min(B, T - t0);
     ARP_TRY(encode_chunk(h, ob_dev + t0 * row_stride_bytes, n, row_stride_bytes, st));
-    ARP_TRY(head_chunk(h, n, nullptr, nullptr, feat_dev + t0 * h->feat_dim, st));
+    ARP_TRY(head_chunk(h, n, nullptr, 0, nullptr, feat_dev + t0 * h->feat_dim, st));
   }
   if (h->adapter && T > 0) {
     l2_normalize_rows_kernel<<<(unsigned)((T + 7) / 8), 256, 0, st>>>(feat_dev, h->feat_dim, T);
@@ -1413,19 +1452,20 @@ extern "C" int arp_encode_taps_chw(ArpHandle* h, const float* chw_dev, int64_t T
   for (int64_t t0 = 0; t0 < T; t0 += B) {
     const int64_t n = std::min(B, T - t0);
     ARP_TRY(encode_chunk(h, nullptr, n, 0, st, chw_dev + t0 * img, taps_dev ? taps_dev + t0 * tw : nullptr));
-    if (feat_dev) ARP_TRY(head_chunk(h, n, nullptr, nullptr, feat_dev + t0 * h->feat_dim, st));
+    if (feat_dev) ARP_TRY(head_chunk(h, n, nullptr, 0, nullptr, feat_dev + t0 * h->feat_dim, st));
   }
   return ARP_OK;
 }
 
+// n_groups reward rows [n_groups, T] over the same episodes -> rtg [n_groups, T], rs / gs [n_groups, T, F]
 static int scan_launch(ArpHandle* h, const float* reward, int64_t T, const int64_t* ep_off, int n_eps, int F,
-                       float gamma, float* rtg, float* rs, float* gs, cudaStream_t st) {
+                       float gamma, float* rtg, float* rs, float* gs, cudaStream_t st, int n_groups = 1) {
   if (n_eps <= 0 || T <= 0) return ARP_OK;
   if (F < 1 || F > 64) return fail(h, ARP_ERR_INVALID, "num_frames must be in [1,64]");
   if (gs && !rtg) return fail(h, ARP_ERR_INVALID, "rtg_stacked needs an rtg buffer");
-  ProfScope prof(h, PC_SCAN, 0.0, (double)T * (4 + 4 + 2.0 * F * 4), st);
-  rtg_scan_stack_kernel<<<n_eps, SCAN_THREADS, 0, st>>>(reward, reinterpret_cast<const long long*>(ep_off), T, F,
-                                                       gamma, rtg, rs, gs);
+  ProfScope prof(h, PC_SCAN, 0.0, (double)n_groups * T * (4 + 4 + 2.0 * F * 4), st);
+  rtg_scan_stack_kernel<<<dim3(n_eps, n_groups), SCAN_THREADS, 0, st>>>(
+      reward, reinterpret_cast<const long long*>(ep_off), T, F, gamma, rtg, rs, gs);
   h->launches++;
   ARP_CUDA(h, cudaGetLastError());
   return ARP_OK;
@@ -1483,11 +1523,11 @@ static int label_device(ArpHandle* h, const uint8_t* ob_dev, int64_t T, int64_t 
   for (int64_t t0 = 0; t0 < T; t0 += B) {
     const int64_t n = std::min(B, T - t0);
     ARP_TRY(encode_chunk(h, ob_dev + t0 * stride, n, stride, st));
-    if (!h->goal) ARP_TRY(head_chunk(h, n, r + t0, nullptr, nullptr, st));
-    else ARP_TRY(head_chunk(h, n, nullptr, nullptr, tmp.feats + t0 * h->feat_dim, st));
+    if (!h->goal) ARP_TRY(head_chunk(h, n, r + t0, T, nullptr, nullptr, st));
+    else ARP_TRY(head_chunk(h, n, nullptr, 0, nullptr, tmp.feats + t0 * h->feat_dim, st));
   }
   if (h->goal) ARP_TRY(goal_rewards(h, tmp, T, ep_off, n_eps, r, st));
-  return scan_launch(h, r, T, ep_off, n_eps, F, 1.0f, g, rs, gs, st);
+  return scan_launch(h, r, T, ep_off, n_eps, F, 1.0f, g, rs, gs, st, h->n_groups);
 }
 
 // two device staging buffers of max_batch frames each (host-buffer entry points)
@@ -1610,16 +1650,18 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
   const int64_t B = c.max_batch;
   const int F = num_frames;
   ARP_TRY(ensure_stage(h));
-  // device outputs (scratch slot 1): [ep_off (n_eps+1) i64][reward T][rtg T][reward_stacked T*F][rtg_stacked T*F]
+  // device outputs (scratch slot 1), G = n_groups:
+  // [ep_off (n_eps+1) i64][reward G*T][rtg G*T][reward_stacked G*T*F][rtg_stacked G*T*F]
+  const size_t G = (size_t)h->n_groups;
   const size_t off_bytes = (((size_t)(n_eps + 1) * 8) + 255) & ~(size_t)255;
-  ARP_TRY(ensure_scratch(h, 1, off_bytes + (size_t)T * 4 * (2 + 2 * F) + 1024));
+  ARP_TRY(ensure_scratch(h, 1, off_bytes + G * T * 4 * (2 + 2 * F) + 1024));
   LabelTmp tmp;
   ARP_TRY(carve_label_tmp(h, T, &tmp));
   int64_t* d_off = reinterpret_cast<int64_t*>(h->scratch[1]);
   float* d_r = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(h->scratch[1]) + off_bytes);
-  float* d_g = d_r + T;
-  float* d_rs = d_g + T;
-  float* d_gs = d_rs + (size_t)T * F;
+  float* d_g = d_r + G * T;
+  float* d_rs = d_g + G * T;
+  float* d_gs = d_rs + G * T * F;
   ARP_CUDA(h, cudaMemcpyAsync(d_off, ep_offsets_host, (size_t)(n_eps + 1) * 8, cudaMemcpyHostToDevice, st));
   const int64_t nchunks = (T + B - 1) / B;
   // pinned (or registered) caller memory goes to the device directly, one strided 2-D copy per chunk; pageable memory is
@@ -1663,8 +1705,8 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
     cudaEventRecord(h->ev_copied[buf], h->copy_stream);
     cudaStreamWaitEvent(st, h->ev_copied[buf], 0);
     if ((rc = encode_chunk(h, h->stage_dev[buf], n, (int64_t)frame_bytes, st)) != ARP_OK) break;
-    if (!h->goal) rc = head_chunk(h, n, d_r + t0, nullptr, nullptr, st);
-    else rc = head_chunk(h, n, nullptr, nullptr, tmp.feats + t0 * h->feat_dim, st);
+    if (!h->goal) rc = head_chunk(h, n, d_r + t0, T, nullptr, nullptr, st);
+    else rc = head_chunk(h, n, nullptr, 0, nullptr, tmp.feats + t0 * h->feat_dim, st);
     cudaEventRecord(h->ev_consumed[buf], st);
   }
   if (staged) {
@@ -1677,13 +1719,14 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
               (long long)T, subs.size(), stager.waited_s);
   }
   if (rc == ARP_OK && h->goal) rc = goal_rewards(h, tmp, T, d_off, n_eps, d_r, st);
-  if (rc == ARP_OK) rc = scan_launch(h, d_r, T, d_off, n_eps, F, 1.0f, d_g, d_rs, d_gs, st);
+  if (rc == ARP_OK) rc = scan_launch(h, d_r, T, d_off, n_eps, F, 1.0f, d_g, d_rs, d_gs, st, h->n_groups);
   if (rc == ARP_OK) {
     cudaError_t e = cudaSuccess;
-    if (reward_host && e == cudaSuccess) e = cudaMemcpyAsync(reward_host, d_r, (size_t)T * 4, cudaMemcpyDeviceToHost, st);
-    if (rtg_host && e == cudaSuccess) e = cudaMemcpyAsync(rtg_host, d_g, (size_t)T * 4, cudaMemcpyDeviceToHost, st);
-    if (reward_stacked_host && e == cudaSuccess) e = cudaMemcpyAsync(reward_stacked_host, d_rs, (size_t)T * F * 4, cudaMemcpyDeviceToHost, st);
-    if (rtg_stacked_host && e == cudaSuccess) e = cudaMemcpyAsync(rtg_stacked_host, d_gs, (size_t)T * F * 4, cudaMemcpyDeviceToHost, st);
+    const size_t b1 = G * T * 4, bF = G * T * F * 4;   // group-major: one contiguous block per output
+    if (reward_host && e == cudaSuccess) e = cudaMemcpyAsync(reward_host, d_r, b1, cudaMemcpyDeviceToHost, st);
+    if (rtg_host && e == cudaSuccess) e = cudaMemcpyAsync(rtg_host, d_g, b1, cudaMemcpyDeviceToHost, st);
+    if (reward_stacked_host && e == cudaSuccess) e = cudaMemcpyAsync(reward_stacked_host, d_rs, bF, cudaMemcpyDeviceToHost, st);
+    if (rtg_stacked_host && e == cudaSuccess) e = cudaMemcpyAsync(rtg_stacked_host, d_gs, bF, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) rc = fail(h, ARP_ERR_CUDA, "label_host tail failed: %s", cudaGetErrorString(e));
   }
@@ -1818,6 +1861,9 @@ extern "C" int arp_online_reward(ArpHandle* h, const uint8_t* ob_host, int32_t n
   ARP_TRY(check_ready(h, ob_host, n, (int64_t)frame_bytes, st));
   const bool text_head = !h->goal;
   if (text_head && !h->text) return fail(h, ARP_ERR_STATE, "arp_set_text has not been called");
+  if (h->n_groups > 1)
+    return fail(h, ARP_ERR_INVALID, "the online reward scores one instruction set: call arp_set_text (%d groups are set)",
+                h->n_groups);
   if (!text_head && (reward_host || logits_host))
     return fail(h, ARP_ERR_INVALID, "goal-conditioned heads produce features only (reward = -||f - f_goal||, vl_reward.py:26-41)");
   ARP_TRY(ensure_stage(h));
@@ -1828,7 +1874,7 @@ extern "C" int arp_online_reward(ArpHandle* h, const uint8_t* ob_host, int32_t n
   float* d_f = d_lg + (size_t)c.max_batch * HEAD_MAX_TEXT;
   auto run = [&]() -> int {
     ARP_TRY(encode_chunk(h, h->stage_dev[0], n, (int64_t)frame_bytes, st));
-    ARP_TRY(head_chunk(h, n, text_head ? d_r : nullptr, text_head ? d_lg : nullptr, d_f, st));
+    ARP_TRY(head_chunk(h, n, text_head ? d_r : nullptr, n, text_head ? d_lg : nullptr, d_f, st));
     if (h->adapter) {
       l2_normalize_rows_kernel<<<(unsigned)((n + 7) / 8), 256, 0, st>>>(d_f, h->feat_dim, n);
       h->launches++;

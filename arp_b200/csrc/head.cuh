@@ -9,6 +9,11 @@
 //  Text embeddings arrive already L2-normalised (cached once per run; the reference re-runs the
 //  text tower every episode, label_reward.py:135-138). All n_text cosines are produced; `reduce`
 //  picks row 0 (what the reference actually does — SURVEY.md Q1) or the mean.
+//  Text groups: the n_text rows are the concatenation of G instruction sets, group g = rows
+//  [group_off[g], group_off[g+1]), and each group is reduced on its own into reward[g * ld + frame]. A group's
+//  reward is bit-identical to a call with that group's rows alone: every cosine is a warp dot product whose order does
+//  not depend on the text's index, and `reduce` accumulates in text order from the group's first row, then divides by
+//  the group size.
 // fp32 throughout: these are a few hundred KFLOP per frame, L2-resident weights.
 #pragma once
 
@@ -16,7 +21,9 @@
 
 namespace arp {
 
-constexpr int HEAD_MAX_TEXT = 16;
+constexpr int HEAD_MAX_TEXT = 16;         // texts of one group
+constexpr int HEAD_MAX_GROUPS = 16;       // groups of one call
+constexpr int HEAD_MAX_TEXT_TOTAL = 64;   // texts of all groups together
 enum HeadReduce : int { REDUCE_FIRST = 0, REDUCE_MEAN = 1 };
 
 template <int NT>
@@ -37,9 +44,10 @@ __device__ __forceinline__ float block_sum(float v, float* scratch) {
 // FR class-token rows (with one frame per CTA the 1.5 MB matrix was re-read from L2 by every CTA).
 //   x        fp32 [B*tokens, W]   residual stream after the last block (row b*tokens = class token)
 //   proj     fp32 [W, E]
-//   text     fp32 [n_text, E] unit rows (may be null when only features are wanted)
+//   text     fp32 [n_text, E] unit rows of all groups (may be null when only features are wanted)
+//   group_off int32 [n_groups + 1] row offsets of the groups into text
 //   feat_out fp32 [B, ld_feat] : un-normalised f written at column feat_col0 (adapter / goal modes) or null
-//   logits   fp32 [B, n_text] or null ; reward fp32 [B] or null
+//   logits   fp32 [B, n_text] or null ; reward fp32 [n_groups, ld] (group-major, frame b at column b) or null
 constexpr int HEAD_FR = 4;
 constexpr int HEAD_SMEM_BYTES = 8 * HEAD_FR * 512 * 4;   // dynamic: the per-warp partial outputs of clip_head_kernel
 
@@ -47,15 +55,15 @@ template <int W, int E>
 __global__ void __launch_bounds__(256)
 clip_head_kernel(const float* __restrict__ x, int tokens, const float* __restrict__ ln_g,
                  const float* __restrict__ ln_b, float eps, const float* __restrict__ proj,
-                 const float* __restrict__ text, int n_text, float scale, int reduce,
-                 float* __restrict__ feat_out, int ld_feat, int feat_col0, float* __restrict__ logits,
-                 float* __restrict__ reward, int n_frames) {
+                 const float* __restrict__ text, int n_text, const int* __restrict__ group_off, int n_groups,
+                 float scale, int reduce, float* __restrict__ feat_out, int ld_feat, int feat_col0,
+                 float* __restrict__ logits, float* __restrict__ reward, long long ld, int n_frames) {
   static_assert(W % 256 == 0 && E % 256 == 0, "head widths must be multiples of the CTA size");
   __shared__ float s_f[HEAD_FR][W];
   __shared__ float s_y[HEAD_FR][E];
   __shared__ float s_red[8];
   __shared__ float s_inv[HEAD_FR];
-  __shared__ float s_logit[HEAD_FR][HEAD_MAX_TEXT];
+  __shared__ float s_logit[HEAD_FR][HEAD_MAX_TEXT_TOTAL];
   const int b0 = blockIdx.x * HEAD_FR, tid = threadIdx.x;
   const int nf = min(HEAD_FR, n_frames - b0);
 
@@ -154,25 +162,29 @@ clip_head_kernel(const float* __restrict__ x, int tokens, const float* __restric
     }
   }
   __syncthreads();
-  if (tid < nf && reward) {
-    float r = s_logit[tid][0];
+  if (tid < nf * n_groups && reward) {       // thread -> (group, frame)
+    const int g = tid / nf, f = tid - g * nf;
+    const int t0 = group_off[g], t1 = group_off[g + 1];
+    float r = s_logit[f][t0];
     if (reduce == REDUCE_MEAN) {
-      for (int t = 1; t < n_text; ++t) r += s_logit[tid][t];
-      r /= static_cast<float>(n_text);
+      for (int t = t0 + 1; t < t1; ++t) r += s_logit[f][t];
+      r /= static_cast<float>(t1 - t0);
     }
-    reward[b0 + tid] = r;
+    reward[g * ld + b0 + f] = r;
   }
 }
 
 // Adapter gate + normalise + cosine. One CTA per frame, one warp per 512-wide scale (S warps).
-//   feat, mlp fp32 [B, S*E]; text fp32 [n_text, S*E] (unit over S*E, or per-scale unit when ensemble)
+//   feat, mlp fp32 [B, S*E]; text fp32 [n_text, S*E] (unit over S*E, or per-scale unit when ensemble), the rows of
+//   n_groups groups at group_off as in clip_head_kernel; reward [n_groups, ld]
 template <int S, int E>
 __global__ void __launch_bounds__(S * 32)
 adapter_head_kernel(const float* __restrict__ feat, const float* __restrict__ mlp, float res,
-                    const float* __restrict__ text, int n_text, float scale, int ensemble, int reduce,
-                    float* __restrict__ logits, float* __restrict__ reward, float* __restrict__ adapted_out) {
+                    const float* __restrict__ text, int n_text, const int* __restrict__ group_off, int n_groups,
+                    float scale, int ensemble, int reduce, float* __restrict__ logits, float* __restrict__ reward,
+                    long long ld, float* __restrict__ adapted_out) {
   __shared__ float s_n2[S];
-  __shared__ float s_dot[S][HEAD_MAX_TEXT];
+  __shared__ float s_dot[S][HEAD_MAX_TEXT_TOTAL];
   const int b = blockIdx.x, sidx = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const size_t base = static_cast<size_t>(b) * S * E + static_cast<size_t>(sidx) * E;
   float a[E / 32];
@@ -196,23 +208,26 @@ adapter_head_kernel(const float* __restrict__ feat, const float* __restrict__ ml
   }
   __syncthreads();
   if (threadIdx.x == 0) {
-    float racc = 0.f;
-    const int n_use = reduce == REDUCE_MEAN ? n_text : 1;
-    for (int t = 0; t < n_text; ++t) {
-      float lg;
-      if (ensemble) {
-        float acc = 0.f;
-        for (int s = 0; s < S; ++s) acc += s_dot[s][t] / fmaxf(sqrtf(s_n2[s]), 1e-12f);
-        lg = scale * acc / static_cast<float>(S);
-      } else {
-        float tot = 0.f, d = 0.f;
-        for (int s = 0; s < S; ++s) { tot += s_n2[s]; d += s_dot[s][t]; }
-        lg = scale * (d / fmaxf(sqrtf(tot), 1e-12f));
+    for (int g = 0; g < n_groups; ++g) {
+      const int t0 = group_off[g], t1 = group_off[g + 1];
+      const int n_use = reduce == REDUCE_MEAN ? t1 - t0 : 1;
+      float racc = 0.f;
+      for (int t = t0; t < t1; ++t) {
+        float lg;
+        if (ensemble) {
+          float acc = 0.f;
+          for (int s = 0; s < S; ++s) acc += s_dot[s][t] / fmaxf(sqrtf(s_n2[s]), 1e-12f);
+          lg = scale * acc / static_cast<float>(S);
+        } else {
+          float tot = 0.f, d = 0.f;
+          for (int s = 0; s < S; ++s) { tot += s_n2[s]; d += s_dot[s][t]; }
+          lg = scale * (d / fmaxf(sqrtf(tot), 1e-12f));
+        }
+        if (logits) logits[static_cast<size_t>(b) * n_text + t] = lg;
+        if (t - t0 < n_use) racc += lg;
       }
-      if (logits) logits[static_cast<size_t>(b) * n_text + t] = lg;
-      if (t < n_use) racc += lg;
+      if (reward) reward[g * ld + b] = racc / static_cast<float>(n_use);
     }
-    if (reward) reward[b] = racc / static_cast<float>(n_use);
   }
 }
 

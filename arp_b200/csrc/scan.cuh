@@ -4,7 +4,8 @@
 //   rtg[T-1] = r[T-1];  rtg[t] = r[t] + gamma * rtg[t+1]      strictly right-to-left, fp32, one add per step
 //   out[i, f] = x[max(0, i - (F-1-f))]                         window left-padded with the episode's first value
 // The scan's rounding is observable (SURVEY.md Appendix C), so the adds stay sequential inside an
-// episode — parallelism is across episodes (one CTA each) and across the stacked writes.
+// episode — parallelism is across episodes (one CTA each), across text groups (blockIdx.y: each group's
+// rewards are scanned over the same episodes) and across the stacked writes.
 // __fmul_rn/__fadd_rn forbid FMA contraction: numpy rounds the product before the add.
 #pragma once
 
@@ -15,8 +16,9 @@ namespace arp {
 constexpr int SCAN_THREADS = 128;
 constexpr int SCAN_CHUNK = 2048;  // floats of one episode processed per smem pass
 
-// reward [T] fp32; ep_off [n_eps+1] int64 (episode e = rows [ep_off[e], min(ep_off[e+1], T)));
-// rtg [T] (optional), reward_stacked / rtg_stacked [T,F] (optional).
+// reward [G,T] fp32; ep_off [n_eps+1] int64 (episode e = rows [ep_off[e], min(ep_off[e+1], T)));
+// rtg [G,T] (optional), reward_stacked / rtg_stacked [G,T,F] (optional). Grid (n_eps, G): block (e, g) scans group g's
+// slices of episode e.
 __global__ void __launch_bounds__(SCAN_THREADS)
 rtg_scan_stack_kernel(const float* __restrict__ reward, const long long* __restrict__ ep_off, long long T, int F,
                       float gamma, float* rtg, float* __restrict__ reward_stacked,
@@ -29,6 +31,13 @@ rtg_scan_stack_kernel(const float* __restrict__ reward, const long long* __restr
   const long long hi = min(ep_off[e + 1], T);
   if (hi <= lo) return;
   const int tid = threadIdx.x;
+  {
+    const long long gy = blockIdx.y;
+    reward += gy * T;
+    if (rtg) rtg += gy * T;
+    if (reward_stacked) reward_stacked += gy * T * F;
+    if (rtg_stacked) rtg_stacked += gy * T * F;
+  }
   const float r_first = reward[lo];
 
   // walk the episode from its end in chunks; the running return crosses chunks through s_carry

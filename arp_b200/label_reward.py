@@ -32,6 +32,10 @@ Keyword-only extensions (all optional; defaults reproduce the reference):
     tokenizer        None: openai/CLIP's clip.tokenize (label_reward.py:136) — if the package is missing the call REFUSES
                      unless ARP_ALLOW_STANDIN_TOKENIZER=1; "standin": the deterministic stand-in (random-init experiments
                      only); or a callable(list[str]) -> int tensor [n, 77].
+    extra_instructions  {inst_type: text or list of texts}: more instruction sets labeled in the SAME pass over the frames
+                     (one decode + encoder pass for all of them). Each writes its own dataset pair, named by its inst_type
+                     with the reference's rule ("none" = no suffix), and equal bit for bit to a separate call with that
+                     text and inst_type. Not for goal-conditioned model types (they take no text).
 """
 from __future__ import annotations
 
@@ -95,6 +99,41 @@ def _head_for(model_type: str) -> tuple[int, int]:
     raise ValueError(f"unsupported model_type {model_type!r}: the labeler only defines clip* reward models")
 
 
+def _texts(text) -> list:
+    return list(text) if isinstance(text, (list, tuple)) else [text]
+
+
+def _text_groups(model_type: str, text, extra_instructions) -> list[list]:
+    """The instruction sets of one labeling pass: `text`, then the values of extra_instructions in order. ValueError for
+    sets one pass cannot label: a goal-conditioned head (it takes no text), more sets or texts than the library holds."""
+    groups = [_texts(text)] + [_texts(t) for t in (extra_instructions or {}).values()]
+    if extra_instructions:
+        head, _ = _head_for(model_type)
+        if head in (capi.HEAD_CLIP_GOAL, capi.HEAD_ADAPTER_GOAL):
+            raise ValueError(f"extra_instructions: {model_type!r} is goal-conditioned and takes no instruction")
+        if len(groups) > capi.MAX_TEXT_GROUPS:
+            raise ValueError(f"extra_instructions: {len(groups)} instruction sets, at most {capi.MAX_TEXT_GROUPS}")
+        for g in groups:
+            if not 1 <= len(g) <= capi.MAX_TEXT:
+                raise ValueError(f"extra_instructions: an instruction set has {len(g)} texts, must be 1..{capi.MAX_TEXT}")
+        if sum(len(g) for g in groups) > capi.MAX_TEXT_TOTAL:
+            raise ValueError(f"extra_instructions: {sum(len(g) for g in groups)} texts in all, at most "
+                             f"{capi.MAX_TEXT_TOTAL}")
+    return groups
+
+
+def _target_keys(model_type: str, inst_type: str, extra_instructions) -> list[str]:
+    """[reward, pos_rtg] key pair of every instruction set, in group order (label_reward.py:257-259: inst_type "none"
+    adds no suffix). ValueError when two sets would write the same datasets."""
+    keys = []
+    for it in [inst_type, *(extra_instructions or {})]:
+        pair = [f"{model_type}_reward", f"{model_type}_pos_rtg"]
+        keys += pair if it == "none" else [f"{x}_{it}" for x in pair]
+    if len(set(keys)) != len(keys):
+        raise ValueError(f"extra_instructions: two instruction sets would write the same datasets ({keys})")
+    return keys
+
+
 def _resolve_clip_weights(clip_state_dict, arch: str) -> dict:
     if clip_state_dict is not None:
         return clip_state_dict
@@ -142,9 +181,13 @@ class RewardLabeler:
 
     def __init__(self, model_type: str, text, frame_hw: tuple[int, int], *, model_ckpt_dir=None,
                  clip_state_dict=None, arch: str = "ViT-B/16", use_crop: bool = False, reduce: str = "first",
-                 max_batch: int = 1024, device: int | None = None, precision: str = "16bit", tokenizer=None):
+                 max_batch: int = 1024, device: int | None = None, precision: str = "16bit", tokenizer=None,
+                 extra_instructions: dict | None = None):
+        """extra_instructions: {inst_type: text(s)} scored with `text` in one pass; label_slab / label_file then return
+        arrays with a leading group axis [1 + len(extra_instructions), ...], `text` first."""
         head, pre = _head_for(model_type)
         prec = capi.precision_enum(precision)
+        groups = _text_groups(model_type, text, extra_instructions)
         adapter = head in (capi.HEAD_ADAPTER, capi.HEAD_ADAPTER_ENSEMBLE, capi.HEAD_ADAPTER_GOAL)
         if adapter:
             assert model_ckpt_dir is not None, "specify model_ckpt_dir"  # label_reward.py:174
@@ -171,26 +214,30 @@ class RewardLabeler:
             raise RuntimeError(f"checkpoint lacks {len(missing)} tensors the {model_type} path needs, e.g. {missing[:3]}")
         self.goal = self.engine.goal
         if not self.goal:
-            texts = list(text) if isinstance(text, (list, tuple)) else [text]
-            tokens = resolve_tokenizer(tokenizer)(texts)
-            # the instruction embedding of the previous call is reused when the very same weight tensors (objects and
+            tokenize = resolve_tokenizer(tokenizer)
+            tokens = [tokenize(g) for g in groups]
+            # the instruction embeddings of the previous call are reused when the very same weight tensors (objects and
             # in-place version counters) and token ids come back — the cached handle keeps them referenced
             text_sd = {k: v for k, v in sd.items() if torch.is_tensor(v) and "visual." not in k}
-            sig = (tokens.tolist(), head, [(k, v._version) for k, v in text_sd.items()])
+            sig = ([t.tolist() for t in tokens], head, [(k, v._version) for k, v in text_sd.items()])
             cached = getattr(self.engine, "_text_cache", None)
             if cached is not None and cached[0] == sig and all(cached[1].get(k) is v for k, v in text_sd.items()):
-                emb, scale = cached[2]
+                embs = cached[2]
             else:
+                # the text tower runs once per group, so each group's rows are exactly those of a call with it alone
                 if adapter:
-                    emb, scale = adapter_text_embedding(sd, tokens, dev, ensemble=head == capi.HEAD_ADAPTER_ENSEMBLE)
+                    embs = [adapter_text_embedding(sd, t, dev, ensemble=head == capi.HEAD_ADAPTER_ENSEMBLE) for t in tokens]
                 else:
-                    emb, scale = clip_text_embedding(sd, tokens, dev)
-                self.engine._text_cache = (sig, text_sd, (emb, scale))
-            self.engine.set_text(emb, scale)
+                    embs = [clip_text_embedding(sd, t, dev) for t in tokens]
+                self.engine._text_cache = (sig, text_sd, embs)
+            if extra_instructions:
+                self.engine.set_text_groups([e for e, _ in embs], embs[0][1])
+            else:
+                self.engine.set_text(*embs[0])
 
     def label_slab(self, ob: np.ndarray, ep_offsets: np.ndarray, num_frames: int):
         """ob: host uint8 [T,F,H,W,3] (or [T,H,W,3]); ep_offsets: int64 [n+1] relative to the slab.
-        Returns host (reward[T], rtg[T], reward_stacked[T,F], rtg_stacked[T,F])."""
+        Returns host (reward[T], rtg[T], reward_stacked[T,F], rtg_stacked[T,F]), each [G, ...] with extra_instructions."""
         return self.engine.label_host(ob, ep_offsets, num_frames)
 
     def label_file(self, fd: int, file_offset: int, T: int, row_stride_bytes: int, ep_offsets: np.ndarray, num_frames: int):
@@ -276,7 +323,12 @@ def label_reward(
     distributed=None,
     precision="16bit",
     tokenizer=None,
+    extra_instructions=None,
 ):
+    # instruction sets this pass cannot label are refused before the dataset is opened or an engine is built
+    target_keys = _target_keys(model_type, inst_type, extra_instructions)
+    _text_groups(model_type, text, extra_instructions)
+    n_groups = len(target_keys) // 2
     image_keys = image_keys.split(", ")
     if data_path is None:
         dirname = (
@@ -307,9 +359,6 @@ def label_reward(
         off = np.minimum(np.asarray(g_traj_idx, dtype=np.int64), len_data)  # min(idx[i+1], len_data) (:267)
         shards = partition_episodes(off, world)
         e_lo, e_hi = shards[rank]
-        target_keys = [f"{model_type}_reward", f"{model_type}_pos_rtg"]
-        if inst_type != "none":
-            target_keys = [f"{x}_{inst_type}" for x in target_keys]
         _mark("open + episode index")
         try:
             H, W = g[image_keys[0]].shape[-3:-1]
@@ -317,14 +366,15 @@ def label_reward(
                 print(f"image_size: {g[image_keys[0]].shape[-2]}")  # label_reward.py:104-105
             labeler = RewardLabeler(model_type, text, (int(H), int(W)), model_ckpt_dir=model_ckpt_dir,
                                     clip_state_dict=clip_state_dict, arch=arch, use_crop=use_crop, reduce=reduce,
-                                    max_batch=max_batch, device=device, precision=precision, tokenizer=tokenizer)
+                                    max_batch=max_batch, device=device, precision=precision, tokenizer=tokenizer,
+                                    extra_instructions=extra_instructions)
             _mark("engine + weights + text tower")
             for img_key in image_keys:
                 ds = g[img_key]
                 side = g.get(img_key + SIDECAR_SUFFIX)
                 if side is not None and (side.shape[0] != ds.shape[0] or tuple(side.shape[1:]) != tuple(ds.shape[2:])):
                     side = None                      # stale or foreign sidecar: fall back to the stacked dataset
-                results[img_key] = _label_rows(labeler, ds, side, off, e_lo, e_hi, num_frames, slab_frames)
+                results[img_key] = _label_rows(labeler, ds, side, off, e_lo, e_hi, num_frames, slab_frames, n_groups)
             _mark("label (decode + encoder + head + scan, H2D / D2H)")
         except Exception as e:  # noqa: BLE001 — reported to every rank below, then re-raised
             failure = e
@@ -342,12 +392,12 @@ def label_reward(
         if distributed:
             rows = [int(off[b] - off[a]) for a, b in shards]
             for img_key in image_keys:
-                rs, gs = results[img_key]
-                both = torch.from_numpy(np.stack([rs, gs], axis=1)).to(cdev)  # [n, 2, F]: the path's one collective
+                # [n, 2G, F] (reward, rtg of group 0, then of group 1, ...): the path's one collective
+                both = torch.from_numpy(np.stack(results[img_key], axis=1)).to(cdev)
                 full = gather_rows(both, rows, dst=0)
                 if rank == 0:
                     full = full.cpu().numpy()
-                    results[img_key] = (np.ascontiguousarray(full[:, 0]), np.ascontiguousarray(full[:, 1]))
+                    results[img_key] = [np.ascontiguousarray(full[:, k]) for k in range(full.shape[1])]
     finally:
         if labeler is not None:
             labeler.close()
@@ -370,18 +420,25 @@ def label_reward(
               + f"; total {_t[-1][1] - _t[0][1]:.3f} s", flush=True)
 
 
-def _label_rows(labeler, ds, side, off, e_lo: int, e_hi: int, num_frames: int, slab_frames: int):
-    """(reward_stacked, rtg_stacked) for episodes [e_lo, e_hi). A memory-mapped container is handed to the library in ONE
-    call (a strided pointer into the file mapping; the native stager overlaps page-cache reads, PCIe and compute). A
-    container that has to be read through its API (h5py: chunked, gzip) is read slab by slab on a reader thread, one slab
-    ahead of the GPU."""
-    empty = np.zeros((0, num_frames), np.float64 if labeler.goal else np.float32)
+def _label_rows(labeler, ds, side, off, e_lo: int, e_hi: int, num_frames: int, slab_frames: int, n_groups: int = 1):
+    """[reward_stacked, rtg_stacked] of each of the n_groups instruction sets in turn (2 * n_groups arrays [rows, F]) for
+    episodes [e_lo, e_hi). A memory-mapped container is handed to the library in ONE call (a strided pointer into the file
+    mapping; the native stager overlaps page-cache reads, PCIe and compute). A container that has to be read through its
+    API (h5py: chunked, gzip) is read slab by slab on a reader thread, one slab ahead of the GPU."""
+    empty = np.zeros((n_groups, 0, num_frames), np.float64 if labeler.goal else np.float32)
     lo_all, hi_all = int(off[e_lo]), int(off[e_hi])
+
+    def pairs(rs, gs):
+        return [a for g in range(n_groups) for a in (rs[g], gs[g])]
+
     if hi_all <= lo_all:
-        return empty, empty
+        return pairs(empty, empty)
 
     def finish(r, rs, gs, rel_off):
-        return _goal_float64(r, rel_off, num_frames) if labeler.goal else (rs, gs)
+        """[G, rows, F] whether or not the labeler returned a group axis"""
+        if labeler.goal:
+            rs, gs = _goal_float64(r, rel_off, num_frames)
+        return (rs, gs) if rs.ndim == 3 else (rs[None], gs[None])
 
     src = side if side is not None else ds
     rel = off[e_lo:e_hi + 1] - lo_all
@@ -397,11 +454,11 @@ def _label_rows(labeler, ds, side, off, e_lo: int, e_hi: int, num_frames: int, s
             r, _, rs, gs = labeler.label_file(fd, first, hi_all - lo_all, stride, rel, num_frames)
         finally:
             os.close(fd)
-        return finish(r, rs, gs, rel)
+        return pairs(*finish(r, rs, gs, rel))
     arr = getattr(src, "array", None)
     if arr is not None and arr.flags.c_contiguous:
         r, _, rs, gs = labeler.label_slab(arr[lo_all:hi_all], rel, num_frames)
-        return finish(r, rs, gs, rel)
+        return pairs(*finish(r, rs, gs, rel))
 
     import threading
     slabs = [(a, b) for a, b in _slabs(off, e_lo, e_hi, slab_frames) if off[b] > off[a]]
@@ -430,7 +487,9 @@ def _label_rows(labeler, ds, side, off, e_lo: int, e_hi: int, num_frames: int, s
         rs, gs = finish(r, rs, gs, rel)
         parts_r.append(rs)
         parts_g.append(gs)
-    return (np.concatenate(parts_r) if parts_r else empty), (np.concatenate(parts_g) if parts_g else empty)
+    if not parts_r:
+        return pairs(empty, empty)
+    return pairs(np.concatenate(parts_r, axis=1), np.concatenate(parts_g, axis=1))
 
 
 def _goal_float64(r: np.ndarray, ep_off: np.ndarray, num_frames: int):
@@ -451,7 +510,8 @@ def _goal_float64(r: np.ndarray, ep_off: np.ndarray, num_frames: int):
 
 
 def _write_labels(g, img_key, target_keys, data, off, n_eps, len_data, num_frames):
-    """label_reward.py:260-289. `data` rows are the labeled rows [off[0], off[n_eps]) in order. When the key does not
+    """label_reward.py:260-289, for every (key, array) of target_keys and data (a reward / rtg pair per instruction
+    set). `data` rows are the labeled rows [off[0], off[n_eps]) in order. When the key does not
     exist the reference creates the dataset from the first episode (gzip, chunks (1,F), maxshape (len_data,F)) and
     APPENDS every later episode (:273-286) — one dataset of off[n_eps]-off[0] rows, whatever off[0] is (it is non-zero
     only in the "time" layout, :84-87). When the key exists it assigns in place at the true row indices (:288-289)."""
@@ -491,14 +551,22 @@ def main():
     parser.add_argument("--max_batch", type=int, default=1024)
     parser.add_argument("--precision", type=str, default="16bit", choices=sorted(capi.PRECISIONS))
     parser.add_argument("--tokenizer", type=str, default=None, choices=["clip", "standin"])
+    parser.add_argument("--extra_inst_types", type=str, default=None,
+                        help="comma-separated inst_types labeled in the same pass as --inst_type, e.g. random1,misinfo")
     args = parser.parse_args()
 
     env_name = f"{args.env_name}" if args.env_type == "none" else f"{args.env_name}_{args.env_type}"
-    if args.inst_type != "none":
-        text = get_clip_special_instruct(env_name, args.inst_type)
-    else:
-        text = get_clip_instruct(env_name)
+
+    def instruction(inst_type):
+        return get_clip_instruct(env_name) if inst_type == "none" else get_clip_special_instruct(env_name, inst_type)
+
+    text = instruction(args.inst_type)
     print(f"[INFO] env_name: {env_name}\t instruction: {text}")
+    extra = None
+    if args.extra_inst_types:
+        extra = {t: instruction(t) for t in (x.strip() for x in args.extra_inst_types.split(",")) if t}
+        for t, x in extra.items():
+            print(f"[INFO] inst_type {t}: {x}")
 
     if "RANK" in os.environ and int(os.environ.get("WORLD_SIZE", "1")) > 1:
         import torch.distributed as dist
@@ -511,7 +579,7 @@ def main():
         start_level=args.start_level, num_demonstrations=args.num_demonstrations, num_frames=args.num_frames,
         base_path=args.base_path, model_type=args.model_type, model_ckpt_dir=args.model_ckpt_dir,
         use_crop=args.use_crop, inst_type=args.inst_type, arch=args.arch, reduce=args.reduce,
-        max_batch=args.max_batch, precision=args.precision, tokenizer=args.tokenizer,
+        max_batch=args.max_batch, precision=args.precision, tokenizer=args.tokenizer, extra_instructions=extra,
     )
 
 

@@ -11,6 +11,11 @@
  *     (a cudaStream_t passed as void*; NULL = the legacy default stream);
  *   - return 0 (ARP_OK) or a negative ArpStatus; arp_last_error() gives the message;
  *   - there is NO CPU fallback: without an sm_100 device arp_create fails with ARP_ERR_NO_DEVICE.
+ *
+ * Instruction sets ("text groups"): arp_set_text_groups sets G sets of instruction embeddings at once, and every
+ * labeling call then scores all of them from ONE decode + encoder pass. Outputs become group-major: reward / rtg
+ * [G, T], stacked arrays [G, T, F]; group g's rows are bit-identical to a call after arp_set_text(group g's rows).
+ * arp_set_text is the G = 1 case, and with G = 1 every output has the shape it always had.
  */
 #ifndef ARP_B200_H_
 #define ARP_B200_H_
@@ -21,7 +26,11 @@
 extern "C" {
 #endif
 
-#define ARP_B200_ABI_VERSION 5   /* 3: + arp_encode_taps_chw, 4: + arp_operand_dtype, 5: + ARP_PREC_F32RESID, arp_ln_gemm, arp_resid_gemm_stats, arp_label_file, arp_wants_weight */
+#define ARP_B200_ABI_VERSION 6   /* 3: + arp_encode_taps_chw, 4: + arp_operand_dtype, 5: + ARP_PREC_F32RESID, arp_ln_gemm, arp_resid_gemm_stats, arp_label_file, arp_wants_weight, 6: + arp_set_text_groups, arp_text_groups */
+
+#define ARP_MAX_TEXT 16          /* texts of one instruction set (arp_set_text's n_text, one group's size) */
+#define ARP_MAX_TEXT_GROUPS 16   /* instruction sets of one arp_set_text_groups call */
+#define ARP_MAX_TEXT_TOTAL 64    /* texts of all groups together */
 
 #if defined(__GNUC__)
 #define ARP_API __attribute__((visibility("default")))
@@ -115,11 +124,26 @@ ARP_API int arp_wants_weight(const ArpHandle* h, const char* name);
 ARP_API int arp_missing_weights(const ArpHandle* h, char* names_out, int64_t names_cap);
 
 /* Cached instruction embedding(s): fp32 [n_text, dim] DEVICE rows, already L2-normalised
- * (per 512-wide scale for ARP_HEAD_ADAPTER_ENSEMBLE); dim = 512 (clip) or 6656 (adapter heads).
+ * (per 512-wide scale for ARP_HEAD_ADAPTER_ENSEMBLE); dim = 512 (clip) or 6656 (adapter heads); 1 <= n_text <= ARP_MAX_TEXT.
  * logit_scale_exp = model.logit_scale.exp() (label_reward.py:141, :213-216).
+ * Sets ONE group (arp_text_groups() == 1): the outputs of the calls below are [T] / [T, F].
  * replaces clip.tokenize + encode_text, which the reference re-runs every episode (:135-138). */
 ARP_API int arp_set_text(ArpHandle* h, const float* text_emb_dev, int32_t n_text, int32_t dim, float logit_scale_exp,
                  void* stream);
+/* G instruction sets scored in one pass (the reference relabels the same demonstrations once per inst_type).
+ *   text_emb_dev        fp32 [n_text_total, dim] DEVICE rows of all groups, concatenated, normalised as for arp_set_text
+ *   group_offsets_host  int32 [n_groups + 1] HOST: group g = rows [off[g], off[g+1]); off[0] = 0, off[G] = n_text_total
+ * Each group is reduced on its own (ArpConfig.reduce: its first row or its mean). Limits: 1..ARP_MAX_TEXT_GROUPS groups of
+ * 1..ARP_MAX_TEXT texts, at most ARP_MAX_TEXT_TOTAL in all; ARP_ERR_INVALID otherwise, and for goal-conditioned heads
+ * (they take no text). After it, with G = n_groups:
+ *   arp_label / arp_label_host / arp_label_file   reward, rtg [G, T]; reward_stacked, rtg_stacked [G, T, F]
+ *   arp_compute_reward                            reward [G, T]; logits [T, n_text_total]
+ *   arp_online_reward                             ARP_ERR_INVALID for G > 1
+ * Group g's values are bit-identical to the same call after arp_set_text(group g's rows). arp_set_text resets to G = 1. */
+ARP_API int arp_set_text_groups(ArpHandle* h, const float* text_emb_dev, int32_t n_text_total, int32_t dim,
+                        const int32_t* group_offsets_host, int32_t n_groups, float logit_scale_exp, void* stream);
+/* the current number of text groups G: 1 after arp_set_text (and before any text is set) */
+ARP_API int arp_text_groups(const ArpHandle* h);
 
 /* ------------------------------------------------------------------------------------------------
  * the hot path
@@ -133,13 +157,14 @@ ARP_API int arp_set_text(ArpHandle* h, const float* text_emb_dev, int32_t n_text
  *   reward_dev        fp32 [T] per-frame reward (may be NULL)
  *   rtg_dev           fp32 [T] per-frame return-to-go (may be NULL)
  *   reward_stacked_dev, rtg_stacked_dev   fp32 [T,F] = the two datasets the reference writes (:270-271)
+ * With G text groups (arp_set_text_groups) the four outputs are [G, T] and [G, T, F], group-major.
  */
 ARP_API int arp_label(ArpHandle* h, const uint8_t* ob_dev, int64_t T, int64_t row_stride_bytes,
               const int64_t* ep_offsets_dev, int32_t n_eps, int32_t num_frames, float* reward_dev, float* rtg_dev,
               float* reward_stacked_dev, float* rtg_stacked_dev, void* stream);
 
-/* Same contract with HOST buffers: frames are streamed to the device in chunks on a copy stream, overlapped with
- * compute, and the four outputs are copied back. Pinned (cudaHostAlloc / cudaHostRegister) frames are copied directly;
+/* Same contract with HOST buffers (G groups: [G, T] / [G, T, F] as for arp_label): frames are streamed to the device in
+ * chunks on a copy stream, overlapped with compute, and the four outputs are copied back. Pinned (cudaHostAlloc / cudaHostRegister) frames are copied directly;
  * pageable ones — e.g. a pointer into the memory-mapped dataset itself — are gathered by a few internal worker threads
  * through a ring of pinned slots, so page-cache reads, PCIe and the GPU overlap and ONE call can cover a whole shard.
  * This is the call a drop-in label_reward() makes per image key; it synchronises before returning. */
@@ -151,6 +176,7 @@ ARP_API int arp_label_host(ArpHandle* h, const uint8_t* ob_host, int64_t T, int6
  * file_offset + t*row_stride_bytes of the open descriptor `fd` — an .npy memory-map's backing file, or a contiguous
  * (unchunked, uncompressed) HDF5 dataset at its data offset. The gather threads pread() into the pinned ring, which
  * avoids the page-table work of touching tens of GB through a mapping (faults on the way in, a long munmap on the way out).
+ * Outputs as for arp_label_host ([G, T] / [G, T, F] with G text groups).
  * replaces g[img_key][traj, -1] (label_reward.py:268) for containers whose rows sit contiguously in a file. */
 ARP_API int arp_label_file(ArpHandle* h, int32_t fd, int64_t file_offset, int64_t T, int64_t row_stride_bytes,
                    const int64_t* ep_offsets_host, int32_t n_eps, int32_t num_frames, float* reward_host,
@@ -162,7 +188,8 @@ ARP_API int arp_label_file(ArpHandle* h, int32_t fd, int64_t file_offset, int64_
  * uint8 [n,H,W,3] and returns, each optional: reward [n] (row 0 or the mean over texts, per ArpConfig.reduce),
  * logits [n, n_text], features [n, feat_dim] (CLIP: un-normalised encode_image; adapter heads: normalised).
  * The kernel sequence is captured into a CUDA graph on first use per n; the call synchronises. Goal heads give
- * features only (the caller takes -||f_obs - f_goal||). */
+ * features only (the caller takes -||f_obs - f_goal||). One text group only: ARP_ERR_INVALID after arp_set_text_groups
+ * with G > 1. */
 ARP_API int arp_online_reward(ArpHandle* h, const uint8_t* ob_host, int32_t n, float* reward_host, float* logits_host,
                       float* feat_host);
 
@@ -182,7 +209,8 @@ ARP_API int arp_preprocess_rtgs(ArpHandle* h, const float* reward_dev, int64_t T
 ARP_API int arp_quantile_f32(ArpHandle* h, const float* x_dev, int64_t n, int64_t k_lo, int64_t k_hi, float* lo_hi_host,
                      void* stream);
 
-/* compute_reward only (label_reward.py:132-146 / :200-230): per-frame rewards, optional [T,n_text] logits. */
+/* compute_reward only (label_reward.py:132-146 / :200-230): per-frame rewards [T], optional [T,n_text] logits;
+ * with G text groups reward is [G, T] and logits [T, n_text_total]. */
 ARP_API int arp_compute_reward(ArpHandle* h, const uint8_t* ob_dev, int64_t T, int64_t row_stride_bytes, float* reward_dev,
                        float* logits_dev, void* stream);
 
