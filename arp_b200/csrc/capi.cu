@@ -1,7 +1,8 @@
 // C-ABI implementation of include/arp_b200.h: handle, weight packing, TMA descriptors and the
 // stream-ordered pipeline   decode -> patch-embed GEMM -> ln_pre -> 12 x [QKV (ln_1 folded), attention, out-proj (+= x,
 // row moments), c_fc (ln_2 folded, QuickGELU), c_proj (+= x, row moments)] (the last block for the class-token row only)
-// -> reward head -> per-episode return-to-go scan.
+// -> reward head -> per-episode return-to-go scan. The embed entry points stop after the head's image side and return the
+// per-frame embedding; arp_label_embeddings runs only the instruction side (head + scan) on such embeddings.
 // Host logic only; every kernel lives in the .cuh next to this file.
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -1380,17 +1381,18 @@ struct LabelTmp {
   float* feats = nullptr;        // [T, feat_dim] goal-conditioned heads
 };
 
-static int carve_label_tmp(ArpHandle* h, int64_t T, LabelTmp* t) {
+// with_feats = false: the caller provides the goal heads' features itself (t->feats stays null)
+static int carve_label_tmp(ArpHandle* h, int64_t T, LabelTmp* t, bool with_feats = true) {
   auto al = [](size_t b) { return (b + 255) & ~static_cast<size_t>(255); };
   const size_t b_r = al((size_t)h->n_groups * T * 4), b_goal = h->goal ? al((size_t)T * 8) : 0;
-  const size_t b_feat = h->goal ? al((size_t)T * h->feat_dim * 4) : 0;
+  const size_t b_feat = h->goal && with_feats ? al((size_t)T * h->feat_dim * 4) : 0;
   ARP_TRY(ensure_scratch(h, 0, 2 * b_r + b_goal + b_feat + 256));
   uint8_t* p = reinterpret_cast<uint8_t*>(h->scratch[0]);
   t->r = reinterpret_cast<float*>(p); p += b_r;
   t->g = reinterpret_cast<float*>(p); p += b_r;
   if (h->goal) {
     t->frame_goal = reinterpret_cast<long long*>(p); p += b_goal;
-    t->feats = reinterpret_cast<float*>(p);
+    if (with_feats) t->feats = reinterpret_cast<float*>(p);
   }
   return ARP_OK;
 }
@@ -1635,34 +1637,42 @@ struct HostStager {
   void stop() { abort.store(true); for (auto& t : threads) t.join(); threads.clear(); }
 };
 
+// emb_host != nullptr: embed mode (arp_embed_host / arp_embed_file) — the same staging and encoder pass, the head writes
+// the per-frame embedding [T, feat_dim] (head_chunk's feat_out) to the device, and it is copied to emb_host once at the
+// end; there is no reward, no scan, and the episode / output arguments are ignored.
 static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t fd_offset, int64_t T,
                            int64_t row_stride_bytes, const int64_t* ep_offsets_host, int32_t n_eps, int32_t num_frames,
-                           float* reward_host, float* rtg_host, float* reward_stacked_host, float* rtg_stacked_host) {
+                           float* reward_host, float* rtg_host, float* reward_stacked_host, float* rtg_stacked_host,
+                           float* emb_host = nullptr) {
   if (!h) return ARP_ERR_INVALID;
   cudaStream_t st = h->own_stream;
+  const bool embed = emb_host != nullptr;
   if (fd >= 0 && fd_offset < 0) return fail(h, ARP_ERR_INVALID, "bad file offset");
   ARP_TRY(check_ready(h, fd >= 0 ? reinterpret_cast<const uint8_t*>(h) : ob_host, T, row_stride_bytes, st));
-  if (!ep_offsets_host || n_eps < 0) return fail(h, ARP_ERR_INVALID, "bad episode offsets");
-  if (num_frames < 1 || num_frames > 64) return fail(h, ARP_ERR_INVALID, "num_frames must be in [1,64]");
+  if (!embed && (!ep_offsets_host || n_eps < 0)) return fail(h, ARP_ERR_INVALID, "bad episode offsets");
+  if (!embed && (num_frames < 1 || num_frames > 64)) return fail(h, ARP_ERR_INVALID, "num_frames must be in [1,64]");
   if (T == 0) return ARP_OK;
   const ArpConfig& c = h->cfg;
   const size_t frame_bytes = (size_t)c.in_h * c.in_w * 3;
   const int64_t B = c.max_batch;
-  const int F = num_frames;
+  const int F = embed ? 1 : num_frames;
   ARP_TRY(ensure_stage(h));
   // device outputs (scratch slot 1), G = n_groups:
-  // [ep_off (n_eps+1) i64][reward G*T][rtg G*T][reward_stacked G*T*F][rtg_stacked G*T*F]
+  // [ep_off (n_eps+1) i64][reward G*T][rtg G*T][reward_stacked G*T*F][rtg_stacked G*T*F]; embed mode: [emb T*feat_dim]
   const size_t G = (size_t)h->n_groups;
-  const size_t off_bytes = (((size_t)(n_eps + 1) * 8) + 255) & ~(size_t)255;
-  ARP_TRY(ensure_scratch(h, 1, off_bytes + G * T * 4 * (2 + 2 * F) + 1024));
+  const size_t off_bytes = embed ? 0 : (((size_t)(n_eps + 1) * 8) + 255) & ~(size_t)255;
+  const size_t out_bytes = embed ? (size_t)T * h->feat_dim * 4 : G * T * 4 * (2 + 2 * F);
+  ARP_TRY(ensure_scratch(h, 1, off_bytes + out_bytes + 1024));
   LabelTmp tmp;
-  ARP_TRY(carve_label_tmp(h, T, &tmp));
+  if (!embed) ARP_TRY(carve_label_tmp(h, T, &tmp));
   int64_t* d_off = reinterpret_cast<int64_t*>(h->scratch[1]);
   float* d_r = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(h->scratch[1]) + off_bytes);
   float* d_g = d_r + G * T;
   float* d_rs = d_g + G * T;
   float* d_gs = d_rs + G * T * F;
-  ARP_CUDA(h, cudaMemcpyAsync(d_off, ep_offsets_host, (size_t)(n_eps + 1) * 8, cudaMemcpyHostToDevice, st));
+  float* d_emb = d_r;
+  if (!embed)
+    ARP_CUDA(h, cudaMemcpyAsync(d_off, ep_offsets_host, (size_t)(n_eps + 1) * 8, cudaMemcpyHostToDevice, st));
   const int64_t nchunks = (T + B - 1) / B;
   // pinned (or registered) caller memory goes to the device directly, one strided 2-D copy per chunk; pageable memory is
   // gathered through the pinned ring by worker threads
@@ -1705,7 +1715,8 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
     cudaEventRecord(h->ev_copied[buf], h->copy_stream);
     cudaStreamWaitEvent(st, h->ev_copied[buf], 0);
     if ((rc = encode_chunk(h, h->stage_dev[buf], n, (int64_t)frame_bytes, st)) != ARP_OK) break;
-    if (!h->goal) rc = head_chunk(h, n, d_r + t0, T, nullptr, nullptr, st);
+    if (embed) rc = head_chunk(h, n, nullptr, 0, nullptr, d_emb + t0 * h->feat_dim, st);
+    else if (!h->goal) rc = head_chunk(h, n, d_r + t0, T, nullptr, nullptr, st);
     else rc = head_chunk(h, n, nullptr, 0, nullptr, tmp.feats + t0 * h->feat_dim, st);
     cudaEventRecord(h->ev_consumed[buf], st);
   }
@@ -1718,9 +1729,22 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
       fprintf(stderr, "arp_label_host: %lld frames staged in %zu sub-chunks, consumer waited %.3f s for the gather threads\n",
               (long long)T, subs.size(), stager.waited_s);
   }
-  if (rc == ARP_OK && h->goal) rc = goal_rewards(h, tmp, T, d_off, n_eps, d_r, st);
-  if (rc == ARP_OK) rc = scan_launch(h, d_r, T, d_off, n_eps, F, 1.0f, d_g, d_rs, d_gs, st, h->n_groups);
-  if (rc == ARP_OK) {
+  if (rc == ARP_OK && embed) {
+    cudaError_t e = cudaMemcpyAsync(emb_host, d_emb, (size_t)T * h->feat_dim * 4, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) rc = fail(h, ARP_ERR_CUDA, "embedding D2H failed: %s", cudaGetErrorString(e));
+  }
+  if (embed) {
+    // the [T, feat_dim] device result (1.9 GB for an adapter head at 73 k frames) is not kept by the handle between calls
+    cudaStreamSynchronize(h->copy_stream);
+    cudaStreamSynchronize(st);
+    cudaFree(h->scratch[1]);
+    h->scratch[1] = nullptr;
+    h->scratch_bytes[1] = 0;
+  }
+  if (rc == ARP_OK && !embed && h->goal) rc = goal_rewards(h, tmp, T, d_off, n_eps, d_r, st);
+  if (rc == ARP_OK && !embed) rc = scan_launch(h, d_r, T, d_off, n_eps, F, 1.0f, d_g, d_rs, d_gs, st, h->n_groups);
+  if (rc == ARP_OK && !embed) {
     cudaError_t e = cudaSuccess;
     const size_t b1 = G * T * 4, bF = G * T * F * 4;   // group-major: one contiguous block per output
     if (reward_host && e == cudaSuccess) e = cudaMemcpyAsync(reward_host, d_r, b1, cudaMemcpyDeviceToHost, st);
@@ -1749,6 +1773,71 @@ extern "C" int arp_label_file(ArpHandle* h, int32_t fd, int64_t file_offset, int
   if (fd < 0) return fail(h, ARP_ERR_INVALID, "bad file descriptor");
   return label_host_impl(h, nullptr, fd, file_offset, T, row_stride_bytes, ep_offsets_host, n_eps, num_frames, reward_host,
                          rtg_host, reward_stacked_host, rtg_stacked_host);
+}
+
+// ------------------------------------------------------------------------------------------------
+// C ABI: stored embeddings (relabeling without frames)
+// ------------------------------------------------------------------------------------------------
+extern "C" int arp_embedding_dim(const ArpHandle* h) { return h ? h->feat_dim : 0; }
+
+extern "C" int arp_embed_host(ArpHandle* h, const uint8_t* ob_host, int64_t T, int64_t row_stride_bytes, float* emb_host) {
+  if (!h || T < 0 || (T > 0 && !emb_host)) return fail(h, ARP_ERR_INVALID, "null argument / bad T");
+  if (T == 0) return check_ready(h, ob_host, T, row_stride_bytes, h->own_stream);
+  return label_host_impl(h, ob_host, -1, 0, T, row_stride_bytes, nullptr, 0, 0, nullptr, nullptr, nullptr, nullptr,
+                         emb_host);
+}
+
+extern "C" int arp_embed_file(ArpHandle* h, int32_t fd, int64_t file_offset, int64_t T, int64_t row_stride_bytes,
+                              float* emb_host) {
+  if (fd < 0) return fail(h, ARP_ERR_INVALID, "bad file descriptor");
+  if (!h || T < 0 || (T > 0 && !emb_host)) return fail(h, ARP_ERR_INVALID, "null argument / bad T");
+  if (T == 0) return check_ready(h, reinterpret_cast<const uint8_t*>(h), T, row_stride_bytes, h->own_stream);
+  return label_host_impl(h, nullptr, fd, file_offset, T, row_stride_bytes, nullptr, 0, 0, nullptr, nullptr, nullptr,
+                         nullptr, emb_host);
+}
+
+// The instruction side of arp_label on stored embeddings: no image-side weight is read (finalize_weights is not called,
+// so a handle that never received them works). Text heads: one head launch + one scan launch for any T and G.
+extern "C" int arp_label_embeddings(ArpHandle* h, const float* emb_dev, int64_t T, const int64_t* ep_offsets_dev,
+                                    int32_t n_eps, int32_t num_frames, float* reward_dev, float* rtg_dev,
+                                    float* reward_stacked_dev, float* rtg_stacked_dev, void* stream) {
+  if (!h) return ARP_ERR_INVALID;
+  if (T < 0 || (T > 0 && !emb_dev)) return fail(h, ARP_ERR_INVALID, "bad embedding buffer / T");
+  if (!ep_offsets_dev || n_eps < 0) return fail(h, ARP_ERR_INVALID, "bad episode offsets");
+  if (num_frames < 1 || num_frames > 64) return fail(h, ARP_ERR_INVALID, "num_frames must be in [1,64]");
+  if (!h->goal && !h->text) return fail(h, ARP_ERR_STATE, "arp_set_text has not been called");
+  if (T > 0x7fffffffLL) return fail(h, ARP_ERR_INVALID, "T too large");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  ARP_CUDA(h, cudaSetDevice(h->cfg.device));
+  if (T == 0) return ARP_OK;
+  LabelTmp tmp;
+  // clip_goal_conditioned measures distances on the stored features themselves (goal_rewards only reads them), so no
+  // feature scratch is carved for it; the adapter variant normalises a copy, as the frames path normalises
+  // LabelTmp::feats in place
+  ARP_TRY(carve_label_tmp(h, T, &tmp, h->adapter));
+  float* r = reward_dev ? reward_dev : tmp.r;
+  float* g = rtg_dev ? rtg_dev : tmp.g;
+  if (h->goal) {
+    if (h->adapter)
+      ARP_CUDA(h, cudaMemcpyAsync(tmp.feats, emb_dev, (size_t)T * h->feat_dim * 4, cudaMemcpyDeviceToDevice, st));
+    else
+      tmp.feats = const_cast<float*>(emb_dev);
+    ARP_TRY(goal_rewards(h, tmp, T, ep_offsets_dev, n_eps, r, st));
+  } else if (h->adapter) {
+    ProfScope prof(h, PC_HEAD, 2.0 * (double)T * h->n_text * h->feat_dim, (double)T * h->feat_dim * 4, st);
+    adapter_head_kernel<13, 512><<<(unsigned)T, 13 * 32, 0, st>>>(
+        emb_dev, nullptr, 0.f, h->text, h->n_text, h->group_off, h->n_groups, h->logit_scale,
+        h->cfg.head == ARP_HEAD_ADAPTER_ENSEMBLE ? 1 : 0, h->cfg.reduce, nullptr, r, T, nullptr);
+    h->launches++;
+  } else {
+    ProfScope prof(h, PC_HEAD, 2.0 * (double)T * h->n_text * h->feat_dim, (double)T * h->feat_dim * 4, st);
+    clip_embedding_head_kernel<512><<<(unsigned)((T + HEAD_FR - 1) / HEAD_FR), 256, 0, st>>>(
+        emb_dev, h->text, h->n_text, h->group_off, h->n_groups, h->logit_scale, h->cfg.reduce, nullptr, r, T, T);
+    h->launches++;
+  }
+  ARP_CUDA(h, cudaGetLastError());
+  return scan_launch(h, r, T, ep_offsets_dev, n_eps, num_frames, 1.0f, g, reward_stacked_dev, rtg_stacked_dev, st,
+                     h->n_groups);
 }
 
 extern "C" int arp_wants_weight(const ArpHandle* h, const char* name) {

@@ -14,6 +14,10 @@
 //  reward is bit-identical to a call with that group's rows alone: every cosine is a warp dot product whose order does
 //  not depend on the text's index, and `reduce` accumulates in text order from the group's first row, then divides by
 //  the group size.
+//  Stored embeddings: the per-frame vector the instruction side starts from (clip: f before normalisation; adapter: the
+//  gated a) can be kept and relabeled later without frames or image weights — clip_embedding_head_kernel, and
+//  adapter_head_kernel with mlp == nullptr. They run the same instruction-side code as the frames path, so the rewards
+//  are bit-identical.
 // fp32 throughout: these are a few hundred KFLOP per frame, L2-resident weights.
 #pragma once
 
@@ -40,6 +44,60 @@ __device__ __forceinline__ float block_sum(float v, float* scratch) {
   return t;
 }
 
+constexpr int HEAD_FR = 4;
+constexpr int HEAD_SMEM_BYTES = 8 * HEAD_FR * 512 * 4;   // dynamic: the per-warp partial outputs of clip_head_kernel
+
+// The instruction side of the clip head, shared by clip_head_kernel (features projected from the class-token rows) and
+// clip_embedding_head_kernel (stored features): s_y[f] holds frame b0+f's un-normalised feature (zeros past nf); thread
+// tid owns columns tid + j*256 of every row. Both kernels run this same code, so the same FMA contractions happen and a
+// stored embedding relabels to the bits of the frames path.
+template <int E>
+__device__ __forceinline__ void clip_head_cosines(float (*s_y)[E], float* s_red, float* s_inv,
+                                                  float (*s_logit)[HEAD_MAX_TEXT_TOTAL], int b0, int nf,
+                                                  const float* __restrict__ text, int n_text,
+                                                  const int* __restrict__ group_off, int n_groups, float scale,
+                                                  int reduce, float* __restrict__ logits, float* __restrict__ reward,
+                                                  long long ld) {
+  const int tid = threadIdx.x;
+  if (text == nullptr) return;
+  for (int f = 0; f < HEAD_FR; ++f) {
+    float n2 = 0.f;
+#pragma unroll
+    for (int j = 0; j < E / 256; ++j) {
+      const float yv = s_y[f][tid + j * 256];
+      n2 += yv * yv;
+    }
+    const float tot = block_sum<256>(n2, s_red);
+    if (tid == 0) s_inv[f] = 1.0f / sqrtf(tot);
+  }
+  __syncthreads();
+
+  // cosines: warp w handles (frame, text) pairs w, w+8, ...
+  const int warp = tid >> 5, lane = tid & 31;
+  for (int p = warp; p < nf * n_text; p += 8) {
+    const int f = p / n_text, t = p - f * n_text;
+    float d = 0.f;
+    for (int k = lane; k < E; k += 32) d = fmaf(s_y[f][k], __ldg(text + static_cast<size_t>(t) * E + k), d);
+    d = warp_sum(d);
+    if (lane == 0) {
+      const float lg = scale * (d * s_inv[f]);
+      s_logit[f][t] = lg;
+      if (logits) logits[static_cast<size_t>(b0 + f) * n_text + t] = lg;
+    }
+  }
+  __syncthreads();
+  if (tid < nf * n_groups && reward) {       // thread -> (group, frame)
+    const int g = tid / nf, f = tid - g * nf;
+    const int t0 = group_off[g], t1 = group_off[g + 1];
+    float r = s_logit[f][t0];
+    if (reduce == REDUCE_MEAN) {
+      for (int t = t0 + 1; t < t1; ++t) r += s_logit[f][t];
+      r /= static_cast<float>(t1 - t0);
+    }
+    reward[g * ld + b0 + f] = r;
+  }
+}
+
 // One CTA (256 threads) per FR consecutive frames: the 768x512 projection is streamed once per CTA and applied to all
 // FR class-token rows (with one frame per CTA the 1.5 MB matrix was re-read from L2 by every CTA).
 //   x        fp32 [B*tokens, W]   residual stream after the last block (row b*tokens = class token)
@@ -48,9 +106,6 @@ __device__ __forceinline__ float block_sum(float v, float* scratch) {
 //   group_off int32 [n_groups + 1] row offsets of the groups into text
 //   feat_out fp32 [B, ld_feat] : un-normalised f written at column feat_col0 (adapter / goal modes) or null
 //   logits   fp32 [B, n_text] or null ; reward fp32 [n_groups, ld] (group-major, frame b at column b) or null
-constexpr int HEAD_FR = 4;
-constexpr int HEAD_SMEM_BYTES = 8 * HEAD_FR * 512 * 4;   // dynamic: the per-warp partial outputs of clip_head_kernel
-
 template <int W, int E>
 __global__ void __launch_bounds__(256)
 clip_head_kernel(const float* __restrict__ x, int tokens, const float* __restrict__ ln_g,
@@ -131,7 +186,6 @@ clip_head_kernel(const float* __restrict__ x, int tokens, const float* __restric
   }
   __syncthreads();
   for (int f = 0; f < HEAD_FR; ++f) {
-    float n2 = 0.f;
 #pragma unroll
     for (int j = 0; j < E / 256; ++j) {
       const int col = tid + j * 256;
@@ -139,44 +193,47 @@ clip_head_kernel(const float* __restrict__ x, int tokens, const float* __restric
 #pragma unroll
       for (int w8 = 0; w8 < 8; ++w8) yv += s_part[(static_cast<size_t>(w8) * HEAD_FR + f) * E + col];
       s_y[f][col] = yv;
-      n2 += yv * yv;
       if (feat_out && f < nf) feat_out[static_cast<size_t>(b0 + f) * ld_feat + feat_col0 + col] = yv;
     }
-    const float tot = block_sum<256>(n2, s_red);
-    if (tid == 0) s_inv[f] = 1.0f / sqrtf(tot);
   }
-  if (text == nullptr) return;
-  __syncthreads();
+  clip_head_cosines<E>(s_y, s_red, s_inv, s_logit, b0, nf, text, n_text, group_off, n_groups, scale, reduce, logits,
+                       reward, ld);
+}
 
-  // cosines: warp w handles (frame, text) pairs w, w+8, ...
-  const int warp = tid >> 5, lane = tid & 31;
-  for (int p = warp; p < nf * n_text; p += 8) {
-    const int f = p / n_text, t = p - f * n_text;
-    float d = 0.f;
-    for (int k = lane; k < E; k += 32) d = fmaf(s_y[f][k], __ldg(text + static_cast<size_t>(t) * E + k), d);
-    d = warp_sum(d);
-    if (lane == 0) {
-      const float lg = scale * (d * s_inv[f]);
-      s_logit[f][t] = lg;
-      if (logits) logits[static_cast<size_t>(b0 + f) * n_text + t] = lg;
+// The clip head from stored features: emb fp32 [n_frames, E], row b = frame b's un-normalised encode_image (what
+// clip_head_kernel writes to feat_out). Same CTA shape, same thread -> column map and the same clip_head_cosines, so
+// reward / logits are bit-identical to clip_head_kernel's on the frames the features came from. Memory-bound: E*4 bytes
+// read per frame, no weights.
+template <int E>
+__global__ void __launch_bounds__(256)
+clip_embedding_head_kernel(const float* __restrict__ emb, const float* __restrict__ text, int n_text,
+                           const int* __restrict__ group_off, int n_groups, float scale, int reduce,
+                           float* __restrict__ logits, float* __restrict__ reward, long long ld, long long n_frames) {
+  static_assert(E % 256 == 0, "head widths must be multiples of the CTA size");
+  __shared__ float s_y[HEAD_FR][E];
+  __shared__ float s_red[8];
+  __shared__ float s_inv[HEAD_FR];
+  __shared__ float s_logit[HEAD_FR][HEAD_MAX_TEXT_TOTAL];
+  const long long b0l = static_cast<long long>(blockIdx.x) * HEAD_FR;
+  const int tid = threadIdx.x;
+  const int nf = static_cast<int>(min(static_cast<long long>(HEAD_FR), n_frames - b0l));
+  const float* src = emb + b0l * E;
+  for (int f = 0; f < HEAD_FR; ++f)
+#pragma unroll
+    for (int j = 0; j < E / 256; ++j) {
+      const int col = tid + j * 256;
+      s_y[f][col] = f < nf ? __ldg(src + static_cast<size_t>(f) * E + col) : 0.f;
     }
-  }
-  __syncthreads();
-  if (tid < nf * n_groups && reward) {       // thread -> (group, frame)
-    const int g = tid / nf, f = tid - g * nf;
-    const int t0 = group_off[g], t1 = group_off[g + 1];
-    float r = s_logit[f][t0];
-    if (reduce == REDUCE_MEAN) {
-      for (int t = t0 + 1; t < t1; ++t) r += s_logit[f][t];
-      r /= static_cast<float>(t1 - t0);
-    }
-    reward[g * ld + b0 + f] = r;
-  }
+  // reward / logits are addressed relative to b0: shift the bases so the shared code sees frame 0 at b0l
+  clip_head_cosines<E>(s_y, s_red, s_inv, s_logit, 0, nf, text, n_text, group_off, n_groups, scale, reduce,
+                       logits ? logits + b0l * n_text : nullptr, reward ? reward + b0l : nullptr, ld);
 }
 
 // Adapter gate + normalise + cosine. One CTA per frame, one warp per 512-wide scale (S warps).
 //   feat, mlp fp32 [B, S*E]; text fp32 [n_text, S*E] (unit over S*E, or per-scale unit when ensemble), the rows of
 //   n_groups groups at group_off as in clip_head_kernel; reward [n_groups, ld]
+//   mlp == nullptr: `feat` already holds the gated feature a (what adapted_out receives; a stored embedding), and the
+//   per-scale norms, dots and reductions below run on it unchanged, so relabeling it gives the frames path's bits.
 template <int S, int E>
 __global__ void __launch_bounds__(S * 32)
 adapter_head_kernel(const float* __restrict__ feat, const float* __restrict__ mlp, float res,
@@ -192,7 +249,7 @@ adapter_head_kernel(const float* __restrict__ feat, const float* __restrict__ ml
 #pragma unroll
   for (int i = 0; i < E / 32; ++i) {
     const int c = lane + i * 32;
-    a[i] = res * feat[base + c] + (1.0f - res) * mlp[base + c];
+    a[i] = mlp ? res * feat[base + c] + (1.0f - res) * mlp[base + c] : feat[base + c];
     n2 += a[i] * a[i];
     if (adapted_out) adapted_out[base + c] = a[i];
   }

@@ -36,10 +36,16 @@ Keyword-only extensions (all optional; defaults reproduce the reference):
                      (one decode + encoder pass for all of them). Each writes its own dataset pair, named by its inst_type
                      with the reference's rule ("none" = no suffix), and equal bit for bit to a separate call with that
                      text and inst_type. Not for goal-conditioned model types (they take no text).
+    embeddings       None (default): label from the frames. "save": run the image side once, store the per-frame
+                     embeddings, and label from them (same reward / pos_rtg datasets, bit for bit, plus the embedding
+                     dataset). "load": label from stored embeddings; no frame is read and no image-side weight is
+                     uploaded. See label_reward().
 """
 from __future__ import annotations
 
 import argparse
+import hashlib
+import json
 import os
 
 import numpy as np
@@ -134,6 +140,63 @@ def _target_keys(model_type: str, inst_type: str, extra_instructions) -> list[st
     return keys
 
 
+def embedding_family(model_type: str) -> str:
+    """"clip" (clip, clip_goal_conditioned: the 512-wide encode_image) or "clip_adapter" (every adapter model type: the
+    13*512-wide gated adapter feature). One stored embedding serves every model type of its family."""
+    head, _ = _head_for(model_type)
+    return "clip" if head in (capi.HEAD_CLIP, capi.HEAD_CLIP_GOAL) else "clip_adapter"
+
+
+EMBEDDING_DIM = {"clip": 512, "clip_adapter": 13 * 512}
+
+
+def embedding_key(img_key: str, model_type: str) -> str:
+    """Dataset of the stored embeddings of img_key: f"{img_key}_clip_emb" or f"{img_key}_clip_adapter_emb"; its SHA-256
+    provenance signature is the uint8 [32] dataset f"{key}_sig"."""
+    return f"{img_key}_{embedding_family(model_type)}_emb"
+
+
+_IMAGE_ADAPTER_PREFIXES = ("image_intermediate_linear.", "image_adapter.", "image_residual_weight")
+
+
+def _image_weights(state_dict: dict, adapter: bool) -> dict:
+    """The image-side tensors Engine.load_state_dict uploads for a head of this family, by their library names ("visual.*"
+    and, for the adapter heads, the image adapter; an adapter checkpoint's "clip_model." prefix removed)."""
+    out = {}
+    for k, v in state_dict.items():
+        if not torch.is_tensor(v):
+            continue
+        name = k[len("clip_model."):] if k.startswith("clip_model.") else k
+        if name.startswith("visual.") or (adapter and name.startswith(_IMAGE_ADAPTER_PREFIXES)):
+            out[name] = v
+    return out
+
+
+SIGNATURE_SAMPLES = 4096
+
+
+def embedding_signature(model_type: str, arch: str, frame_hw, use_crop: bool, precision: str,
+                        state_dict: dict) -> np.ndarray:
+    """uint8 [32]: SHA-256 over what decides a stored embedding's bits — the embedding family, arch, frame H x W,
+    use_crop, the precision's pipeline, the library's operand format, and a digest of the image-side weights: every tensor
+    Engine.load_state_dict uploads for the family, by name, shape and its values at <= 4096 fixed, evenly spaced flat
+    indices (cheap on a 2 GB adapter checkpoint). This is a provenance check, not a guarantee: two checkpoints that differ
+    only at unsampled indices get the same signature."""
+    family = embedding_family(model_type)
+    h = hashlib.sha256()
+    h.update(json.dumps({"family": family, "arch": arch, "frame_hw": [int(x) for x in frame_hw],
+                         "use_crop": bool(use_crop), "precision": capi.precision_enum(precision),
+                         "operand_dtype": str(capi.operand_dtype())}, sort_keys=True).encode())
+    for name, t in sorted(_image_weights(state_dict, family == "clip_adapter").items()):
+        flat = t.detach().reshape(-1)
+        n = flat.numel()
+        k = min(n, SIGNATURE_SAMPLES)
+        idx = torch.arange(k, dtype=torch.int64) * max(n - 1, 0) // max(k - 1, 1)
+        h.update(json.dumps([name, list(t.shape)]).encode())
+        h.update(flat[idx.to(flat.device)].float().cpu().numpy().astype("<f4").tobytes())
+    return np.frombuffer(h.digest(), np.uint8).copy()
+
+
 def _resolve_clip_weights(clip_state_dict, arch: str) -> dict:
     if clip_state_dict is not None:
         return clip_state_dict
@@ -163,6 +226,22 @@ def release_cached_engine():
     _ENGINE_CACHE.clear()
 
 
+def _model_state_dict(model_type: str, model_ckpt_dir, clip_state_dict, arch: str) -> dict:
+    """The state_dict a labeler of model_type uploads: CLIP weights, or the adapter checkpoint with CLIP nested under
+    "clip_model." (label_reward.py:165-176)."""
+    head, _ = _head_for(model_type)
+    if head in (capi.HEAD_ADAPTER, capi.HEAD_ADAPTER_ENSEMBLE, capi.HEAD_ADAPTER_GOAL):
+        assert model_ckpt_dir is not None, "specify model_ckpt_dir"  # label_reward.py:174
+        sd = load_checkpoint(model_ckpt_dir) if not isinstance(model_ckpt_dir, dict) else model_ckpt_dir
+        if not any(k.startswith("clip_model.") for k in sd):
+            # strict=False load in the reference (:176): CLIP tensors missing from the checkpoint keep
+            # the values clip.load gave them.
+            base = _resolve_clip_weights(clip_state_dict, arch)
+            sd = {**{"clip_model." + k: v for k, v in base.items()}, **sd}
+        return sd
+    return _resolve_clip_weights(clip_state_dict, arch)
+
+
 def _cached_engine(**cfg):
     key = tuple(sorted(cfg.items()))
     e = _ENGINE_CACHE.get(key)
@@ -182,9 +261,10 @@ class RewardLabeler:
     def __init__(self, model_type: str, text, frame_hw: tuple[int, int], *, model_ckpt_dir=None,
                  clip_state_dict=None, arch: str = "ViT-B/16", use_crop: bool = False, reduce: str = "first",
                  max_batch: int = 1024, device: int | None = None, precision: str = "16bit", tokenizer=None,
-                 extra_instructions: dict | None = None):
-        """extra_instructions: {inst_type: text(s)} scored with `text` in one pass; label_slab / label_file then return
-        arrays with a leading group axis [1 + len(extra_instructions), ...], `text` first."""
+                 extra_instructions: dict | None = None, relabel_only: bool = False):
+        """extra_instructions: {inst_type: text(s)} scored with `text` in one pass; label_slab / label_file /
+        label_embeddings then return arrays with a leading group axis [1 + len(extra_instructions), ...], `text` first.
+        relabel_only: the labeler only labels stored embeddings (label_embeddings); no image-side weight is uploaded."""
         head, pre = _head_for(model_type)
         prec = capi.precision_enum(precision)
         groups = _text_groups(model_type, text, extra_instructions)
@@ -200,18 +280,11 @@ class RewardLabeler:
                                      reduce=capi.REDUCE_MEAN if reduce == "mean" else capi.REDUCE_FIRST,
                                      max_batch=int(max_batch), precision=prec)
         dev = self.engine.device
-        if adapter:
-            sd = load_checkpoint(model_ckpt_dir) if not isinstance(model_ckpt_dir, dict) else model_ckpt_dir
-            if not any(k.startswith("clip_model.") for k in sd):
-                # strict=False load in the reference (:176): CLIP tensors missing from the checkpoint keep
-                # the values clip.load gave them.
-                base = _resolve_clip_weights(clip_state_dict, arch)
-                sd = {**{"clip_model." + k: v for k, v in base.items()}, **sd}
-        else:
-            sd = _resolve_clip_weights(clip_state_dict, arch)
-        missing = self.engine.load_state_dict(sd, strict=False)
-        if missing:
-            raise RuntimeError(f"checkpoint lacks {len(missing)} tensors the {model_type} path needs, e.g. {missing[:3]}")
+        sd = _model_state_dict(model_type, model_ckpt_dir, clip_state_dict, arch)
+        if not relabel_only:
+            missing = self.engine.load_state_dict(sd, strict=False)
+            if missing:
+                raise RuntimeError(f"checkpoint lacks {len(missing)} tensors the {model_type} path needs, e.g. {missing[:3]}")
         self.goal = self.engine.goal
         if not self.goal:
             tokenize = resolve_tokenizer(tokenizer)
@@ -243,6 +316,26 @@ class RewardLabeler:
     def label_file(self, fd: int, file_offset: int, T: int, row_stride_bytes: int, ep_offsets: np.ndarray, num_frames: int):
         """Same, the scored frame of row t read by the library from `fd` at file_offset + t*row_stride_bytes."""
         return self.engine.label_file(fd, file_offset, T, row_stride_bytes, ep_offsets, num_frames)
+
+    @property
+    def embedding_dim(self) -> int:
+        return self.engine.embedding_dim
+
+    def embed_slab(self, ob: np.ndarray) -> np.ndarray:
+        """The image side of label_slab: float32 [T, embedding_dim] host array, one stored embedding per row."""
+        return self.engine.embed_host(ob)
+
+    def embed_file(self, fd: int, file_offset: int, T: int, row_stride_bytes: int) -> np.ndarray:
+        """The image side of label_file."""
+        return self.engine.embed_file(fd, file_offset, T, row_stride_bytes)
+
+    def label_embeddings(self, emb: np.ndarray, ep_offsets: np.ndarray, num_frames: int):
+        """label_slab's outputs (host arrays) from stored embeddings [T, embedding_dim] of the same rows."""
+        dev = self.engine.device
+        # a read-only memory map (a stored dataset) is copied once: torch does not wrap non-writable arrays
+        out = self.engine.label_embeddings(torch.from_numpy(np.require(emb, np.float32, ["C", "W"])).to(dev),
+                                           torch.from_numpy(np.asarray(ep_offsets, np.int64)), num_frames)
+        return tuple(a.cpu().numpy() for a in out)
 
     def close(self, release: bool = False):
         """The native handle stays cached for the next call of this process unless release=True."""
@@ -324,7 +417,28 @@ def label_reward(
     precision="16bit",
     tokenizer=None,
     extra_instructions=None,
+    embeddings=None,
 ):
+    """embeddings (keyword-only):
+        None    label from the frames (the reference's behaviour).
+        "save"  embed the frames (the image side: decode, ViT, projection / adapter), label from the embeddings on the
+                device, and write, next to the same reward / pos_rtg datasets as None (bit for bit), the float32
+                [rows, dim] dataset embedding_key(img_key, model_type) over the labeled rows [off[0], off[n_eps]),
+                uncompressed (assigned in place when it exists with that shape; ValueError when its shape differs), and
+                its SHA-256 signature f"{key}_sig" (embedding_signature). dim = 512 for the clip family, 13*512 for the
+                adapter family. Sharded, each rank embeds and labels its own episodes and the embeddings reach rank 0
+                through a second gather: rank 0 then holds all of them, 4 * rows * dim bytes (the adapter family at
+                73 k frames: 1.9 GB; at configs[4] size: 38 GB). With NCCL that gather lands in rank 0's DEVICE
+                memory first (plus the padded all-gather buffer), then is copied to the host.
+        "load"  label from the stored embeddings instead of the frames: the done key and the image dataset's shape are
+                read, never its frames, and no image-side weight is uploaded. ValueError before any engine is created
+                when the embedding dataset or its signature is missing, its row count or width differs, or the signature
+                differs (another checkpoint, crop, frame size, arch or precision). Combines with extra_instructions, both
+                reduce values and goal-conditioned model types; an embedding saved by one model type loads in any model
+                type of its family (clip_ft -> clip_multiscale_ensemble, clip -> clip_goal_conditioned). Sharded, each
+                rank reads its own rows."""
+    if embeddings not in (None, "save", "load"):
+        raise ValueError(f"embeddings must be None, 'save' or 'load', got {embeddings!r}")
     # instruction sets this pass cannot label are refused before the dataset is opened or an engine is built
     target_keys = _target_keys(model_type, inst_type, extra_instructions)
     _text_groups(model_type, text, extra_instructions)
@@ -353,6 +467,7 @@ def label_reward(
     labeler = None
     failure = None
     results = {}
+    embs, sigs = {}, {}
     try:
         len_data, num_frames, g_traj_idx = episode_index(g)  # num_frames comes from the file (Q4)
         n_eps = len(g_traj_idx) - 1
@@ -364,17 +479,36 @@ def label_reward(
             H, W = g[image_keys[0]].shape[-3:-1]
             if use_crop:
                 print(f"image_size: {g[image_keys[0]].shape[-2]}")  # label_reward.py:104-105
+            if embeddings is not None:
+                # the weights are resolved once here: the signature needs them, and a refused load builds no engine
+                sd = _model_state_dict(model_type, model_ckpt_dir, clip_state_dict, arch)
+                model_ckpt_dir, clip_state_dict = (sd, None) if embedding_family(model_type) == "clip_adapter" else \
+                    (model_ckpt_dir, sd)
+                for img_key in image_keys:
+                    sigs[img_key] = embedding_signature(model_type, arch, g[img_key].shape[-3:-1], use_crop, precision,
+                                                        sd)
+                    _check_stored_embeddings(g, img_key, model_type, off, n_eps, sigs[img_key], embeddings)
             labeler = RewardLabeler(model_type, text, (int(H), int(W)), model_ckpt_dir=model_ckpt_dir,
                                     clip_state_dict=clip_state_dict, arch=arch, use_crop=use_crop, reduce=reduce,
                                     max_batch=max_batch, device=device, precision=precision, tokenizer=tokenizer,
-                                    extra_instructions=extra_instructions)
+                                    extra_instructions=extra_instructions, relabel_only=embeddings == "load")
             _mark("engine + weights + text tower")
             for img_key in image_keys:
+                if embeddings == "load":
+                    key, first = embedding_key(img_key, model_type), int(off[0])
+                    emb = np.ascontiguousarray(g[key][int(off[e_lo]) - first:int(off[e_hi]) - first], np.float32)
+                    results[img_key] = _label_embedding_rows(labeler, emb, off, e_lo, e_hi, num_frames, n_groups)
+                    continue
                 ds = g[img_key]
                 side = g.get(img_key + SIDECAR_SUFFIX)
                 if side is not None and (side.shape[0] != ds.shape[0] or tuple(side.shape[1:]) != tuple(ds.shape[2:])):
                     side = None                      # stale or foreign sidecar: fall back to the stacked dataset
-                results[img_key] = _label_rows(labeler, ds, side, off, e_lo, e_hi, num_frames, slab_frames, n_groups)
+                if embeddings == "save":
+                    embs[img_key] = _embed_rows(labeler, ds, side, off, e_lo, e_hi, slab_frames)
+                    results[img_key] = _label_embedding_rows(labeler, embs[img_key], off, e_lo, e_hi, num_frames,
+                                                             n_groups)
+                else:
+                    results[img_key] = _label_rows(labeler, ds, side, off, e_lo, e_hi, num_frames, slab_frames, n_groups)
             _mark("label (decode + encoder + head + scan, H2D / D2H)")
         except Exception as e:  # noqa: BLE001 — reported to every rank below, then re-raised
             failure = e
@@ -398,6 +532,9 @@ def label_reward(
                 if rank == 0:
                     full = full.cpu().numpy()
                     results[img_key] = [np.ascontiguousarray(full[:, k]) for k in range(full.shape[1])]
+                if embeddings == "save":             # the second gather: every rank's embeddings to rank 0
+                    full = gather_rows(torch.from_numpy(embs[img_key]).to(cdev), rows, dst=0)
+                    embs[img_key] = full.cpu().numpy() if rank == 0 else None
     finally:
         if labeler is not None:
             labeler.close()
@@ -410,6 +547,8 @@ def label_reward(
         try:
             for img_key in image_keys:
                 _write_labels(g, img_key, target_keys, results[img_key], off, n_eps, len_data, num_frames)
+                if embeddings == "save" and n_eps > 0:
+                    _write_embeddings(g, embedding_key(img_key, model_type), embs[img_key], sigs[img_key])
         finally:
             g.close()
     _mark("write labels")
@@ -420,46 +559,37 @@ def label_reward(
               + f"; total {_t[-1][1] - _t[0][1]:.3f} s", flush=True)
 
 
-def _label_rows(labeler, ds, side, off, e_lo: int, e_hi: int, num_frames: int, slab_frames: int, n_groups: int = 1):
-    """[reward_stacked, rtg_stacked] of each of the n_groups instruction sets in turn (2 * n_groups arrays [rows, F]) for
-    episodes [e_lo, e_hi). A memory-mapped container is handed to the library in ONE call (a strided pointer into the file
-    mapping; the native stager overlaps page-cache reads, PCIe and compute). A container that has to be read through its
-    API (h5py: chunked, gzip) is read slab by slab on a reader thread, one slab ahead of the GPU."""
+def _empty_pairs(labeler, n_groups: int, num_frames: int):
     empty = np.zeros((n_groups, 0, num_frames), np.float64 if labeler.goal else np.float32)
-    lo_all, hi_all = int(off[e_lo]), int(off[e_hi])
+    return _pairs(empty, empty)
 
-    def pairs(rs, gs):
-        return [a for g in range(n_groups) for a in (rs[g], gs[g])]
 
-    if hi_all <= lo_all:
-        return pairs(empty, empty)
+def _pairs(rs, gs):
+    """[G, rows, F] x 2 -> [reward_stacked, rtg_stacked] of each group in turn"""
+    return [a for g in range(rs.shape[0]) for a in (rs[g], gs[g])]
 
-    def finish(r, rs, gs, rel_off):
-        """[G, rows, F] whether or not the labeler returned a group axis"""
-        if labeler.goal:
-            rs, gs = _goal_float64(r, rel_off, num_frames)
-        return (rs, gs) if rs.ndim == 3 else (rs[None], gs[None])
 
-    src = side if side is not None else ds
-    rel = off[e_lo:e_hi + 1] - lo_all
-    fsrc = src.file_source() if hasattr(src, "file_source") and hasattr(labeler, "label_file") else None
-    if fsrc is not None:
-        # rows contiguous in a file: the library preads the scored frame of every row itself (arp_label_file)
-        path, base = fsrc
-        frame = int(np.prod(src.shape[-3:]))
-        stride = frame * (src.shape[1] if len(src.shape) == 5 else 1)
-        first = base + lo_all * stride + (stride - frame)            # last stacked frame of row lo_all
-        fd = os.open(path, os.O_RDONLY)
-        try:
-            r, _, rs, gs = labeler.label_file(fd, first, hi_all - lo_all, stride, rel, num_frames)
-        finally:
-            os.close(fd)
-        return pairs(*finish(r, rs, gs, rel))
-    arr = getattr(src, "array", None)
-    if arr is not None and arr.flags.c_contiguous:
-        r, _, rs, gs = labeler.label_slab(arr[lo_all:hi_all], rel, num_frames)
-        return pairs(*finish(r, rs, gs, rel))
+def _finish(labeler, r, rs, gs, rel_off, num_frames):
+    """[G, rows, F] whether or not the labeler returned a group axis (goal heads: the float64 scan of their rewards)"""
+    if labeler.goal:
+        rs, gs = _goal_float64(r, rel_off, num_frames)
+    return (rs, gs) if rs.ndim == 3 else (rs[None], gs[None])
 
+
+def _file_rows(labeler, src, method: str, lo_all: int):
+    """(path, byte offset of row lo_all's scored frame, row stride) when the rows sit contiguously in a file and the
+    labeler reads files itself (`method`), else None"""
+    fsrc = src.file_source() if hasattr(src, "file_source") and hasattr(labeler, method) else None
+    if fsrc is None:
+        return None
+    path, base = fsrc
+    frame = int(np.prod(src.shape[-3:]))
+    stride = frame * (src.shape[1] if len(src.shape) == 5 else 1)
+    return path, base + lo_all * stride + (stride - frame), stride        # last stacked frame of row lo_all
+
+
+def _read_slabs(ds, side, off, e_lo: int, e_hi: int, slab_frames: int):
+    """(a, b, rows) of every non-empty slab of whole episodes [a, b), read on a thread one slab ahead of the consumer"""
     import threading
     slabs = [(a, b) for a, b in _slabs(off, e_lo, e_hi, slab_frames) if off[b] > off[a]]
     box = {}
@@ -471,7 +601,8 @@ def _label_rows(labeler, ds, side, off, e_lo: int, e_hi: int, num_frames: int, s
         except Exception as e:  # noqa: BLE001 — re-raised on the consumer side
             box[i] = e
 
-    parts_r, parts_g = [], []
+    if not slabs:
+        return
     th = threading.Thread(target=read, args=(0,))
     th.start()
     for i, (a, b) in enumerate(slabs):
@@ -482,14 +613,111 @@ def _label_rows(labeler, ds, side, off, e_lo: int, e_hi: int, num_frames: int, s
         if i + 1 < len(slabs):
             th = threading.Thread(target=read, args=(i + 1,))
             th.start()
+        yield a, b, rows
+
+
+def _label_rows(labeler, ds, side, off, e_lo: int, e_hi: int, num_frames: int, slab_frames: int, n_groups: int = 1):
+    """[reward_stacked, rtg_stacked] of each of the n_groups instruction sets in turn (2 * n_groups arrays [rows, F]) for
+    episodes [e_lo, e_hi). A memory-mapped container is handed to the library in ONE call (a strided pointer into the file
+    mapping; the native stager overlaps page-cache reads, PCIe and compute). A container that has to be read through its
+    API (h5py: chunked, gzip) is read slab by slab on a reader thread, one slab ahead of the GPU."""
+    lo_all, hi_all = int(off[e_lo]), int(off[e_hi])
+    if hi_all <= lo_all:
+        return _empty_pairs(labeler, n_groups, num_frames)
+    src = side if side is not None else ds
+    rel = off[e_lo:e_hi + 1] - lo_all
+    frows = _file_rows(labeler, src, "label_file", lo_all)
+    if frows is not None:
+        # rows contiguous in a file: the library preads the scored frame of every row itself (arp_label_file)
+        path, first, stride = frows
+        fd = os.open(path, os.O_RDONLY)
+        try:
+            r, _, rs, gs = labeler.label_file(fd, first, hi_all - lo_all, stride, rel, num_frames)
+        finally:
+            os.close(fd)
+        return _pairs(*_finish(labeler, r, rs, gs, rel, num_frames))
+    arr = getattr(src, "array", None)
+    if arr is not None and arr.flags.c_contiguous:
+        r, _, rs, gs = labeler.label_slab(arr[lo_all:hi_all], rel, num_frames)
+        return _pairs(*_finish(labeler, r, rs, gs, rel, num_frames))
+
+    parts_r, parts_g = [], []
+    for a, b, rows in _read_slabs(ds, side, off, e_lo, e_hi, slab_frames):
         rel = off[a:b + 1] - off[a]
         r, _, rs, gs = labeler.label_slab(rows, rel, num_frames)
-        rs, gs = finish(r, rs, gs, rel)
+        rs, gs = _finish(labeler, r, rs, gs, rel, num_frames)
         parts_r.append(rs)
         parts_g.append(gs)
     if not parts_r:
-        return pairs(empty, empty)
-    return pairs(np.concatenate(parts_r, axis=1), np.concatenate(parts_g, axis=1))
+        return _empty_pairs(labeler, n_groups, num_frames)
+    return _pairs(np.concatenate(parts_r, axis=1), np.concatenate(parts_g, axis=1))
+
+
+def _embed_rows(labeler, ds, side, off, e_lo: int, e_hi: int, slab_frames: int) -> np.ndarray:
+    """float32 [rows, dim]: the stored embedding of every row of episodes [e_lo, e_hi), read from the container as
+    _label_rows reads it (same calls, same chunking of the encoder pass)."""
+    lo_all, hi_all = int(off[e_lo]), int(off[e_hi])
+    if hi_all <= lo_all:
+        return np.zeros((0, labeler.embedding_dim), np.float32)
+    src = side if side is not None else ds
+    frows = _file_rows(labeler, src, "embed_file", lo_all)
+    if frows is not None:
+        path, first, stride = frows
+        fd = os.open(path, os.O_RDONLY)
+        try:
+            return labeler.embed_file(fd, first, hi_all - lo_all, stride)
+        finally:
+            os.close(fd)
+    arr = getattr(src, "array", None)
+    if arr is not None and arr.flags.c_contiguous:
+        return labeler.embed_slab(arr[lo_all:hi_all])
+    parts = [labeler.embed_slab(rows) for _, _, rows in _read_slabs(ds, side, off, e_lo, e_hi, slab_frames)]
+    return np.concatenate(parts) if parts else np.zeros((0, labeler.embedding_dim), np.float32)
+
+
+def _label_embedding_rows(labeler, emb: np.ndarray, off, e_lo: int, e_hi: int, num_frames: int, n_groups: int = 1):
+    """_label_rows' result from the stored embeddings of the same rows, labeled in one call on the device"""
+    lo_all, hi_all = int(off[e_lo]), int(off[e_hi])
+    if hi_all <= lo_all:
+        return _empty_pairs(labeler, n_groups, num_frames)
+    rel = off[e_lo:e_hi + 1] - lo_all
+    r, _, rs, gs = labeler.label_embeddings(emb, rel, num_frames)
+    return _pairs(*_finish(labeler, r, rs, gs, rel, num_frames))
+
+
+def _check_stored_embeddings(g, img_key, model_type, off, n_eps, sig, mode):
+    """"load": the embedding dataset and its signature exist, cover the labeled rows and match `sig`. "save": an existing
+    embedding dataset has the shape this pass writes. ValueError otherwise."""
+    key = embedding_key(img_key, model_type)
+    shape = (int(off[n_eps] - off[0]) if n_eps > 0 else 0, EMBEDDING_DIM[embedding_family(model_type)])
+    ds = g.get(key)
+    if mode == "save":
+        if ds is not None and tuple(ds.shape) != shape:
+            raise ValueError(f"embeddings='save': {key} exists with shape {tuple(ds.shape)}, this pass writes {shape}")
+        return
+    if ds is None:
+        raise ValueError(f"embeddings='load': no dataset {key}; label once with embeddings='save'")
+    sds = g.get(key + "_sig")
+    if sds is None:
+        raise ValueError(f"embeddings='load': {key} has no signature dataset {key}_sig")
+    if tuple(ds.shape) != shape:
+        raise ValueError(f"embeddings='load': {key} has shape {tuple(ds.shape)}, the labeled rows need {shape}")
+    stored = np.asarray(sds[:], np.uint8).reshape(-1)
+    if not np.array_equal(stored, sig):
+        raise ValueError(f"embeddings='load': the signature of {key} differs: it was saved with another checkpoint, crop, "
+                         "frame size, arch or precision")
+
+
+def _write_embeddings(g, key, emb: np.ndarray, sig: np.ndarray):
+    """float32 [rows, dim] uncompressed (assigned in place when it exists with this shape) + the uint8 [32] signature"""
+    for k, a in ((key, np.ascontiguousarray(emb, np.float32)), (key + "_sig", sig)):
+        existing = g.get(k)
+        if existing is None:
+            g.create_dataset(k, data=a)
+        elif tuple(existing.shape) != a.shape:
+            raise ValueError(f"embeddings='save': {k} exists with shape {tuple(existing.shape)}, this pass writes {a.shape}")
+        else:
+            existing[...] = a
 
 
 def _goal_float64(r: np.ndarray, ep_off: np.ndarray, num_frames: int):
@@ -553,6 +781,8 @@ def main():
     parser.add_argument("--tokenizer", type=str, default=None, choices=["clip", "standin"])
     parser.add_argument("--extra_inst_types", type=str, default=None,
                         help="comma-separated inst_types labeled in the same pass as --inst_type, e.g. random1,misinfo")
+    parser.add_argument("--embeddings", type=str, default=None, choices=["save", "load"],
+                        help="save: also store per-frame image embeddings; load: label from stored embeddings, no frames")
     args = parser.parse_args()
 
     env_name = f"{args.env_name}" if args.env_type == "none" else f"{args.env_name}_{args.env_type}"
@@ -580,6 +810,7 @@ def main():
         base_path=args.base_path, model_type=args.model_type, model_ckpt_dir=args.model_ckpt_dir,
         use_crop=args.use_crop, inst_type=args.inst_type, arch=args.arch, reduce=args.reduce,
         max_batch=args.max_batch, precision=args.precision, tokenizer=args.tokenizer, extra_instructions=extra,
+        embeddings=args.embeddings,
     )
 
 

@@ -16,6 +16,12 @@
  * labeling call then scores all of them from ONE decode + encoder pass. Outputs become group-major: reward / rtg
  * [G, T], stacked arrays [G, T, F]; group g's rows are bit-identical to a call after arp_set_text(group g's rows).
  * arp_set_text is the G = 1 case, and with G = 1 every output has the shape it always had.
+ *
+ * Stored embeddings: labeling splits into an image side (decode, ViT, the head's projection / adapter) and an
+ * instruction side (cosine, group reduction, return-to-go scan). arp_embed_host / arp_embed_file run the image side once
+ * and return one fp32 vector per frame; arp_label_embeddings runs the instruction side on such vectors, with no frames
+ * and no image-side weights, and gives arp_label's outputs bit for bit. A new instruction, inst_type, reduce mode or
+ * text-head variant of the same checkpoint then costs a read of the vectors and one memory-bound head launch.
  */
 #ifndef ARP_B200_H_
 #define ARP_B200_H_
@@ -26,7 +32,7 @@
 extern "C" {
 #endif
 
-#define ARP_B200_ABI_VERSION 6   /* 3: + arp_encode_taps_chw, 4: + arp_operand_dtype, 5: + ARP_PREC_F32RESID, arp_ln_gemm, arp_resid_gemm_stats, arp_label_file, arp_wants_weight, 6: + arp_set_text_groups, arp_text_groups */
+#define ARP_B200_ABI_VERSION 7   /* 3: + arp_encode_taps_chw, 4: + arp_operand_dtype, 5: + ARP_PREC_F32RESID, arp_ln_gemm, arp_resid_gemm_stats, arp_label_file, arp_wants_weight, 6: + arp_set_text_groups, arp_text_groups, 7: + arp_embedding_dim, arp_embed_host, arp_embed_file, arp_label_embeddings */
 
 #define ARP_MAX_TEXT 16          /* texts of one instruction set (arp_set_text's n_text, one group's size) */
 #define ARP_MAX_TEXT_GROUPS 16   /* instruction sets of one arp_set_text_groups call */
@@ -181,6 +187,29 @@ ARP_API int arp_label_host(ArpHandle* h, const uint8_t* ob_host, int64_t T, int6
 ARP_API int arp_label_file(ArpHandle* h, int32_t fd, int64_t file_offset, int64_t T, int64_t row_stride_bytes,
                    const int64_t* ep_offsets_host, int32_t n_eps, int32_t num_frames, float* reward_host,
                    float* rtg_host, float* reward_stacked_host, float* rtg_stacked_host);
+
+/* Per-frame embedding width: 512 for the clip heads (ARP_HEAD_CLIP, ARP_HEAD_CLIP_GOAL), 13*512 for the adapter heads. */
+ARP_API int arp_embedding_dim(const ArpHandle* h);   /* 512 (clip heads) or 13*512 (adapter heads) */
+/* The image side of arp_label_host, stopped before the instruction: the per-frame embedding [T, dim] fp32 is written to
+ * emb_host (clip heads: encode_image un-normalised, label_reward.py:156; adapter heads: the gated feature
+ * a = sigmoid(w) * feat + (1 - sigmoid(w)) * mlp(feat) before F.normalize, clip_multiscale_adapter.py:145-151). Same
+ * frame arguments, staging and encoder pass as arp_label_host / arp_label_file; the result is assembled on the device and
+ * copied to the host once at the end (T * dim * 4 bytes of device memory, freed before the call returns). Synchronises.
+ * replaces the image half of compute_reward (label_reward.py:132-146, :200-230) when its output is to be kept. */
+/* per-frame embedding [T, dim] fp32 (clip: encode_image un-normalised; adapter: gated feature before F.normalize) */
+ARP_API int arp_embed_host(ArpHandle* h, const uint8_t* ob_host, int64_t T, int64_t row_stride_bytes, float* emb_host);
+ARP_API int arp_embed_file(ArpHandle* h, int32_t fd, int64_t file_offset, int64_t T, int64_t row_stride_bytes,
+                           float* emb_host);
+/* arp_label's outputs ([G,T] / [G,T,F] with text groups) from stored embeddings; needs no image-side weights */
+/* emb_dev [T, arp_embedding_dim] fp32 DEVICE rows from arp_embed_* of a handle with the same checkpoint; the other
+ * arguments and the four outputs are those of arp_label. Bit-identical to arp_label on the frames the rows came from. An
+ * embedding serves every head of its family: a clip row labels on ARP_HEAD_CLIP and ARP_HEAD_CLIP_GOAL, an adapter row on
+ * ARP_HEAD_ADAPTER, ARP_HEAD_ADAPTER_ENSEMBLE and ARP_HEAD_ADAPTER_GOAL. Works on a handle whose image-side weights were
+ * never set. ARP_ERR_STATE only when a text head has no text. Text heads make exactly two launches (head, scan).
+ * replaces compute_reward's cosine + discount_cumsum + stack_outputs (label_reward.py:141-146, :213-254) */
+ARP_API int arp_label_embeddings(ArpHandle* h, const float* emb_dev, int64_t T, const int64_t* ep_offsets_dev,
+                                 int32_t n_eps, int32_t num_frames, float* reward_dev, float* rtg_dev,
+                                 float* reward_stacked_dev, float* rtg_stacked_dev, void* stream);
 
 /* Latency mode — the online reward of a rollout (arp_dt/envs/vl_reward.py:11-23 get_torch_clip_reward, :44-59
  * get_torch_clip_adapter_reward, and the two encode_image calls of the goal-conditioned variants :26-41, :62-77;
