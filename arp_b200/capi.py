@@ -38,7 +38,7 @@ EXPORTS = (
     "arp_profile_begin", "arp_profile_end", "arp_online_reward", "arp_preprocess_rtgs",
     "arp_quantile_f32", "arp_encode_taps_chw", "arp_operand_dtype", "arp_ln_gemm", "arp_resid_gemm_stats", "arp_label_file", "arp_wants_weight",
     "arp_set_text_groups", "arp_text_groups", "arp_embedding_dim", "arp_embed_host", "arp_embed_file",
-    "arp_label_embeddings",
+    "arp_label_embeddings", "arp_tower_dim", "arp_embed_tower_host", "arp_embed_tower_file", "arp_label_tower",
 )
 PROFILE_CLASSES = ("gemm", "attention", "layernorm", "decode", "head", "scan", "other")
 
@@ -104,6 +104,10 @@ def load_library() -> C.CDLL:
     lib.arp_embed_host.argtypes = [vp, vp, i64, i64, vp]
     lib.arp_embed_file.argtypes = [vp, i32, i64, i64, i64, vp]
     lib.arp_label_embeddings.argtypes = [vp, vp, i64, vp, i32, i32, vp, vp, vp, vp, vp]
+    lib.arp_tower_dim.argtypes = [vp]
+    lib.arp_embed_tower_host.argtypes = [vp, vp, i64, i64, vp]
+    lib.arp_embed_tower_file.argtypes = [vp, i32, i64, i64, i64, vp]
+    lib.arp_label_tower.argtypes = [vp, vp, i64, vp, i32, i32, vp, vp, vp, vp, vp]
     lib.arp_compute_reward.argtypes = [vp, vp, i64, i64, vp, vp, vp]
     lib.arp_online_reward.argtypes = [vp, vp, i32, vp, vp, vp]
     lib.arp_preprocess_rtgs.argtypes = [vp, vp, i64, vp, i32, i32, i32, vp, vp, vp, vp, vp]
@@ -346,25 +350,31 @@ class Engine:
         """Width of the per-frame embedding: 512 for the clip heads, 13*512 for the adapter heads."""
         return int(self._lib.arp_embedding_dim(self._h))
 
-    def _emb_out(self, T: int, out):
+    def _emb_out(self, T: int, out, dim: "int | None" = None):
+        dim = self.embedding_dim if dim is None else dim
         if out is None:
-            return torch.empty((T, self.embedding_dim), dtype=torch.float32, pin_memory=True).numpy()
-        assert out.dtype == np.float32 and out.flags.c_contiguous and out.shape == (T, self.embedding_dim), out.shape
+            return torch.empty((T, dim), dtype=torch.float32, pin_memory=True).numpy()
+        assert out.dtype == np.float32 and out.flags.c_contiguous and out.shape == (T, dim), out.shape
         return out
 
-    def embed_host(self, ob: "np.ndarray | torch.Tensor", out: "np.ndarray | None" = None) -> np.ndarray:
-        """arp_embed_host: host frames as label_host takes them -> float32 [T, embedding_dim] host array (clip heads:
-        encode_image before normalisation; adapter heads: the gated feature before normalisation). Without `out` each
-        call allocates a new pinned array of T * embedding_dim * 4 bytes; pass `out` to reuse one across calls."""
+    @staticmethod
+    def _host_frames(ob: "np.ndarray | torch.Tensor"):
+        """(T, pointer to row 0's scored frame, row stride) of host frames as label_host takes them"""
         if isinstance(ob, np.ndarray):
             assert ob.dtype == np.uint8 and ob.flags.c_contiguous and ob.ndim in (4, 5)
             base, shape = ob.ctypes.data, ob.shape
         else:
             assert ob.device.type == "cpu" and ob.dtype == torch.uint8 and ob.is_contiguous()
             base, shape = ob.data_ptr(), tuple(ob.shape)
-        T = shape[0]
         frame = int(np.prod(shape[-3:]))
         p, stride = (base + (shape[1] - 1) * frame, shape[1] * frame) if len(shape) == 5 else (base, frame)
+        return shape[0], p, stride
+
+    def embed_host(self, ob: "np.ndarray | torch.Tensor", out: "np.ndarray | None" = None) -> np.ndarray:
+        """arp_embed_host: host frames as label_host takes them -> float32 [T, embedding_dim] host array (clip heads:
+        encode_image before normalisation; adapter heads: the gated feature before normalisation). Without `out` each
+        call allocates a new pinned array of T * embedding_dim * 4 bytes; pass `out` to reuse one across calls."""
+        T, p, stride = self._host_frames(ob)
         out = self._emb_out(T, out)
         self._check(self._lib.arp_embed_host(self._h, C.c_void_p(p), T, stride, C.c_void_p(out.ctypes.data)))
         return out
@@ -377,6 +387,13 @@ class Engine:
                                              C.c_void_p(out.ctypes.data)))
         return out
 
+    def _device_outputs(self, T: int, num_frames: int):
+        lead = self._lead()
+        return (torch.empty(lead + (T,), device=self.device, dtype=torch.float32),
+                torch.empty(lead + (T,), device=self.device, dtype=torch.float32),
+                torch.empty(lead + (T, num_frames), device=self.device, dtype=torch.float32),
+                torch.empty(lead + (T, num_frames), device=self.device, dtype=torch.float32))
+
     def label_embeddings(self, emb: torch.Tensor, ep_offsets: torch.Tensor, num_frames: int):
         """arp_label_embeddings: stored embeddings [T, embedding_dim] in, label's outputs out (device tensors, a leading
         group axis after set_text_groups). Needs no image-side weights."""
@@ -384,13 +401,43 @@ class Engine:
         assert x.dim() == 2 and x.shape[1] == self.embedding_dim, (tuple(x.shape), self.embedding_dim)
         T = x.shape[0]
         off = ep_offsets.to(self.device, torch.int64).contiguous()
-        lead = self._lead()
-        r = torch.empty(lead + (T,), device=self.device, dtype=torch.float32)
-        g = torch.empty(lead + (T,), device=self.device, dtype=torch.float32)
-        rs = torch.empty(lead + (T, num_frames), device=self.device, dtype=torch.float32)
-        gs = torch.empty(lead + (T, num_frames), device=self.device, dtype=torch.float32)
+        r, g, rs, gs = self._device_outputs(T, num_frames)
         self._check(self._lib.arp_label_embeddings(self._h, _ptr(x), T, _ptr(off), off.numel() - 1, num_frames, _ptr(r),
                                                    _ptr(g), _ptr(rs), _ptr(gs), _stream_ptr(self.device)))
+        return r, g, rs, gs
+
+    # -- CLIP tower records -----------------------------------------------------------------------
+    @property
+    def tower_dim(self) -> int:
+        """Width of the CLIP tower record: 12*768 + 512 = 9728 for the adapter heads, 0 for the clip heads."""
+        return int(self._lib.arp_tower_dim(self._h))
+
+    def embed_tower_host(self, ob: "np.ndarray | torch.Tensor", out: "np.ndarray | None" = None) -> np.ndarray:
+        """arp_embed_tower_host (adapter heads): host frames as label_host takes them -> float32 [T, tower_dim] host array,
+        the frozen CLIP tower's class-token taps and un-normalised feature per frame. Allocation as embed_host."""
+        T, p, stride = self._host_frames(ob)
+        out = self._emb_out(T, out, self.tower_dim)
+        self._check(self._lib.arp_embed_tower_host(self._h, C.c_void_p(p), T, stride, C.c_void_p(out.ctypes.data)))
+        return out
+
+    def embed_tower_file(self, fd: int, file_offset: int, T: int, row_stride_bytes: int,
+                         out: "np.ndarray | None" = None) -> np.ndarray:
+        """arp_embed_tower_file: the scored frame of row t read from `fd` at file_offset + t*row_stride_bytes."""
+        out = self._emb_out(int(T), out, self.tower_dim)
+        self._check(self._lib.arp_embed_tower_file(self._h, int(fd), int(file_offset), int(T), int(row_stride_bytes),
+                                                   C.c_void_p(out.ctypes.data)))
+        return out
+
+    def label_tower(self, rec: torch.Tensor, ep_offsets: torch.Tensor, num_frames: int):
+        """arp_label_tower: tower records [T, tower_dim] in, label's outputs out (device tensors, a leading group axis after
+        set_text_groups), computed with this handle's adapter. Needs only the image-adapter tensors."""
+        x = rec.to(self.device, torch.float32).contiguous()
+        assert x.dim() == 2 and x.shape[1] == self.tower_dim, (tuple(x.shape), self.tower_dim)
+        T = x.shape[0]
+        off = ep_offsets.to(self.device, torch.int64).contiguous()
+        r, g, rs, gs = self._device_outputs(T, num_frames)
+        self._check(self._lib.arp_label_tower(self._h, _ptr(x), T, _ptr(off), off.numel() - 1, num_frames, _ptr(r),
+                                              _ptr(g), _ptr(rs), _ptr(gs), _stream_ptr(self.device)))
         return r, g, rs, gs
 
     def compute_reward(self, ob: torch.Tensor, want_logits: bool = False):

@@ -2,7 +2,8 @@
 // stream-ordered pipeline   decode -> patch-embed GEMM -> ln_pre -> 12 x [QKV (ln_1 folded), attention, out-proj (+= x,
 // row moments), c_fc (ln_2 folded, QuickGELU), c_proj (+= x, row moments)] (the last block for the class-token row only)
 // -> reward head -> per-episode return-to-go scan. The embed entry points stop after the head's image side and return the
-// per-frame embedding; arp_label_embeddings runs only the instruction side (head + scan) on such embeddings.
+// per-frame embedding; arp_label_embeddings runs only the instruction side (head + scan) on such embeddings. The tower
+// entry points stop the adapter heads after the frozen CLIP tower; arp_label_tower runs the adapter tail from there.
 // Host logic only; every kernel lives in the .cuh next to this file.
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -34,6 +35,7 @@
 #include "layernorm.cuh"
 #include "rtgstats.cuh"
 #include "scan.cuh"
+#include "tower.cuh"
 
 using namespace arp;
 static_assert(ARP_MAX_TEXT == HEAD_MAX_TEXT && ARP_MAX_TEXT_GROUPS == HEAD_MAX_GROUPS &&
@@ -139,6 +141,7 @@ struct ArpHandle {
   float *fc1_b = nullptr, *fc2_b = nullptr, *res_w = nullptr;
   float res_sigmoid = 0.f;
   bool finalized = false;
+  bool adapter_ready = false;   // the image-adapter tensors are set and res_sigmoid is current (arp_label_tower)
   std::map<std::string, WeightSlot> slots;
 
   // text: n_text rows = n_groups instruction sets concatenated, group g = rows [group_off[g], group_off[g+1])
@@ -718,6 +721,7 @@ extern "C" int arp_set_weight(ArpHandle* h, const char* name, const void* data, 
   ARP_CUDA(h, cudaGetLastError());
   s.set = true;
   h->finalized = false;
+  h->adapter_ready = false;
   h->online_epoch++;
   return ARP_OK;
 }
@@ -740,6 +744,15 @@ extern "C" int arp_missing_weights(const ArpHandle* h, char* names_out, int64_t 
   return missing;
 }
 
+// the adapter gate sigmoid(image_residual_weight) (clip_multiscale_adapter.py:145-151), read once per weight upload
+static int read_res_sigmoid(ArpHandle* h, cudaStream_t st) {
+  float w = 0.f;
+  ARP_CUDA(h, cudaMemcpyAsync(&w, h->res_w, 4, cudaMemcpyDeviceToHost, st));
+  ARP_CUDA(h, cudaStreamSynchronize(st));
+  h->res_sigmoid = 1.0f / (1.0f + expf(-w));
+  return ARP_OK;
+}
+
 static int finalize_weights(ArpHandle* h, cudaStream_t st) {
   if (h->finalized) return ARP_OK;
   char buf[256];
@@ -756,14 +769,23 @@ static int finalize_weights(ArpHandle* h, cudaStream_t st) {
       h->launches += 2;
     }
   }
-  if (h->adapter) {
-    float w = 0.f;
-    ARP_CUDA(h, cudaMemcpyAsync(&w, h->res_w, 4, cudaMemcpyDeviceToHost, st));
-    ARP_CUDA(h, cudaStreamSynchronize(st));
-    h->res_sigmoid = 1.0f / (1.0f + expf(-w));
-  }
+  if (h->adapter) ARP_TRY(read_res_sigmoid(h, st));
   ARP_CUDA(h, cudaGetLastError());
   h->finalized = true;
+  return ARP_OK;
+}
+
+// arp_label_tower's readiness: only the image-adapter tensors are needed (no visual.* slot, no rowtab, no LayerNorm fold),
+// and res_sigmoid is computed from image_residual_weight as finalize_weights computes it
+static int adapter_weights_ready(ArpHandle* h, cudaStream_t st) {
+  if (h->adapter_ready || h->finalized) return ARP_OK;
+  static const char* names[] = {"image_intermediate_linear.weight", "image_adapter.layers.0.weight",
+                                "image_adapter.layers.0.bias", "image_adapter.layers.3.weight",
+                                "image_adapter.layers.3.bias", "image_residual_weight"};
+  for (const char* n : names)
+    if (!h->slots.at(n).set) return fail(h, ARP_ERR_STATE, "adapter weight '%s' not set", n);
+  ARP_TRY(read_res_sigmoid(h, st));
+  h->adapter_ready = true;
   return ARP_OK;
 }
 
@@ -1290,39 +1312,38 @@ static int encode_chunk_f32(ArpHandle* h, const uint8_t* ob, int64_t n, int64_t 
   return ARP_OK;
 }
 
-// heads. reward_out [n_groups, ld] (this chunk's column 0; ld = the call's T) / logits_out [n, n_text] /
-// feat_out [n, feat_dim] may each be null.
-static int head_chunk(ArpHandle* h, int64_t n, float* reward_out, int64_t ld, float* logits_out, float* feat_out,
-                      cudaStream_t st) {
+// The adapter heads' final CLIP feature: clip_head_kernel on the class-token rows -> the last 512 columns of ws.featf
+// (un-normalised, clip_multiscale_adapter.py:136,145). The tower record stores these columns.
+static void adapter_clip_feature(ArpHandle* h, int64_t n, cudaStream_t st) {
+  const ArpConfig& c = h->cfg;
+  ArpHandle::Work& ws = h->ws;
+  const float* xsrc = h->f32 ? ws.x : ws.xcls;     // class-token rows: compact after the tensor-core paths' pruned last block
+  const int xtok = h->f32 ? h->tokens : 1;
+  clip_head_kernel<768, 512><<<(unsigned)((n + HEAD_FR - 1) / HEAD_FR), 256, HEAD_SMEM_BYTES, st>>>(
+      xsrc, xtok, h->ln_post_g, h->ln_post_b, 1e-5f, h->proj, nullptr, 0, nullptr, 0, 0.f, 0, ws.featf, h->feat_dim,
+      c.layers * c.embed_dim, nullptr, nullptr, 0, (int)n);
+  h->launches++;
+}
+
+// The adapter tail, from the class-token taps (ws.taps; ws.taps32 on the fp32 path) and the CLIP feature in
+// ws.featf[:, Dmid:] of n rows: the intermediate GEMM, the AdapterMLP, then the gate + head. head_chunk runs it after the
+// encoder, arp_label_tower after unpacking a tower record: one code path, so both give the same bits from the same values.
+// Arguments as head_chunk's.
+static int adapter_tail(ArpHandle* h, int64_t n, float* reward_out, int64_t ld, float* logits_out, float* feat_out,
+                        cudaStream_t st) {
   const ArpConfig& c = h->cfg;
   ArpHandle::Work& ws = h->ws;
   const bool need_text = reward_out || logits_out;
-  if (need_text && !h->goal && !h->text) return fail(h, ARP_ERR_STATE, "arp_set_text has not been called");
-  const float* xsrc = h->f32 ? ws.x : ws.xcls;     // class-token rows: compact after the tensor-core paths' pruned last block
-  const int xtok = h->f32 ? h->tokens : 1;
-  if (!h->adapter) {
-    ProfScope prof(h, PC_HEAD, 2.0 * (double)n * 768 * 512, (double)n * 768 * 4 + 768.0 * 512 * 4, st);
-    clip_head_kernel<768, 512><<<(unsigned)((n + HEAD_FR - 1) / HEAD_FR), 256, HEAD_SMEM_BYTES, st>>>(
-        xsrc, xtok, h->ln_post_g, h->ln_post_b, 1e-5f, h->proj, (need_text && !h->goal) ? h->text : nullptr,
-        h->n_text, h->group_off, h->n_groups, h->logit_scale, c.reduce, feat_out, c.embed_dim, 0, logits_out,
-        h->goal ? nullptr : reward_out, ld, (int)n);
-    h->launches++;
+  const int D = h->feat_dim, Dmid = c.layers * c.embed_dim, Din = c.layers * c.width;
+  const int64_t B = c.max_batch;
+  if (h->f32) {
+    ARP_TRY(launch_sgemm(h, ws.taps32, Din, h->inter_w, ws.featf, D, F32_ACT_NONE, n, Dmid, Din, nullptr, nullptr, 0,
+                         nullptr, 0, st));
+    ARP_TRY(launch_sgemm(h, ws.featf, D, h->fc1_w, ws.hid2_32, 2 * D, F32_ACT_RELU, n, 2 * D, D, h->fc1_b, nullptr, 0,
+                         nullptr, 0, st));
+    ARP_TRY(launch_sgemm(h, ws.hid2_32, 2 * D, h->fc2_w, ws.mlp, D, F32_ACT_NONE, n, D, 2 * D, h->fc2_b, nullptr, 0,
+                         nullptr, 0, st));
   } else {
-    const int D = h->feat_dim, Dmid = c.layers * c.embed_dim, Din = c.layers * c.width;
-    const int64_t B = c.max_batch;
-    // final CLIP feature -> last 512 columns of feat (un-normalised, clip_multiscale_adapter.py:136,145)
-    clip_head_kernel<768, 512><<<(unsigned)((n + HEAD_FR - 1) / HEAD_FR), 256, HEAD_SMEM_BYTES, st>>>(
-        xsrc, xtok, h->ln_post_g, h->ln_post_b, 1e-5f, h->proj, nullptr, 0, nullptr, 0, 0.f, 0, ws.featf, D, Dmid,
-        nullptr, nullptr, 0, (int)n);
-    h->launches++;
-    if (h->f32) {
-      ARP_TRY(launch_sgemm(h, ws.taps32, Din, h->inter_w, ws.featf, D, F32_ACT_NONE, n, Dmid, Din, nullptr, nullptr, 0,
-                           nullptr, 0, st));
-      ARP_TRY(launch_sgemm(h, ws.featf, D, h->fc1_w, ws.hid2_32, 2 * D, F32_ACT_RELU, n, 2 * D, D, h->fc1_b, nullptr, 0,
-                           nullptr, 0, st));
-      ARP_TRY(launch_sgemm(h, ws.hid2_32, 2 * D, h->fc2_w, ws.mlp, D, F32_ACT_NONE, n, D, 2 * D, h->fc2_b, nullptr, 0,
-                           nullptr, 0, st));
-    } else {
     // image_intermediate_linear (no bias) over the 12 CLS taps -> first 6144 columns (:143-144)
     ARP_TRY(launch_gemm(h, ws.taps, B, h->inter_w, ws.featf, true, ACT_NONE, n, Dmid, Din, D, nullptr, nullptr, 0,
                         nullptr, 0, st));
@@ -1333,12 +1354,37 @@ static int head_chunk(ArpHandle* h, int64_t n, float* reward_out, int64_t ld, fl
                         nullptr, 0, st));
     ARP_TRY(launch_gemm(h, ws.hid2, B, h->fc2_w, ws.mlp, true, ACT_NONE, n, D, 2 * D, D, h->fc2_b, nullptr, 0, nullptr,
                         0, st));
-    }
-    const bool ens = c.head == ARP_HEAD_ADAPTER_ENSEMBLE;
-    adapter_head_kernel<13, 512><<<(unsigned)n, 13 * 32, 0, st>>>(
-        ws.featf, ws.mlp, h->res_sigmoid, (need_text && !h->goal) ? h->text : nullptr,
-        (need_text && !h->goal) ? h->n_text : 0, h->group_off, (need_text && !h->goal) ? h->n_groups : 0,
-        h->logit_scale, ens ? 1 : 0, c.reduce, logits_out, h->goal ? nullptr : reward_out, ld, feat_out);
+  }
+  const bool ens = c.head == ARP_HEAD_ADAPTER_ENSEMBLE;
+  adapter_head_kernel<13, 512><<<(unsigned)n, 13 * 32, 0, st>>>(
+      ws.featf, ws.mlp, h->res_sigmoid, (need_text && !h->goal) ? h->text : nullptr,
+      (need_text && !h->goal) ? h->n_text : 0, h->group_off, (need_text && !h->goal) ? h->n_groups : 0,
+      h->logit_scale, ens ? 1 : 0, c.reduce, logits_out, h->goal ? nullptr : reward_out, ld, feat_out);
+  h->launches++;
+  ARP_CUDA(h, cudaGetLastError());
+  return ARP_OK;
+}
+
+// heads. reward_out [n_groups, ld] (this chunk's column 0; ld = the call's T) / logits_out [n, n_text] /
+// feat_out [n, feat_dim] may each be null.
+static int head_chunk(ArpHandle* h, int64_t n, float* reward_out, int64_t ld, float* logits_out, float* feat_out,
+                      cudaStream_t st) {
+  const ArpConfig& c = h->cfg;
+  ArpHandle::Work& ws = h->ws;
+  const bool need_text = reward_out || logits_out;
+  if (need_text && !h->goal && !h->text) return fail(h, ARP_ERR_STATE, "arp_set_text has not been called");
+  if (h->adapter) {
+    adapter_clip_feature(h, n, st);
+    return adapter_tail(h, n, reward_out, ld, logits_out, feat_out, st);
+  }
+  const float* xsrc = h->f32 ? ws.x : ws.xcls;     // class-token rows: compact after the tensor-core paths' pruned last block
+  const int xtok = h->f32 ? h->tokens : 1;
+  {
+    ProfScope prof(h, PC_HEAD, 2.0 * (double)n * 768 * 512, (double)n * 768 * 4 + 768.0 * 512 * 4, st);
+    clip_head_kernel<768, 512><<<(unsigned)((n + HEAD_FR - 1) / HEAD_FR), 256, HEAD_SMEM_BYTES, st>>>(
+        xsrc, xtok, h->ln_post_g, h->ln_post_b, 1e-5f, h->proj, (need_text && !h->goal) ? h->text : nullptr,
+        h->n_text, h->group_off, h->n_groups, h->logit_scale, c.reduce, feat_out, c.embed_dim, 0, logits_out,
+        h->goal ? nullptr : reward_out, ld, (int)n);
     h->launches++;
   }
   ARP_CUDA(h, cudaGetLastError());
@@ -1637,16 +1683,33 @@ struct HostStager {
   void stop() { abort.store(true); for (auto& t : threads) t.join(); threads.clear(); }
 };
 
+// arp_embed_tower_*: the adapter head stopped after the CLIP feature; the chunk's taps and feature become n tower records
+static int tower_chunk(ArpHandle* h, int64_t n, float* rec, cudaStream_t st) {
+  ArpHandle::Work& ws = h->ws;
+  adapter_clip_feature(h, n, st);
+  const int Dmid = h->cfg.layers * h->cfg.embed_dim;
+  ProfScope prof(h, PC_OTHER, 0.0, (double)n * (TOWER_TAPS * (h->f32 ? 4 : 2) + TOWER_FEAT * 4 + TOWER_DIM * 4), st);
+  if (h->f32)
+    tower_pack_kernel<float><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(ws.taps32, ws.featf, h->feat_dim, Dmid, rec, (int)n);
+  else
+    tower_pack_kernel<bf16><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(ws.taps, ws.featf, h->feat_dim, Dmid, rec, (int)n);
+  h->launches++;
+  ARP_CUDA(h, cudaGetLastError());
+  return ARP_OK;
+}
+
 // emb_host != nullptr: embed mode (arp_embed_host / arp_embed_file) — the same staging and encoder pass, the head writes
 // the per-frame embedding [T, feat_dim] (head_chunk's feat_out) to the device, and it is copied to emb_host once at the
-// end; there is no reward, no scan, and the episode / output arguments are ignored.
+// end; there is no reward, no scan, and the episode / output arguments are ignored. tower (adapter heads,
+// arp_embed_tower_*): the head stops after the CLIP feature and the rows are tower records [T, TOWER_DIM] instead.
 static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t fd_offset, int64_t T,
                            int64_t row_stride_bytes, const int64_t* ep_offsets_host, int32_t n_eps, int32_t num_frames,
                            float* reward_host, float* rtg_host, float* reward_stacked_host, float* rtg_stacked_host,
-                           float* emb_host = nullptr) {
+                           float* emb_host = nullptr, bool tower = false) {
   if (!h) return ARP_ERR_INVALID;
   cudaStream_t st = h->own_stream;
   const bool embed = emb_host != nullptr;
+  const int64_t ew = tower ? TOWER_DIM : h->feat_dim;   // embed mode: floats per row
   if (fd >= 0 && fd_offset < 0) return fail(h, ARP_ERR_INVALID, "bad file offset");
   ARP_TRY(check_ready(h, fd >= 0 ? reinterpret_cast<const uint8_t*>(h) : ob_host, T, row_stride_bytes, st));
   if (!embed && (!ep_offsets_host || n_eps < 0)) return fail(h, ARP_ERR_INVALID, "bad episode offsets");
@@ -1658,10 +1721,10 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
   const int F = embed ? 1 : num_frames;
   ARP_TRY(ensure_stage(h));
   // device outputs (scratch slot 1), G = n_groups:
-  // [ep_off (n_eps+1) i64][reward G*T][rtg G*T][reward_stacked G*T*F][rtg_stacked G*T*F]; embed mode: [emb T*feat_dim]
+  // [ep_off (n_eps+1) i64][reward G*T][rtg G*T][reward_stacked G*T*F][rtg_stacked G*T*F]; embed mode: [emb T*ew]
   const size_t G = (size_t)h->n_groups;
   const size_t off_bytes = embed ? 0 : (((size_t)(n_eps + 1) * 8) + 255) & ~(size_t)255;
-  const size_t out_bytes = embed ? (size_t)T * h->feat_dim * 4 : G * T * 4 * (2 + 2 * F);
+  const size_t out_bytes = embed ? (size_t)T * ew * 4 : G * T * 4 * (2 + 2 * F);
   ARP_TRY(ensure_scratch(h, 1, off_bytes + out_bytes + 1024));
   LabelTmp tmp;
   if (!embed) ARP_TRY(carve_label_tmp(h, T, &tmp));
@@ -1715,7 +1778,8 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
     cudaEventRecord(h->ev_copied[buf], h->copy_stream);
     cudaStreamWaitEvent(st, h->ev_copied[buf], 0);
     if ((rc = encode_chunk(h, h->stage_dev[buf], n, (int64_t)frame_bytes, st)) != ARP_OK) break;
-    if (embed) rc = head_chunk(h, n, nullptr, 0, nullptr, d_emb + t0 * h->feat_dim, st);
+    if (tower) rc = tower_chunk(h, n, d_emb + t0 * ew, st);
+    else if (embed) rc = head_chunk(h, n, nullptr, 0, nullptr, d_emb + t0 * ew, st);
     else if (!h->goal) rc = head_chunk(h, n, d_r + t0, T, nullptr, nullptr, st);
     else rc = head_chunk(h, n, nullptr, 0, nullptr, tmp.feats + t0 * h->feat_dim, st);
     cudaEventRecord(h->ev_consumed[buf], st);
@@ -1730,12 +1794,13 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
               (long long)T, subs.size(), stager.waited_s);
   }
   if (rc == ARP_OK && embed) {
-    cudaError_t e = cudaMemcpyAsync(emb_host, d_emb, (size_t)T * h->feat_dim * 4, cudaMemcpyDeviceToHost, st);
+    cudaError_t e = cudaMemcpyAsync(emb_host, d_emb, (size_t)T * ew * 4, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) rc = fail(h, ARP_ERR_CUDA, "embedding D2H failed: %s", cudaGetErrorString(e));
   }
   if (embed) {
-    // the [T, feat_dim] device result (1.9 GB for an adapter head at 73 k frames) is not kept by the handle between calls
+    // the [T, ew] device result (1.9 GB for an adapter head at 73 k frames, 2.8 GB of tower records) is not kept by the
+    // handle between calls
     cudaStreamSynchronize(h->copy_stream);
     cudaStreamSynchronize(st);
     cudaFree(h->scratch[1]);
@@ -1836,6 +1901,76 @@ extern "C" int arp_label_embeddings(ArpHandle* h, const float* emb_dev, int64_t 
     h->launches++;
   }
   ARP_CUDA(h, cudaGetLastError());
+  return scan_launch(h, r, T, ep_offsets_dev, n_eps, num_frames, 1.0f, g, reward_stacked_dev, rtg_stacked_dev, st,
+                     h->n_groups);
+}
+
+// ------------------------------------------------------------------------------------------------
+// C ABI: CLIP tower records (relabeling with another adapter checkpoint without frames or the ViT)
+// ------------------------------------------------------------------------------------------------
+extern "C" int arp_tower_dim(const ArpHandle* h) { return h && h->adapter ? TOWER_DIM : 0; }
+
+extern "C" int arp_embed_tower_host(ArpHandle* h, const uint8_t* ob_host, int64_t T, int64_t row_stride_bytes,
+                                    float* rec_host) {
+  if (!h || T < 0 || (T > 0 && !rec_host)) return fail(h, ARP_ERR_INVALID, "null argument / bad T");
+  if (!h->adapter) return fail(h, ARP_ERR_INVALID, "tower records serve the adapter heads only");
+  if (T == 0) return check_ready(h, ob_host, T, row_stride_bytes, h->own_stream);
+  return label_host_impl(h, ob_host, -1, 0, T, row_stride_bytes, nullptr, 0, 0, nullptr, nullptr, nullptr, nullptr,
+                         rec_host, true);
+}
+
+extern "C" int arp_embed_tower_file(ArpHandle* h, int32_t fd, int64_t file_offset, int64_t T, int64_t row_stride_bytes,
+                                    float* rec_host) {
+  if (fd < 0) return fail(h, ARP_ERR_INVALID, "bad file descriptor");
+  if (!h || T < 0 || (T > 0 && !rec_host)) return fail(h, ARP_ERR_INVALID, "null argument / bad T");
+  if (!h->adapter) return fail(h, ARP_ERR_INVALID, "tower records serve the adapter heads only");
+  if (T == 0) return check_ready(h, reinterpret_cast<const uint8_t*>(h), T, row_stride_bytes, h->own_stream);
+  return label_host_impl(h, nullptr, fd, file_offset, T, row_stride_bytes, nullptr, 0, 0, nullptr, nullptr, nullptr,
+                         nullptr, rec_host, true);
+}
+
+// arp_label's outputs from tower records: per max_batch chunk one unpack launch, then adapter_tail — the launches of
+// head_chunk's adapter branch after its clip_head_kernel — and one scan for the call. Reads only the image-adapter
+// tensors (adapter_weights_ready, not finalize_weights), so a handle whose visual.* weights were never set works.
+extern "C" int arp_label_tower(ArpHandle* h, const float* rec_dev, int64_t T, const int64_t* ep_offsets_dev,
+                               int32_t n_eps, int32_t num_frames, float* reward_dev, float* rtg_dev,
+                               float* reward_stacked_dev, float* rtg_stacked_dev, void* stream) {
+  if (!h) return ARP_ERR_INVALID;
+  if (!h->adapter) return fail(h, ARP_ERR_INVALID, "tower records serve the adapter heads only");
+  if (T < 0 || (T > 0 && !rec_dev)) return fail(h, ARP_ERR_INVALID, "bad record buffer / T");
+  if (reinterpret_cast<uintptr_t>(rec_dev) & 15) return fail(h, ARP_ERR_INVALID, "record buffer must be 16-byte aligned");
+  if (!ep_offsets_dev || n_eps < 0) return fail(h, ARP_ERR_INVALID, "bad episode offsets");
+  if (num_frames < 1 || num_frames > 64) return fail(h, ARP_ERR_INVALID, "num_frames must be in [1,64]");
+  if (T > 0x7fffffffLL) return fail(h, ARP_ERR_INVALID, "T too large");
+  if (!h->goal && !h->text) return fail(h, ARP_ERR_STATE, "arp_set_text has not been called");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  ARP_CUDA(h, cudaSetDevice(h->cfg.device));
+  ARP_TRY(adapter_weights_ready(h, st));
+  if (T == 0) return ARP_OK;
+  LabelTmp tmp;
+  ARP_TRY(carve_label_tmp(h, T, &tmp));
+  float* r = reward_dev ? reward_dev : tmp.r;
+  float* g = rtg_dev ? rtg_dev : tmp.g;
+  ArpHandle::Work& ws = h->ws;
+  const int Dmid = h->cfg.layers * h->cfg.embed_dim;
+  const int64_t B = h->cfg.max_batch;
+  for (int64_t t0 = 0; t0 < T; t0 += B) {
+    const int64_t n = std::min(B, T - t0);
+    const float* rec = rec_dev + t0 * TOWER_DIM;
+    {
+      ProfScope prof(h, PC_OTHER, 0.0, (double)n * (TOWER_DIM * 4 + TOWER_TAPS * (h->f32 ? 4 : 2) + TOWER_FEAT * 4), st);
+      if (h->f32)
+        tower_unpack_kernel<float><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(rec, ws.taps32, ws.featf, h->feat_dim, Dmid,
+                                                                           (int)n);
+      else
+        tower_unpack_kernel<bf16><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(rec, ws.taps, ws.featf, h->feat_dim, Dmid,
+                                                                          (int)n);
+      h->launches++;
+    }
+    if (!h->goal) ARP_TRY(adapter_tail(h, n, r + t0, T, nullptr, nullptr, st));
+    else ARP_TRY(adapter_tail(h, n, nullptr, 0, nullptr, tmp.feats + t0 * h->feat_dim, st));
+  }
+  if (h->goal) ARP_TRY(goal_rewards(h, tmp, T, ep_offsets_dev, n_eps, r, st));
   return scan_launch(h, r, T, ep_offsets_dev, n_eps, num_frames, 1.0f, g, reward_stacked_dev, rtg_stacked_dev, st,
                      h->n_groups);
 }

@@ -39,7 +39,8 @@ Keyword-only extensions (all optional; defaults reproduce the reference):
     embeddings       None (default): label from the frames. "save": run the image side once, store the per-frame
                      embeddings, and label from them (same reward / pos_rtg datasets, bit for bit, plus the embedding
                      dataset). "load": label from stored embeddings; no frame is read and no image-side weight is
-                     uploaded. See label_reward().
+                     uploaded. "save_tower" / "load_tower" (adapter model types): the same with the CLIP tower record,
+                     which any adapter checkpoint fine-tuned from the same CLIP relabels. See label_reward().
 """
 from __future__ import annotations
 
@@ -156,6 +157,15 @@ def embedding_key(img_key: str, model_type: str) -> str:
     return f"{img_key}_{embedding_family(model_type)}_emb"
 
 
+#: the CLIP tower record of the adapter family: 12 class-token taps of 768 + the 512-wide CLIP feature (include/arp_b200.h)
+TOWER_DIM = 12 * 768 + 512
+
+
+def tower_key(img_key: str) -> str:
+    """Dataset of the CLIP tower records of img_key, f"{img_key}_clip_tower_emb"; its signature is f"{key}_sig"."""
+    return f"{img_key}_clip_tower_emb"
+
+
 _IMAGE_ADAPTER_PREFIXES = ("image_intermediate_linear.", "image_adapter.", "image_residual_weight")
 
 
@@ -176,13 +186,15 @@ SIGNATURE_SAMPLES = 4096
 
 
 def embedding_signature(model_type: str, arch: str, frame_hw, use_crop: bool, precision: str,
-                        state_dict: dict) -> np.ndarray:
+                        state_dict: dict, *, tower: bool = False) -> np.ndarray:
     """uint8 [32]: SHA-256 over what decides a stored embedding's bits — the embedding family, arch, frame H x W,
     use_crop, the precision's pipeline, the library's operand format, and a digest of the image-side weights: every tensor
     Engine.load_state_dict uploads for the family, by name, shape and its values at <= 4096 fixed, evenly spaced flat
     indices (cheap on a 2 GB adapter checkpoint). This is a provenance check, not a guarantee: two checkpoints that differ
-    only at unsampled indices get the same signature."""
-    family = embedding_family(model_type)
+    only at unsampled indices get the same signature.
+    tower=True: the signature of a CLIP tower record (family "clip_tower"): the same fields, but only the visual.*
+    tensors (an adapter checkpoint's "clip_model.visual.*"), not the image adapter — the record does not depend on it."""
+    family = "clip_tower" if tower else embedding_family(model_type)
     h = hashlib.sha256()
     h.update(json.dumps({"family": family, "arch": arch, "frame_hw": [int(x) for x in frame_hw],
                          "use_crop": bool(use_crop), "precision": capi.precision_enum(precision),
@@ -261,10 +273,12 @@ class RewardLabeler:
     def __init__(self, model_type: str, text, frame_hw: tuple[int, int], *, model_ckpt_dir=None,
                  clip_state_dict=None, arch: str = "ViT-B/16", use_crop: bool = False, reduce: str = "first",
                  max_batch: int = 1024, device: int | None = None, precision: str = "16bit", tokenizer=None,
-                 extra_instructions: dict | None = None, relabel_only: bool = False):
+                 extra_instructions: dict | None = None, relabel_only: bool = False, tower_only: bool = False):
         """extra_instructions: {inst_type: text(s)} scored with `text` in one pass; label_slab / label_file /
         label_embeddings then return arrays with a leading group axis [1 + len(extra_instructions), ...], `text` first.
-        relabel_only: the labeler only labels stored embeddings (label_embeddings); no image-side weight is uploaded."""
+        relabel_only: the labeler only labels stored embeddings (label_embeddings); no image-side weight is uploaded.
+        tower_only (adapter model types): the labeler only labels CLIP tower records (label_tower); of the image-side
+        weights only the image adapter is uploaded."""
         head, pre = _head_for(model_type)
         prec = capi.precision_enum(precision)
         groups = _text_groups(model_type, text, extra_instructions)
@@ -281,7 +295,13 @@ class RewardLabeler:
                                      max_batch=int(max_batch), precision=prec)
         dev = self.engine.device
         sd = _model_state_dict(model_type, model_ckpt_dir, clip_state_dict, arch)
-        if not relabel_only:
+        if tower_only:
+            assert adapter, "tower records serve the adapter model types"
+            self.engine.load_state_dict({k: v for k, v in sd.items() if k.startswith(_IMAGE_ADAPTER_PREFIXES)})
+            missing = [k for k in self.engine.missing_weights() if k.startswith(_IMAGE_ADAPTER_PREFIXES)]
+            if missing:
+                raise RuntimeError(f"checkpoint lacks {len(missing)} image-adapter tensors, e.g. {missing[:3]}")
+        elif not relabel_only:
             missing = self.engine.load_state_dict(sd, strict=False)
             if missing:
                 raise RuntimeError(f"checkpoint lacks {len(missing)} tensors the {model_type} path needs, e.g. {missing[:3]}")
@@ -335,6 +355,26 @@ class RewardLabeler:
         # a read-only memory map (a stored dataset) is copied once: torch does not wrap non-writable arrays
         out = self.engine.label_embeddings(torch.from_numpy(np.require(emb, np.float32, ["C", "W"])).to(dev),
                                            torch.from_numpy(np.asarray(ep_offsets, np.int64)), num_frames)
+        return tuple(a.cpu().numpy() for a in out)
+
+    @property
+    def tower_dim(self) -> int:
+        return self.engine.tower_dim
+
+    def embed_tower_slab(self, ob: np.ndarray) -> np.ndarray:
+        """The frozen-CLIP side of label_slab (adapter model types): float32 [T, tower_dim] host array of tower records."""
+        return self.engine.embed_tower_host(ob)
+
+    def embed_tower_file(self, fd: int, file_offset: int, T: int, row_stride_bytes: int) -> np.ndarray:
+        """The frozen-CLIP side of label_file."""
+        return self.engine.embed_tower_file(fd, file_offset, T, row_stride_bytes)
+
+    def label_tower(self, rec: np.ndarray, ep_offsets: np.ndarray, num_frames: int):
+        """label_slab's outputs (host arrays) from the CLIP tower records [T, tower_dim] of the same rows, with this
+        labeler's adapter."""
+        dev = self.engine.device
+        out = self.engine.label_tower(torch.from_numpy(np.require(rec, np.float32, ["C", "W"])).to(dev),
+                                      torch.from_numpy(np.asarray(ep_offsets, np.int64)), num_frames)
         return tuple(a.cpu().numpy() for a in out)
 
     def close(self, release: bool = False):
@@ -436,9 +476,25 @@ def label_reward(
                 differs (another checkpoint, crop, frame size, arch or precision). Combines with extra_instructions, both
                 reduce values and goal-conditioned model types; an embedding saved by one model type loads in any model
                 type of its family (clip_ft -> clip_multiscale_ensemble, clip -> clip_goal_conditioned). Sharded, each
-                rank reads its own rows."""
-    if embeddings not in (None, "save", "load"):
-        raise ValueError(f"embeddings must be None, 'save' or 'load', got {embeddings!r}")
+                rank reads its own rows.
+        "save_tower" / "load_tower"  (adapter model types only) the same with the CLIP tower record instead of the gated
+                adapter feature: the float32 [rows, TOWER_DIM] dataset tower_key(img_key) = f"{img_key}_clip_tower_emb"
+                (the 12 class-token taps and the un-normalised CLIP feature of every row, 38 912 bytes per row) and its
+                signature embedding_signature(..., tower=True), which covers the visual.* weights but not the image
+                adapter. Fine-tuning freezes CLIP, so the records of one CLIP serve every adapter checkpoint trained from
+                it: "load_tower" with a new model_ckpt_dir relabels with only that checkpoint's adapter GEMMs (0.468
+                GFLOP per frame instead of the ViT's 35.1), uploads only its image-adapter tensors, and writes what
+                embeddings=None with that checkpoint writes. Which to keep: "save" (26.6 KB per row) relabels new
+                instructions of ONE checkpoint with a single head launch; "save_tower" (38.9 KB per row) survives
+                re-fine-tuning the adapter. Refusals as for "load", and a clip-family model_type is refused (its
+                512-wide embedding does not depend on a checkpoint of its own: use "save" / "load")."""
+    if embeddings not in (None, "save", "load", "save_tower", "load_tower"):
+        raise ValueError(f"embeddings must be None, 'save', 'load', 'save_tower' or 'load_tower', got {embeddings!r}")
+    tower = embeddings in ("save_tower", "load_tower")
+    stored = embeddings.split("_")[0] if embeddings else None     # "save" / "load" / None, records of either kind
+    if tower and embedding_family(model_type) != "clip_adapter":
+        raise ValueError(f"embeddings={embeddings!r}: tower records serve the adapter model types, not {model_type!r}; "
+                         "the clip family's embeddings='save' / 'load' already serve any instruction")
     # instruction sets this pass cannot label are refused before the dataset is opened or an engine is built
     target_keys = _target_keys(model_type, inst_type, extra_instructions)
     _text_groups(model_type, text, extra_instructions)
@@ -486,27 +542,28 @@ def label_reward(
                     (model_ckpt_dir, sd)
                 for img_key in image_keys:
                     sigs[img_key] = embedding_signature(model_type, arch, g[img_key].shape[-3:-1], use_crop, precision,
-                                                        sd)
+                                                        sd, tower=tower)
                     _check_stored_embeddings(g, img_key, model_type, off, n_eps, sigs[img_key], embeddings)
             labeler = RewardLabeler(model_type, text, (int(H), int(W)), model_ckpt_dir=model_ckpt_dir,
                                     clip_state_dict=clip_state_dict, arch=arch, use_crop=use_crop, reduce=reduce,
                                     max_batch=max_batch, device=device, precision=precision, tokenizer=tokenizer,
-                                    extra_instructions=extra_instructions, relabel_only=embeddings == "load")
+                                    extra_instructions=extra_instructions, relabel_only=embeddings == "load",
+                                    tower_only=embeddings == "load_tower")
             _mark("engine + weights + text tower")
             for img_key in image_keys:
-                if embeddings == "load":
-                    key, first = embedding_key(img_key, model_type), int(off[0])
+                if stored == "load":
+                    key, first = _stored_key(img_key, model_type, tower), int(off[0])
                     emb = np.ascontiguousarray(g[key][int(off[e_lo]) - first:int(off[e_hi]) - first], np.float32)
-                    results[img_key] = _label_embedding_rows(labeler, emb, off, e_lo, e_hi, num_frames, n_groups)
+                    results[img_key] = _label_embedding_rows(labeler, emb, off, e_lo, e_hi, num_frames, n_groups, tower)
                     continue
                 ds = g[img_key]
                 side = g.get(img_key + SIDECAR_SUFFIX)
                 if side is not None and (side.shape[0] != ds.shape[0] or tuple(side.shape[1:]) != tuple(ds.shape[2:])):
                     side = None                      # stale or foreign sidecar: fall back to the stacked dataset
-                if embeddings == "save":
-                    embs[img_key] = _embed_rows(labeler, ds, side, off, e_lo, e_hi, slab_frames)
+                if stored == "save":
+                    embs[img_key] = _embed_rows(labeler, ds, side, off, e_lo, e_hi, slab_frames, tower)
                     results[img_key] = _label_embedding_rows(labeler, embs[img_key], off, e_lo, e_hi, num_frames,
-                                                             n_groups)
+                                                             n_groups, tower)
                 else:
                     results[img_key] = _label_rows(labeler, ds, side, off, e_lo, e_hi, num_frames, slab_frames, n_groups)
             _mark("label (decode + encoder + head + scan, H2D / D2H)")
@@ -532,7 +589,7 @@ def label_reward(
                 if rank == 0:
                     full = full.cpu().numpy()
                     results[img_key] = [np.ascontiguousarray(full[:, k]) for k in range(full.shape[1])]
-                if embeddings == "save":             # the second gather: every rank's embeddings to rank 0
+                if stored == "save":                 # the second gather: every rank's embeddings (records) to rank 0
                     full = gather_rows(torch.from_numpy(embs[img_key]).to(cdev), rows, dst=0)
                     embs[img_key] = full.cpu().numpy() if rank == 0 else None
     finally:
@@ -547,8 +604,9 @@ def label_reward(
         try:
             for img_key in image_keys:
                 _write_labels(g, img_key, target_keys, results[img_key], off, n_eps, len_data, num_frames)
-                if embeddings == "save" and n_eps > 0:
-                    _write_embeddings(g, embedding_key(img_key, model_type), embs[img_key], sigs[img_key])
+                if stored == "save" and n_eps > 0:
+                    _write_embeddings(g, _stored_key(img_key, model_type, tower), embs[img_key], sigs[img_key],
+                                      embeddings)
         finally:
             g.close()
     _mark("write labels")
@@ -653,69 +711,84 @@ def _label_rows(labeler, ds, side, off, e_lo: int, e_hi: int, num_frames: int, s
     return _pairs(np.concatenate(parts_r, axis=1), np.concatenate(parts_g, axis=1))
 
 
-def _embed_rows(labeler, ds, side, off, e_lo: int, e_hi: int, slab_frames: int) -> np.ndarray:
-    """float32 [rows, dim]: the stored embedding of every row of episodes [e_lo, e_hi), read from the container as
-    _label_rows reads it (same calls, same chunking of the encoder pass)."""
+def _embed_rows(labeler, ds, side, off, e_lo: int, e_hi: int, slab_frames: int, tower: bool = False) -> np.ndarray:
+    """float32 [rows, dim]: the stored embedding (tower: the CLIP tower record) of every row of episodes [e_lo, e_hi),
+    read from the container as _label_rows reads it (same calls, same chunking of the encoder pass)."""
+    embed_file, embed_slab = ("embed_tower_file", "embed_tower_slab") if tower else ("embed_file", "embed_slab")
+    dim = labeler.tower_dim if tower else labeler.embedding_dim
     lo_all, hi_all = int(off[e_lo]), int(off[e_hi])
     if hi_all <= lo_all:
-        return np.zeros((0, labeler.embedding_dim), np.float32)
+        return np.zeros((0, dim), np.float32)
     src = side if side is not None else ds
-    frows = _file_rows(labeler, src, "embed_file", lo_all)
+    frows = _file_rows(labeler, src, embed_file, lo_all)
     if frows is not None:
         path, first, stride = frows
         fd = os.open(path, os.O_RDONLY)
         try:
-            return labeler.embed_file(fd, first, hi_all - lo_all, stride)
+            return getattr(labeler, embed_file)(fd, first, hi_all - lo_all, stride)
         finally:
             os.close(fd)
     arr = getattr(src, "array", None)
     if arr is not None and arr.flags.c_contiguous:
-        return labeler.embed_slab(arr[lo_all:hi_all])
-    parts = [labeler.embed_slab(rows) for _, _, rows in _read_slabs(ds, side, off, e_lo, e_hi, slab_frames)]
-    return np.concatenate(parts) if parts else np.zeros((0, labeler.embedding_dim), np.float32)
+        return getattr(labeler, embed_slab)(arr[lo_all:hi_all])
+    parts = [getattr(labeler, embed_slab)(rows) for _, _, rows in _read_slabs(ds, side, off, e_lo, e_hi, slab_frames)]
+    return np.concatenate(parts) if parts else np.zeros((0, dim), np.float32)
 
 
-def _label_embedding_rows(labeler, emb: np.ndarray, off, e_lo: int, e_hi: int, num_frames: int, n_groups: int = 1):
-    """_label_rows' result from the stored embeddings of the same rows, labeled in one call on the device"""
+def _label_embedding_rows(labeler, emb: np.ndarray, off, e_lo: int, e_hi: int, num_frames: int, n_groups: int = 1,
+                          tower: bool = False):
+    """_label_rows' result from the stored embeddings (tower: CLIP tower records) of the same rows, labeled in one call
+    on the device"""
     lo_all, hi_all = int(off[e_lo]), int(off[e_hi])
     if hi_all <= lo_all:
         return _empty_pairs(labeler, n_groups, num_frames)
     rel = off[e_lo:e_hi + 1] - lo_all
-    r, _, rs, gs = labeler.label_embeddings(emb, rel, num_frames)
+    label = labeler.label_tower if tower else labeler.label_embeddings
+    r, _, rs, gs = label(emb, rel, num_frames)
     return _pairs(*_finish(labeler, r, rs, gs, rel, num_frames))
 
 
-def _check_stored_embeddings(g, img_key, model_type, off, n_eps, sig, mode):
-    """"load": the embedding dataset and its signature exist, cover the labeled rows and match `sig`. "save": an existing
-    embedding dataset has the shape this pass writes. ValueError otherwise."""
-    key = embedding_key(img_key, model_type)
-    shape = (int(off[n_eps] - off[0]) if n_eps > 0 else 0, EMBEDDING_DIM[embedding_family(model_type)])
+def _stored_key(img_key: str, model_type: str, tower: bool) -> str:
+    return tower_key(img_key) if tower else embedding_key(img_key, model_type)
+
+
+def _check_stored_embeddings(g, img_key, model_type, off, n_eps, sig, embeddings):
+    """"load" / "load_tower": the embedding (tower record) dataset and its signature exist, cover the labeled rows and
+    match `sig`. "save" / "save_tower": an existing dataset has the shape this pass writes. ValueError otherwise."""
+    tower = embeddings in ("save_tower", "load_tower")
+    key = _stored_key(img_key, model_type, tower)
+    shape = (int(off[n_eps] - off[0]) if n_eps > 0 else 0,
+             TOWER_DIM if tower else EMBEDDING_DIM[embedding_family(model_type)])
     ds = g.get(key)
-    if mode == "save":
+    if embeddings in ("save", "save_tower"):
         if ds is not None and tuple(ds.shape) != shape:
-            raise ValueError(f"embeddings='save': {key} exists with shape {tuple(ds.shape)}, this pass writes {shape}")
+            raise ValueError(f"embeddings={embeddings!r}: {key} exists with shape {tuple(ds.shape)}, this pass writes "
+                             f"{shape}")
         return
+    save = "save_tower" if tower else "save"
     if ds is None:
-        raise ValueError(f"embeddings='load': no dataset {key}; label once with embeddings='save'")
+        raise ValueError(f"embeddings={embeddings!r}: no dataset {key}; label once with embeddings={save!r}")
     sds = g.get(key + "_sig")
     if sds is None:
-        raise ValueError(f"embeddings='load': {key} has no signature dataset {key}_sig")
+        raise ValueError(f"embeddings={embeddings!r}: {key} has no signature dataset {key}_sig")
     if tuple(ds.shape) != shape:
-        raise ValueError(f"embeddings='load': {key} has shape {tuple(ds.shape)}, the labeled rows need {shape}")
+        raise ValueError(f"embeddings={embeddings!r}: {key} has shape {tuple(ds.shape)}, the labeled rows need {shape}")
     stored = np.asarray(sds[:], np.uint8).reshape(-1)
     if not np.array_equal(stored, sig):
-        raise ValueError(f"embeddings='load': the signature of {key} differs: it was saved with another checkpoint, crop, "
-                         "frame size, arch or precision")
+        what = "CLIP weights" if tower else "checkpoint"
+        raise ValueError(f"embeddings={embeddings!r}: the signature of {key} differs: it was saved with another {what}, "
+                         "crop, frame size, arch or precision")
 
 
-def _write_embeddings(g, key, emb: np.ndarray, sig: np.ndarray):
+def _write_embeddings(g, key, emb: np.ndarray, sig: np.ndarray, embeddings: str = "save"):
     """float32 [rows, dim] uncompressed (assigned in place when it exists with this shape) + the uint8 [32] signature"""
     for k, a in ((key, np.ascontiguousarray(emb, np.float32)), (key + "_sig", sig)):
         existing = g.get(k)
         if existing is None:
             g.create_dataset(k, data=a)
         elif tuple(existing.shape) != a.shape:
-            raise ValueError(f"embeddings='save': {k} exists with shape {tuple(existing.shape)}, this pass writes {a.shape}")
+            raise ValueError(f"embeddings={embeddings!r}: {k} exists with shape {tuple(existing.shape)}, this pass "
+                             f"writes {a.shape}")
         else:
             existing[...] = a
 
@@ -781,8 +854,10 @@ def main():
     parser.add_argument("--tokenizer", type=str, default=None, choices=["clip", "standin"])
     parser.add_argument("--extra_inst_types", type=str, default=None,
                         help="comma-separated inst_types labeled in the same pass as --inst_type, e.g. random1,misinfo")
-    parser.add_argument("--embeddings", type=str, default=None, choices=["save", "load"],
-                        help="save: also store per-frame image embeddings; load: label from stored embeddings, no frames")
+    parser.add_argument("--embeddings", type=str, default=None, choices=["save", "load", "save_tower", "load_tower"],
+                        help="save: also store per-frame image embeddings; load: label from stored embeddings, no frames; "
+                             "save_tower / load_tower (adapter model types): the same with CLIP tower records, which "
+                             "relabel with any adapter checkpoint fine-tuned from the same CLIP")
     args = parser.parse_args()
 
     env_name = f"{args.env_name}" if args.env_type == "none" else f"{args.env_name}_{args.env_type}"

@@ -22,6 +22,15 @@
  * and return one fp32 vector per frame; arp_label_embeddings runs the instruction side on such vectors, with no frames
  * and no image-side weights, and gives arp_label's outputs bit for bit. A new instruction, inst_type, reduce mode or
  * text-head variant of the same checkpoint then costs a read of the vectors and one memory-bound head launch.
+ *
+ * CLIP tower records (adapter heads): the adapter heads' stored embedding depends on the adapter checkpoint, but
+ * fine-tuning freezes CLIP, so what the adapter reads from the CLIP tower is the same for every checkpoint made from the
+ * same CLIP. arp_embed_tower_host / arp_embed_tower_file run the frozen tower once and return one fp32 record of
+ * arp_tower_dim() = 12*768 + 512 = 9728 floats per frame: the 12 class-token taps (block l at columns [l*768, (l+1)*768),
+ * each the value the image_intermediate_linear GEMM multiplies), then the un-normalised CLIP feature. arp_label_tower
+ * runs only the adapter (three GEMMs, the gate, the head) and the scan on such records, with no frames and no visual.*
+ * weights, and gives arp_label's outputs bit for bit — also for an adapter checkpoint other than the one the records were
+ * written with. A new fine-tuned adapter then costs 0.468 GFLOP per frame instead of the ViT's 35.1.
  */
 #ifndef ARP_B200_H_
 #define ARP_B200_H_
@@ -32,7 +41,7 @@
 extern "C" {
 #endif
 
-#define ARP_B200_ABI_VERSION 7   /* 3: + arp_encode_taps_chw, 4: + arp_operand_dtype, 5: + ARP_PREC_F32RESID, arp_ln_gemm, arp_resid_gemm_stats, arp_label_file, arp_wants_weight, 6: + arp_set_text_groups, arp_text_groups, 7: + arp_embedding_dim, arp_embed_host, arp_embed_file, arp_label_embeddings */
+#define ARP_B200_ABI_VERSION 8   /* 3: + arp_encode_taps_chw, 4: + arp_operand_dtype, 5: + ARP_PREC_F32RESID, arp_ln_gemm, arp_resid_gemm_stats, arp_label_file, arp_wants_weight, 6: + arp_set_text_groups, arp_text_groups, 7: + arp_embedding_dim, arp_embed_host, arp_embed_file, arp_label_embeddings, 8: + arp_tower_dim, arp_embed_tower_host, arp_embed_tower_file, arp_label_tower */
 
 #define ARP_MAX_TEXT 16          /* texts of one instruction set (arp_set_text's n_text, one group's size) */
 #define ARP_MAX_TEXT_GROUPS 16   /* instruction sets of one arp_set_text_groups call */
@@ -210,6 +219,33 @@ ARP_API int arp_embed_file(ArpHandle* h, int32_t fd, int64_t file_offset, int64_
 ARP_API int arp_label_embeddings(ArpHandle* h, const float* emb_dev, int64_t T, const int64_t* ep_offsets_dev,
                                  int32_t n_eps, int32_t num_frames, float* reward_dev, float* rtg_dev,
                                  float* reward_stacked_dev, float* rtg_stacked_dev, void* stream);
+
+/* CLIP tower record width: 9728 (12 class-token taps of 768 + the 512-wide CLIP feature) for the adapter heads, 0 for the
+ * clip heads. The layout is the same for every precision and operand format. */
+ARP_API int arp_tower_dim(const ArpHandle* h);
+/* The frozen-CLIP side of arp_label_host / arp_label_file on an adapter head, stopped after the CLIP feature: one record
+ * [T, arp_tower_dim] fp32 per frame is written to rec_host. Columns [0, 9216): the class-token taps the adapter's
+ * image_intermediate_linear reads (the 16-bit paths: the operand-format taps widened to fp32, which is exact; block 11's
+ * is the 16-bit rounding of the pruned last block's fp32 class row; ARP_PREC_F32: the fp32 taps). Columns [9216, 9728):
+ * encode_image before normalisation (clip_multiscale_adapter.py:136,145). Same frame arguments, staging and encoder pass
+ * as arp_embed_host; the result is assembled on the device and copied to the host once at the end (T * 38 912 bytes of
+ * device memory, freed before the call returns). Synchronises. ARP_ERR_INVALID on clip heads. */
+ARP_API int arp_embed_tower_host(ArpHandle* h, const uint8_t* ob_host, int64_t T, int64_t row_stride_bytes,
+                                 float* rec_host);
+ARP_API int arp_embed_tower_file(ArpHandle* h, int32_t fd, int64_t file_offset, int64_t T, int64_t row_stride_bytes,
+                                 float* rec_host);
+/* arp_label's outputs ([G,T] / [G,T,F] with text groups, the goal-conditioned adapter head included) from tower records:
+ * rec_dev [T, arp_tower_dim] fp32 DEVICE rows (16-byte aligned) from arp_embed_tower_* of a handle with the same CLIP
+ * weights, arch, frame size, crop and precision; the other arguments and the four outputs are those of arp_label. Needs
+ * only the image-adapter tensors (image_intermediate_linear.weight, image_adapter.layers.{0,3}.*, image_residual_weight):
+ * works on a handle whose visual.* weights were never set, and with any adapter checkpoint of that CLIP. Bit-identical to
+ * arp_label on the frames the records came from, with this handle's adapter. Per max_batch chunk: one unpack launch and
+ * the adapter's launches; one scan for the call. ARP_ERR_INVALID on clip heads, a null or unaligned buffer, T < 0, bad
+ * offsets, num_frames outside [1, 64]; ARP_ERR_STATE when an adapter tensor is missing or a text head has no text.
+ * replaces compute_reward's model(images, text) for a new adapter checkpoint (label_reward.py:200-230) */
+ARP_API int arp_label_tower(ArpHandle* h, const float* rec_dev, int64_t T, const int64_t* ep_offsets_dev,
+                            int32_t n_eps, int32_t num_frames, float* reward_dev, float* rtg_dev,
+                            float* reward_stacked_dev, float* rtg_stacked_dev, void* stream);
 
 /* Latency mode — the online reward of a rollout (arp_dt/envs/vl_reward.py:11-23 get_torch_clip_reward, :44-59
  * get_torch_clip_adapter_reward, and the two encode_image calls of the goal-conditioned variants :26-41, :62-77;
