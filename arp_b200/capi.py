@@ -26,6 +26,9 @@ PREC_BF16, PREC_F32, PREC_F32RESID = 0, 1, 2   # PREC_BF16 = the 16-bit tensor-c
 PREC_16BIT = PREC_BF16
 #: precision names of the Python entry points ("bf16" / "fp16" name the 16-bit path whatever the operand format)
 PRECISIONS = {"16bit": PREC_16BIT, "bf16": PREC_16BIT, "fp16": PREC_16BIT, "fp32resid": PREC_F32RESID, "fp32": PREC_F32}
+#: ArpInflateStatus: per-row result of the device zlib inflate (inflate_rows)
+(ARP_INFLATE_OK, ARP_INFLATE_TRUNCATED, ARP_INFLATE_BAD_HEADER, ARP_INFLATE_BAD_BLOCK, ARP_INFLATE_BAD_CODE,
+ ARP_INFLATE_DISTANCE_TOO_FAR, ARP_INFLATE_TOO_LONG, ARP_INFLATE_TOO_SHORT, ARP_INFLATE_BAD_ADLER) = range(9)
 MAX_TEXT = 16            # texts of one instruction set (one text group)
 MAX_TEXT_GROUPS = 16     # instruction sets of one set_text_groups call
 MAX_TEXT_TOTAL = 64      # texts of all groups together
@@ -39,6 +42,7 @@ EXPORTS = (
     "arp_quantile_f32", "arp_encode_taps_chw", "arp_operand_dtype", "arp_ln_gemm", "arp_resid_gemm_stats", "arp_label_file", "arp_wants_weight",
     "arp_set_text_groups", "arp_text_groups", "arp_embedding_dim", "arp_embed_host", "arp_embed_file",
     "arp_label_embeddings", "arp_tower_dim", "arp_embed_tower_host", "arp_embed_tower_file", "arp_label_tower",
+    "arp_label_zfile", "arp_embed_zfile", "arp_embed_tower_zfile", "arp_inflate_rows",
 )
 PROFILE_CLASSES = ("gemm", "attention", "layernorm", "decode", "head", "scan", "other")
 
@@ -108,6 +112,10 @@ def load_library() -> C.CDLL:
     lib.arp_embed_tower_host.argtypes = [vp, vp, i64, i64, vp]
     lib.arp_embed_tower_file.argtypes = [vp, i32, i64, i64, i64, vp]
     lib.arp_label_tower.argtypes = [vp, vp, i64, vp, i32, i32, vp, vp, vp, vp, vp]
+    lib.arp_label_zfile.argtypes = [vp, i32, vp, vp, i64, i64, vp, i32, i32, vp, vp, vp, vp]
+    lib.arp_embed_zfile.argtypes = [vp, i32, vp, vp, i64, i64, vp]
+    lib.arp_embed_tower_zfile.argtypes = [vp, i32, vp, vp, i64, i64, vp]
+    lib.arp_inflate_rows.argtypes = [vp, vp, vp, vp, i64, i64, vp, vp, vp]
     lib.arp_compute_reward.argtypes = [vp, vp, i64, i64, vp, vp, vp]
     lib.arp_online_reward.argtypes = [vp, vp, i32, vp, vp, vp]
     lib.arp_preprocess_rtgs.argtypes = [vp, vp, i64, vp, i32, i32, i32, vp, vp, vp, vp, vp]
@@ -439,6 +447,60 @@ class Engine:
         self._check(self._lib.arp_label_tower(self._h, _ptr(x), T, _ptr(off), off.numel() - 1, num_frames, _ptr(r),
                                               _ptr(g), _ptr(rs), _ptr(gs), _stream_ptr(self.device)))
         return r, g, rs, gs
+
+    # -- compressed rows (gzip-chunked HDF5) --------------------------------------------------------
+    @staticmethod
+    def _chunk_table(chunk_offsets, chunk_bytes):
+        off = np.ascontiguousarray(chunk_offsets, dtype=np.int64)
+        nb = np.ascontiguousarray(chunk_bytes, dtype=np.int64)
+        assert off.ndim == 1 and off.shape == nb.shape, (off.shape, nb.shape)
+        return off, nb, C.c_void_p(off.ctypes.data), C.c_void_p(nb.ctypes.data)
+
+    def label_zfile(self, fd: int, chunk_offsets: np.ndarray, chunk_bytes: np.ndarray, row_bytes: int,
+                    ep_offsets: np.ndarray, num_frames: int, out=None):
+        """arp_label_zfile: label_file's outputs when row t is the zlib stream of chunk_bytes[t] bytes at file offset
+        chunk_offsets[t] of `fd`, inflating to row_bytes = F*H*W*3 bytes (F stacked frames, the last one scored)."""
+        off, nb, p_off, p_nb = self._chunk_table(chunk_offsets, chunk_bytes)
+        ep = np.ascontiguousarray(ep_offsets, dtype=np.int64)
+        T = off.size
+        if out is None:
+            out = self._host_outputs(T, num_frames)
+        hp = lambda a: C.c_void_p(a.ctypes.data)  # noqa: E731
+        self._check(self._lib.arp_label_zfile(self._h, int(fd), p_off, p_nb, T, int(row_bytes), hp(ep), ep.size - 1,
+                                              num_frames, hp(out[0]), hp(out[1]), hp(out[2]), hp(out[3])))
+        return out
+
+    def embed_zfile(self, fd: int, chunk_offsets: np.ndarray, chunk_bytes: np.ndarray, row_bytes: int,
+                    out: "np.ndarray | None" = None) -> np.ndarray:
+        """arp_embed_zfile: embed_file's result from compressed rows as label_zfile takes them."""
+        off, nb, p_off, p_nb = self._chunk_table(chunk_offsets, chunk_bytes)
+        out = self._emb_out(off.size, out)
+        self._check(self._lib.arp_embed_zfile(self._h, int(fd), p_off, p_nb, off.size, int(row_bytes),
+                                              C.c_void_p(out.ctypes.data)))
+        return out
+
+    def embed_tower_zfile(self, fd: int, chunk_offsets: np.ndarray, chunk_bytes: np.ndarray, row_bytes: int,
+                          out: "np.ndarray | None" = None) -> np.ndarray:
+        """arp_embed_tower_zfile: embed_tower_file's result from compressed rows as label_zfile takes them."""
+        off, nb, p_off, p_nb = self._chunk_table(chunk_offsets, chunk_bytes)
+        out = self._emb_out(off.size, out, self.tower_dim)
+        self._check(self._lib.arp_embed_tower_zfile(self._h, int(fd), p_off, p_nb, off.size, int(row_bytes),
+                                                    C.c_void_p(out.ctypes.data)))
+        return out
+
+    def inflate_rows(self, src: torch.Tensor, src_offsets: torch.Tensor, src_bytes: torch.Tensor, row_bytes: int):
+        """arp_inflate_rows on device tensors: uint8 src (concatenated zlib streams), int64 offsets and sizes [n] ->
+        (uint8 rows [n, row_bytes], int32 ArpInflateStatus [n]). Rows that fail are zero past where they stopped."""
+        assert src.dtype == torch.uint8 and src.is_cuda and src.is_contiguous()
+        so = src_offsets.to(self.device, torch.int64).contiguous()
+        sb = src_bytes.to(self.device, torch.int64).contiguous()
+        n = so.numel()
+        assert sb.numel() == n
+        out = torch.zeros((n, int(row_bytes)), device=self.device, dtype=torch.uint8)
+        status = torch.full((n,), -1, device=self.device, dtype=torch.int32)
+        self._check(self._lib.arp_inflate_rows(self._h, _ptr(src), _ptr(so), _ptr(sb), n, int(row_bytes), _ptr(out),
+                                               _ptr(status), _stream_ptr(self.device)))
+        return out, status
 
     def compute_reward(self, ob: torch.Tensor, want_logits: bool = False):
         """reward [T] (or [G, T] after set_text_groups); logits [T, n_text] over the texts of all groups."""

@@ -32,6 +32,7 @@
 #include "fp32_path.cuh"
 #include "gemm_tcgen05.cuh"
 #include "head.cuh"
+#include "inflate.cuh"
 #include "layernorm.cuh"
 #include "rtgstats.cuh"
 #include "scan.cuh"
@@ -177,6 +178,14 @@ struct ArpHandle {
   size_t scratch_bytes[2] = {0, 0};
   uint8_t* stage_dev[2] = {nullptr, nullptr};
   size_t stage_bytes = 0;
+  // compressed-row entry points (arp_*_zfile): two device buffers of one chunk's compressed rows, the inflated rows of one
+  // chunk [max_batch, row_bytes], and the call's per-row tables (packed offset, size, inflate status)
+  uint8_t* zsrc_dev[2] = {nullptr, nullptr};
+  size_t zsrc_bytes = 0;
+  uint8_t* zrows_dev = nullptr;
+  size_t zrows_bytes = 0;
+  void* ztab_dev = nullptr;
+  size_t ztab_bytes = 0;
   uint8_t* pin_ring = nullptr;     // pinned staging ring for pageable callers of arp_label_host (STG_SLOTS x STG_SUB frames)
   size_t pin_bytes = 0;
   cudaEvent_t ev_slot[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
@@ -516,9 +525,12 @@ extern "C" void arp_destroy(ArpHandle* h) {
   for (int i = 0; i < 2; ++i) if (h->scratch[i]) cudaFree(h->scratch[i]);
   for (int i = 0; i < 2; ++i) {
     if (h->stage_dev[i]) cudaFree(h->stage_dev[i]);
+    if (h->zsrc_dev[i]) cudaFree(h->zsrc_dev[i]);
     if (h->ev_copied[i]) cudaEventDestroy(h->ev_copied[i]);
     if (h->ev_consumed[i]) cudaEventDestroy(h->ev_consumed[i]);
   }
+  if (h->zrows_dev) cudaFree(h->zrows_dev);
+  if (h->ztab_dev) cudaFree(h->ztab_dev);
   if (h->pin_ring) cudaFreeHost(h->pin_ring);
   for (cudaEvent_t e : h->ev_slot) if (e) cudaEventDestroy(e);
   for (auto& kv : h->online_graphs) if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
@@ -1411,12 +1423,17 @@ __global__ void episode_goal_kernel(const long long* __restrict__ ep_off, int n_
   for (long long t = lo + threadIdx.x; t < hi; t += blockDim.x) frame_goal[t] = hi - 1;
 }
 
-static int ensure_scratch(ArpHandle* h, int slot, size_t bytes) {
-  if (h->scratch_bytes[slot] >= bytes) return ARP_OK;
-  if (h->scratch[slot]) { cudaDeviceSynchronize(); cudaFree(h->scratch[slot]); h->scratch[slot] = nullptr; h->scratch_bytes[slot] = 0; }
-  ARP_CUDA(h, cudaMalloc(&h->scratch[slot], bytes));
-  h->scratch_bytes[slot] = bytes;
+// a device buffer *p of *have bytes grown to at least need (contents not kept)
+static int grow(ArpHandle* h, void** p, size_t* have, size_t need) {
+  if (*have >= need) return ARP_OK;
+  if (*p) { cudaDeviceSynchronize(); cudaFree(*p); *p = nullptr; *have = 0; }
+  ARP_CUDA(h, cudaMalloc(p, need));
+  *have = need;
   return ARP_OK;
+}
+
+static int ensure_scratch(ArpHandle* h, int slot, size_t bytes) {
+  return grow(h, &h->scratch[slot], &h->scratch_bytes[slot], bytes);
 }
 
 // temporaries of one label call, carved from scratch slot 0
@@ -1607,8 +1624,9 @@ static bool host_ptr_is_pinned(const void* p) {
   return a.type == cudaMemoryTypeHost;   // pageable memory reports cudaMemoryTypeUnregistered
 }
 
-static int ensure_pinned_ring(ArpHandle* h, size_t frame_bytes) {
-  const size_t need = frame_bytes * STG_SUB * STG_SLOTS;
+// row_bytes: the ring's row pitch (a frame, or the largest compressed chunk of a zfile call)
+static int ensure_pinned_ring(ArpHandle* h, size_t row_bytes) {
+  const size_t need = row_bytes * STG_SUB * STG_SLOTS;
   if (h->pin_bytes >= need) return ARP_OK;
   if (h->pin_ring) { cudaFreeHost(h->pin_ring); h->pin_ring = nullptr; h->pin_bytes = 0; }
   ARP_CUDA(h, cudaHostAlloc((void**)&h->pin_ring, need, cudaHostAllocDefault));
@@ -1621,9 +1639,25 @@ static int ensure_pinned_ring(ArpHandle* h, size_t frame_bytes) {
 struct SubChunk { int64_t t0; int n; };   // rows [t0, t0+n) of the call, never straddling a device chunk
 
 // gathers sub-chunk after sub-chunk into the pinned ring; the main thread consumes them in order
+// pread() exactly n bytes at off; 0, errno, or -1 at end of file
+static int pread_full(int fd, uint8_t* dst, size_t n, int64_t off) {
+  size_t got = 0;
+  while (got < n) {
+    const ssize_t r = pread(fd, dst + got, n - got, (off_t)(off + (int64_t)got));
+    if (r <= 0) return r == 0 ? -1 : errno;
+    got += (size_t)r;
+  }
+  return 0;
+}
+
+// compressed rows of a zfile call: row t is the zlib stream of bytes[t] bytes at file offset off[t]; pos[t] is its byte
+// offset in its device chunk's packed buffer
+struct ZRows { const int64_t* off; const int64_t* bytes; std::vector<int64_t> pos; int64_t row_bytes; int64_t max_chunk; };
+
 struct HostStager {
   const uint8_t* src; int64_t stride; size_t frame_bytes; uint8_t* ring; cudaEvent_t* ev_slot; int device;
   int fd = -1; int64_t fd_base = 0;          // fd >= 0: rows are pread() from a file (no page-table traffic) instead of src
+  const ZRows* z = nullptr;                  // compressed rows: a slot holds its rows' chunks packed, pitch frame_bytes
   std::atomic<int> io_error{0};
   const std::vector<SubChunk>* subs;
   std::atomic<int64_t> next{0}, issued{0};   // next task to start | sub-chunks whose H2D has been enqueued
@@ -1648,18 +1682,17 @@ struct HostStager {
       }
       const SubChunk& sc = (*subs)[j];
       uint8_t* dst = ring + (size_t)slot * STG_SUB * frame_bytes;
-      if (fd < 0) {
+      if (z) {
+        for (int f = 0; f < sc.n && !io_error.load(); ++f) {
+          const int64_t t = sc.t0 + f;
+          if (const int e = pread_full(fd, dst + (z->pos[t] - z->pos[sc.t0]), (size_t)z->bytes[t], z->off[t])) io_error.store(e);
+        }
+      } else if (fd < 0) {
         for (int f = 0; f < sc.n; ++f) memcpy(dst + (size_t)f * frame_bytes, src + (sc.t0 + f) * stride, frame_bytes);
       } else {
-        for (int f = 0; f < sc.n && !io_error.load(); ++f) {
-          size_t got = 0;
-          while (got < frame_bytes) {
-            const ssize_t r = pread(fd, dst + (size_t)f * frame_bytes + got, frame_bytes - got,
-                                    (off_t)(fd_base + (sc.t0 + f) * stride + (int64_t)got));
-            if (r <= 0) { io_error.store(r == 0 ? -1 : errno); break; }
-            got += (size_t)r;
-          }
-        }
+        for (int f = 0; f < sc.n && !io_error.load(); ++f)
+          if (const int e = pread_full(fd, dst + (size_t)f * frame_bytes, frame_bytes, fd_base + (sc.t0 + f) * stride))
+            io_error.store(e);
       }
       { std::lock_guard<std::mutex> lk(mu); done[j] = 1; }
       cv.notify_all();
@@ -1683,6 +1716,99 @@ struct HostStager {
   void stop() { abort.store(true); for (auto& t : threads) t.join(); threads.clear(); }
 };
 
+// ---- compressed rows (arp_*_zfile) --------------------------------------------------------------------------------
+struct ZDev { int64_t* pos = nullptr; int64_t* bytes = nullptr; int* status = nullptr; };   // [T] each, device
+
+static int launch_inflate(ArpHandle* h, const uint8_t* src, const int64_t* off, const int64_t* bytes, int64_t n,
+                          int64_t row_bytes, uint8_t* out, int* status, cudaStream_t st) {
+  if (n <= 0) return ARP_OK;
+  ProfScope prof(h, PC_DECODE, 0.0, (double)n * row_bytes * 2, st);
+  arp_inflate::inflate_rows_kernel<<<(unsigned)((n + arp_inflate::INF_WARPS - 1) / arp_inflate::INF_WARPS),
+                                     arp_inflate::INF_WARPS * 32, 0, st>>>(src, off, bytes, (int)n, row_bytes, out, status);
+  h->launches++;
+  ARP_CUDA(h, cudaGetLastError());
+  return ARP_OK;
+}
+
+// packs each max_batch chunk's compressed rows back to back (z->pos), sizes the device buffers from the call's largest
+// chunk, and uploads the per-row tables
+static int prepare_zrows(ArpHandle* h, ZRows* z, int64_t T, int64_t B, ZDev* zd, cudaStream_t st) {
+  z->pos.assign((size_t)T, 0);
+  size_t zsrc = 1;
+  z->max_chunk = 1;
+  for (int64_t t0 = 0; t0 < T; t0 += B) {
+    int64_t p = 0;
+    for (int64_t t = t0; t < std::min(T, t0 + B); ++t) {
+      z->pos[t] = p;
+      p += z->bytes[t];
+      z->max_chunk = std::max(z->max_chunk, z->bytes[t]);
+    }
+    zsrc = std::max(zsrc, (size_t)p);
+  }
+  if (h->zsrc_bytes < zsrc) {
+    for (int i = 0; i < 2; ++i) {
+      size_t have = h->zsrc_bytes;
+      ARP_TRY(grow(h, reinterpret_cast<void**>(&h->zsrc_dev[i]), &have, zsrc));
+    }
+    h->zsrc_bytes = zsrc;
+  }
+  ARP_TRY(grow(h, reinterpret_cast<void**>(&h->zrows_dev), &h->zrows_bytes, (size_t)std::min(B, T) * z->row_bytes));
+  ARP_TRY(grow(h, &h->ztab_dev, &h->ztab_bytes, (size_t)T * 20));
+  zd->pos = reinterpret_cast<int64_t*>(h->ztab_dev);
+  zd->bytes = zd->pos + T;
+  zd->status = reinterpret_cast<int*>(zd->bytes + T);
+  ARP_CUDA(h, cudaMemcpyAsync(zd->pos, z->pos.data(), (size_t)T * 8, cudaMemcpyHostToDevice, st));
+  ARP_CUDA(h, cudaMemcpyAsync(zd->bytes, z->bytes, (size_t)T * 8, cudaMemcpyHostToDevice, st));
+  return ARP_OK;
+}
+
+static const char* inflate_status_name(int s) {
+  switch (s) {
+    case ARP_INFLATE_TRUNCATED: return "truncated stream";
+    case ARP_INFLATE_BAD_HEADER: return "bad zlib header";
+    case ARP_INFLATE_BAD_BLOCK: return "bad block type or stored length";
+    case ARP_INFLATE_BAD_CODE: return "bad Huffman code";
+    case ARP_INFLATE_DISTANCE_TOO_FAR: return "distance before the start of the row";
+    case ARP_INFLATE_TOO_LONG: return "output longer than row_bytes";
+    case ARP_INFLATE_TOO_SHORT: return "output shorter than row_bytes";
+    case ARP_INFLATE_BAD_ADLER: return "Adler-32 mismatch";
+    default: return "unknown status";
+  }
+}
+
+// ARP_ERR_INVALID naming the first row that did not inflate
+static int check_zrows(ArpHandle* h, const ZRows& z, const ZDev& zd, int64_t T, cudaStream_t st) {
+  std::vector<int> status((size_t)T);
+  ARP_CUDA(h, cudaMemcpyAsync(status.data(), zd.status, (size_t)T * 4, cudaMemcpyDeviceToHost, st));
+  ARP_CUDA(h, cudaStreamSynchronize(st));
+  for (int64_t t = 0; t < T; ++t)
+    if (status[t] != ARP_INFLATE_OK)
+      return fail(h, ARP_ERR_INVALID, "row %lld of the call (chunk at file offset %lld, %lld bytes) does not inflate to "
+                  "%lld bytes: %s (ArpInflateStatus %d)", (long long)t, (long long)z.off[t], (long long)z.bytes[t],
+                  (long long)z.row_bytes, inflate_status_name(status[t]), status[t]);
+  return ARP_OK;
+}
+
+// the checks the zfile entry points share; row_bytes must be F whole frames, F in [1, 64]
+static int check_row_bytes(ArpHandle* h, int64_t row_bytes) {
+  const int64_t frame = (int64_t)h->cfg.in_h * h->cfg.in_w * 3;
+  if (row_bytes <= 0 || row_bytes % frame != 0 || row_bytes / frame > 64)
+    return fail(h, ARP_ERR_INVALID, "row_bytes %lld is not F * %lld with F in [1, 64]", (long long)row_bytes, (long long)frame);
+  return ARP_OK;
+}
+
+static int check_zargs(ArpHandle* h, int32_t fd, const int64_t* off, const int64_t* bytes, int64_t T, int64_t row_bytes) {
+  if (!h) return ARP_ERR_INVALID;
+  if (fd < 0) return fail(h, ARP_ERR_INVALID, "bad file descriptor");
+  if (T < 0) return fail(h, ARP_ERR_INVALID, "bad T");
+  if (T > 0 && (!off || !bytes)) return fail(h, ARP_ERR_INVALID, "null chunk table");
+  ARP_TRY(check_row_bytes(h, row_bytes));
+  for (int64_t t = 0; t < T; ++t)
+    if (off[t] < 0 || bytes[t] < 0)
+      return fail(h, ARP_ERR_INVALID, "row %lld: negative chunk offset or size", (long long)t);
+  return ARP_OK;
+}
+
 // arp_embed_tower_*: the adapter head stopped after the CLIP feature; the chunk's taps and feature become n tower records
 static int tower_chunk(ArpHandle* h, int64_t n, float* rec, cudaStream_t st) {
   ArpHandle::Work& ws = h->ws;
@@ -1705,7 +1831,7 @@ static int tower_chunk(ArpHandle* h, int64_t n, float* rec, cudaStream_t st) {
 static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t fd_offset, int64_t T,
                            int64_t row_stride_bytes, const int64_t* ep_offsets_host, int32_t n_eps, int32_t num_frames,
                            float* reward_host, float* rtg_host, float* reward_stacked_host, float* rtg_stacked_host,
-                           float* emb_host = nullptr, bool tower = false) {
+                           float* emb_host = nullptr, bool tower = false, ZRows* z = nullptr) {
   if (!h) return ARP_ERR_INVALID;
   cudaStream_t st = h->own_stream;
   const bool embed = emb_host != nullptr;
@@ -1720,6 +1846,8 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
   const int64_t B = c.max_batch;
   const int F = embed ? 1 : num_frames;
   ARP_TRY(ensure_stage(h));
+  ZDev zd;
+  if (z) ARP_TRY(prepare_zrows(h, z, T, B, &zd, st));
   // device outputs (scratch slot 1), G = n_groups:
   // [ep_off (n_eps+1) i64][reward G*T][rtg G*T][reward_stacked G*T*F][rtg_stacked G*T*F]; embed mode: [emb T*ew]
   const size_t G = (size_t)h->n_groups;
@@ -1740,17 +1868,18 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
   // pinned (or registered) caller memory goes to the device directly, one strided 2-D copy per chunk; pageable memory is
   // gathered through the pinned ring by worker threads
   const bool staged = fd >= 0 || !host_ptr_is_pinned(ob_host);
+  const size_t pitch = z ? (size_t)z->max_chunk : frame_bytes;   // pinned ring: bytes per row of a slot
   std::vector<SubChunk> subs;
   HostStager stager;
   if (staged) {
-    ARP_TRY(ensure_pinned_ring(h, frame_bytes));
+    ARP_TRY(ensure_pinned_ring(h, pitch));
     for (int64_t ci = 0; ci < nchunks; ++ci) {
       const int64_t t0 = ci * B, n = std::min(B, T - t0);
       for (int64_t s0 = 0; s0 < n; s0 += STG_SUB) subs.push_back(SubChunk{t0 + s0, (int)std::min<int64_t>(STG_SUB, n - s0)});
     }
-    stager.src = ob_host; stager.stride = row_stride_bytes; stager.frame_bytes = frame_bytes; stager.ring = h->pin_ring;
+    stager.src = ob_host; stager.stride = row_stride_bytes; stager.frame_bytes = pitch; stager.ring = h->pin_ring;
     stager.ev_slot = h->ev_slot; stager.device = c.device; stager.subs = &subs;
-    stager.fd = fd; stager.fd_base = fd_offset;
+    stager.fd = fd; stager.fd_base = fd_offset; stager.z = z;
     stager.start();
   }
   // double-buffered: chunk i+1's frames (only the scored image of each row) cross PCIe while chunk i is encoded
@@ -1768,8 +1897,15 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
       for (int64_t s0 = 0; s0 < n && e == cudaSuccess; s0 += STG_SUB, ++sub_j) {
         stager.wait(sub_j);
         const int slot = (int)(sub_j % STG_SLOTS);
-        e = cudaMemcpyAsync(h->stage_dev[buf] + (size_t)s0 * frame_bytes, h->pin_ring + (size_t)slot * STG_SUB * frame_bytes,
-                            (size_t)subs[sub_j].n * frame_bytes, cudaMemcpyHostToDevice, h->copy_stream);
+        const uint8_t* ring_slot = h->pin_ring + (size_t)slot * STG_SUB * pitch;
+        if (z) {   // the sub-chunk's compressed rows, packed, to their place in the chunk's packed buffer
+          const int64_t a = t0 + s0, b = a + subs[sub_j].n - 1;
+          e = cudaMemcpyAsync(h->zsrc_dev[buf] + z->pos[a], ring_slot, (size_t)(z->pos[b] + z->bytes[b] - z->pos[a]),
+                              cudaMemcpyHostToDevice, h->copy_stream);
+        } else {
+          e = cudaMemcpyAsync(h->stage_dev[buf] + (size_t)s0 * frame_bytes, ring_slot, (size_t)subs[sub_j].n * frame_bytes,
+                              cudaMemcpyHostToDevice, h->copy_stream);
+        }
         if (e == cudaSuccess) e = cudaEventRecord(h->ev_slot[slot], h->copy_stream);
         stager.issued.store(sub_j + 1, std::memory_order_release);
       }
@@ -1777,7 +1913,15 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
     if (e != cudaSuccess) { rc = fail(h, ARP_ERR_CUDA, "H2D frames failed: %s", cudaGetErrorString(e)); break; }
     cudaEventRecord(h->ev_copied[buf], h->copy_stream);
     cudaStreamWaitEvent(st, h->ev_copied[buf], 0);
-    if ((rc = encode_chunk(h, h->stage_dev[buf], n, (int64_t)frame_bytes, st)) != ARP_OK) break;
+    if (z) {   // whole rows inflated into zrows_dev; the encoder reads each row's last frame with stride row_bytes
+      if ((rc = launch_inflate(h, h->zsrc_dev[buf], zd.pos + t0, zd.bytes + t0, n, z->row_bytes, h->zrows_dev,
+                               zd.status + t0, st)) != ARP_OK)
+        break;
+      rc = encode_chunk(h, h->zrows_dev + (z->row_bytes - (int64_t)frame_bytes), n, z->row_bytes, st);
+    } else {
+      rc = encode_chunk(h, h->stage_dev[buf], n, (int64_t)frame_bytes, st);
+    }
+    if (rc != ARP_OK) break;
     if (tower) rc = tower_chunk(h, n, d_emb + t0 * ew, st);
     else if (embed) rc = head_chunk(h, n, nullptr, 0, nullptr, d_emb + t0 * ew, st);
     else if (!h->goal) rc = head_chunk(h, n, d_r + t0, T, nullptr, nullptr, st);
@@ -1793,6 +1937,7 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
       fprintf(stderr, "arp_label_host: %lld frames staged in %zu sub-chunks, consumer waited %.3f s for the gather threads\n",
               (long long)T, subs.size(), stager.waited_s);
   }
+  if (rc == ARP_OK && z) rc = check_zrows(h, *z, zd, T, st);
   if (rc == ARP_OK && embed) {
     cudaError_t e = cudaMemcpyAsync(emb_host, d_emb, (size_t)T * ew * 4, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
@@ -1927,6 +2072,50 @@ extern "C" int arp_embed_tower_file(ArpHandle* h, int32_t fd, int64_t file_offse
   if (T == 0) return check_ready(h, reinterpret_cast<const uint8_t*>(h), T, row_stride_bytes, h->own_stream);
   return label_host_impl(h, nullptr, fd, file_offset, T, row_stride_bytes, nullptr, 0, 0, nullptr, nullptr, nullptr,
                          nullptr, rec_host, true);
+}
+
+extern "C" int arp_label_zfile(ArpHandle* h, int32_t fd, const int64_t* chunk_offset_host, const int64_t* chunk_bytes_host,
+                               int64_t T, int64_t row_bytes, const int64_t* ep_offsets_host, int32_t n_eps,
+                               int32_t num_frames, float* reward_host, float* rtg_host, float* reward_stacked_host,
+                               float* rtg_stacked_host) {
+  ARP_TRY(check_zargs(h, fd, chunk_offset_host, chunk_bytes_host, T, row_bytes));
+  ZRows z{chunk_offset_host, chunk_bytes_host, {}, row_bytes, 0};
+  return label_host_impl(h, nullptr, fd, 0, T, row_bytes, ep_offsets_host, n_eps, num_frames, reward_host, rtg_host,
+                         reward_stacked_host, rtg_stacked_host, nullptr, false, &z);
+}
+
+extern "C" int arp_embed_zfile(ArpHandle* h, int32_t fd, const int64_t* chunk_offset_host, const int64_t* chunk_bytes_host,
+                               int64_t T, int64_t row_bytes, float* emb_host) {
+  ARP_TRY(check_zargs(h, fd, chunk_offset_host, chunk_bytes_host, T, row_bytes));
+  if (T > 0 && !emb_host) return fail(h, ARP_ERR_INVALID, "null argument");
+  if (T == 0) return check_ready(h, reinterpret_cast<const uint8_t*>(h), T, row_bytes, h->own_stream);
+  ZRows z{chunk_offset_host, chunk_bytes_host, {}, row_bytes, 0};
+  return label_host_impl(h, nullptr, fd, 0, T, row_bytes, nullptr, 0, 0, nullptr, nullptr, nullptr, nullptr, emb_host,
+                         false, &z);
+}
+
+extern "C" int arp_embed_tower_zfile(ArpHandle* h, int32_t fd, const int64_t* chunk_offset_host,
+                                     const int64_t* chunk_bytes_host, int64_t T, int64_t row_bytes, float* rec_host) {
+  ARP_TRY(check_zargs(h, fd, chunk_offset_host, chunk_bytes_host, T, row_bytes));
+  if (T > 0 && !rec_host) return fail(h, ARP_ERR_INVALID, "null argument");
+  if (!h->adapter) return fail(h, ARP_ERR_INVALID, "tower records serve the adapter heads only");
+  if (T == 0) return check_ready(h, reinterpret_cast<const uint8_t*>(h), T, row_bytes, h->own_stream);
+  ZRows z{chunk_offset_host, chunk_bytes_host, {}, row_bytes, 0};
+  return label_host_impl(h, nullptr, fd, 0, T, row_bytes, nullptr, 0, 0, nullptr, nullptr, nullptr, nullptr, rec_host,
+                         true, &z);
+}
+
+extern "C" int arp_inflate_rows(ArpHandle* h, const uint8_t* src_dev, const int64_t* src_off_dev,
+                                const int64_t* src_bytes_dev, int64_t n, int64_t row_bytes, uint8_t* out_dev,
+                                int32_t* status_dev, void* stream) {
+  if (!h) return ARP_ERR_INVALID;
+  if (n < 0 || n > 0x7fffffffLL) return fail(h, ARP_ERR_INVALID, "bad n");
+  if (n > 0 && (!src_dev || !src_off_dev || !src_bytes_dev || !out_dev || !status_dev))
+    return fail(h, ARP_ERR_INVALID, "null argument");
+  ARP_TRY(check_row_bytes(h, row_bytes));
+  ARP_CUDA(h, cudaSetDevice(h->cfg.device));
+  return launch_inflate(h, src_dev, src_off_dev, src_bytes_dev, n, row_bytes, out_dev, status_dev,
+                        static_cast<cudaStream_t>(stream));
 }
 
 // arp_label's outputs from tower records: per max_batch chunk one unpack launch, then adapter_tail — the launches of

@@ -369,6 +369,20 @@ class RewardLabeler:
         """The frozen-CLIP side of label_file."""
         return self.engine.embed_tower_file(fd, file_offset, T, row_stride_bytes)
 
+    def label_zfile(self, fd: int, chunk_offsets: np.ndarray, chunk_bytes: np.ndarray, row_bytes: int,
+                    ep_offsets: np.ndarray, num_frames: int):
+        """label_file's outputs when row t is the zlib stream of chunk_bytes[t] bytes at chunk_offsets[t] of `fd` (a gzip
+        dataset chunked one row per chunk), inflated on the device."""
+        return self.engine.label_zfile(fd, chunk_offsets, chunk_bytes, row_bytes, ep_offsets, num_frames)
+
+    def embed_zfile(self, fd: int, chunk_offsets: np.ndarray, chunk_bytes: np.ndarray, row_bytes: int) -> np.ndarray:
+        """The image side of label_zfile."""
+        return self.engine.embed_zfile(fd, chunk_offsets, chunk_bytes, row_bytes)
+
+    def embed_tower_zfile(self, fd: int, chunk_offsets: np.ndarray, chunk_bytes: np.ndarray, row_bytes: int) -> np.ndarray:
+        """The frozen-CLIP side of label_zfile."""
+        return self.engine.embed_tower_zfile(fd, chunk_offsets, chunk_bytes, row_bytes)
+
     def label_tower(self, rec: np.ndarray, ep_offsets: np.ndarray, num_frames: int):
         """label_slab's outputs (host arrays) from the CLIP tower records [T, tower_dim] of the same rows, with this
         labeler's adapter."""
@@ -646,6 +660,38 @@ def _file_rows(labeler, src, method: str, lo_all: int):
     return path, base + lo_all * stride + (stride - frame), stride        # last stacked frame of row lo_all
 
 
+def _zfile_rows(ds):
+    """(path, chunk byte offsets [T], chunk sizes [T], row bytes) when every row of the image dataset `ds` is one plain
+    zlib stream at a known place of its HDF5 file, else None: an h5py dataset (its low-level chunk index is read through
+    DatasetID.get_num_chunks / get_chunk_info) of uint8 rows chunked (1, *shape[1:]), gzip and no other filter (no shuffle,
+    fletcher32 or scale-offset), every row's chunk allocated and written with filter_mask 0. No HDF5 structure is parsed
+    here: h5py says where each chunk is, and the library inflates it."""
+    dsid = getattr(ds, "id", None)
+    if dsid is None or not hasattr(dsid, "get_chunk_info") or getattr(getattr(ds, "file", None), "filename", None) is None:
+        return None
+    shape = tuple(ds.shape)
+    if len(shape) not in (4, 5) or np.dtype(ds.dtype) != np.uint8 or tuple(ds.chunks or ()) != (1,) + shape[1:]:
+        return None
+    if ds.compression != "gzip" or ds.shuffle or ds.fletcher32 or getattr(ds, "scaleoffset", None) is not None:
+        return None
+    plist = getattr(dsid, "get_create_plist", None)
+    if plist is not None and plist().get_nfilters() != 1:      # a filter h5py has no property for
+        return None
+    T = shape[0]
+    n = dsid.get_num_chunks()
+    if n != T:                                                   # an unallocated row
+        return None
+    offsets = np.full(T, -1, np.int64)
+    sizes = np.zeros(T, np.int64)
+    for i in range(n):
+        info = dsid.get_chunk_info(i)
+        t = int(info.chunk_offset[0])
+        if info.filter_mask != 0 or info.byte_offset is None or not 0 <= t < T or offsets[t] >= 0:
+            return None
+        offsets[t], sizes[t] = int(info.byte_offset), int(info.size)
+    return ds.file.filename, offsets, sizes, int(np.prod(shape[1:]))
+
+
 def _read_slabs(ds, side, off, e_lo: int, e_hi: int, slab_frames: int):
     """(a, b, rows) of every non-empty slab of whole episodes [a, b), read on a thread one slab ahead of the consumer"""
     import threading
@@ -677,13 +723,26 @@ def _read_slabs(ds, side, off, e_lo: int, e_hi: int, slab_frames: int):
 def _label_rows(labeler, ds, side, off, e_lo: int, e_hi: int, num_frames: int, slab_frames: int, n_groups: int = 1):
     """[reward_stacked, rtg_stacked] of each of the n_groups instruction sets in turn (2 * n_groups arrays [rows, F]) for
     episodes [e_lo, e_hi). A memory-mapped container is handed to the library in ONE call (a strided pointer into the file
-    mapping; the native stager overlaps page-cache reads, PCIe and compute). A container that has to be read through its
-    API (h5py: chunked, gzip) is read slab by slab on a reader thread, one slab ahead of the GPU."""
+    mapping; the native stager overlaps page-cache reads, PCIe and compute). An h5py gzip dataset chunked one row per
+    chunk (_zfile_rows) is handed over as its chunk table: the library reads the compressed rows and inflates them on the
+    device. Any other container that has to be read through its API is read slab by slab on a reader thread, one slab
+    ahead of the GPU."""
     lo_all, hi_all = int(off[e_lo]), int(off[e_hi])
     if hi_all <= lo_all:
         return _empty_pairs(labeler, n_groups, num_frames)
     src = side if side is not None else ds
     rel = off[e_lo:e_hi + 1] - lo_all
+    zrows = _zfile_rows(ds) if side is None and hasattr(labeler, "label_zfile") else None
+    if zrows is not None:
+        # gzip rows, one per chunk: the library preads this shard's compressed chunks and inflates them on the device
+        path, offsets, sizes, row_bytes = zrows
+        fd = os.open(path, os.O_RDONLY)
+        try:
+            r, _, rs, gs = labeler.label_zfile(fd, offsets[lo_all:hi_all], sizes[lo_all:hi_all], row_bytes, rel,
+                                               num_frames)
+        finally:
+            os.close(fd)
+        return _pairs(*_finish(labeler, r, rs, gs, rel, num_frames))
     frows = _file_rows(labeler, src, "label_file", lo_all)
     if frows is not None:
         # rows contiguous in a file: the library preads the scored frame of every row itself (arp_label_file)
@@ -720,6 +779,15 @@ def _embed_rows(labeler, ds, side, off, e_lo: int, e_hi: int, slab_frames: int, 
     if hi_all <= lo_all:
         return np.zeros((0, dim), np.float32)
     src = side if side is not None else ds
+    embed_zfile = "embed_tower_zfile" if tower else "embed_zfile"
+    zrows = _zfile_rows(ds) if side is None and hasattr(labeler, embed_zfile) else None
+    if zrows is not None:
+        path, offsets, sizes, row_bytes = zrows
+        fd = os.open(path, os.O_RDONLY)
+        try:
+            return getattr(labeler, embed_zfile)(fd, offsets[lo_all:hi_all], sizes[lo_all:hi_all], row_bytes)
+        finally:
+            os.close(fd)
     frows = _file_rows(labeler, src, embed_file, lo_all)
     if frows is not None:
         path, first, stride = frows

@@ -31,6 +31,12 @@
  * runs only the adapter (three GEMMs, the gate, the head) and the scan on such records, with no frames and no visual.*
  * weights, and gives arp_label's outputs bit for bit — also for an adapter checkpoint other than the one the records were
  * written with. A new fine-tuned adapter then costs 0.468 GFLOP per frame instead of the ViT's 35.1.
+ *
+ * Compressed rows: the recorder writes `ob` as gzip-chunked HDF5 with one row (F stacked frames) per chunk, and HDF5's
+ * deflate filter stores every chunk as one plain zlib stream. arp_label_zfile / arp_embed_zfile / arp_embed_tower_zfile
+ * take the file offset and size of every row's chunk (h5py: DatasetID.get_chunk_info), pread() the compressed bytes and
+ * inflate them on the device (one warp per row, Adler-32 checked) before the unchanged encoder pass. No HDF5 parsing
+ * happens here: the caller's chunk index says where the streams are.
  */
 #ifndef ARP_B200_H_
 #define ARP_B200_H_
@@ -41,7 +47,7 @@
 extern "C" {
 #endif
 
-#define ARP_B200_ABI_VERSION 8   /* 3: + arp_encode_taps_chw, 4: + arp_operand_dtype, 5: + ARP_PREC_F32RESID, arp_ln_gemm, arp_resid_gemm_stats, arp_label_file, arp_wants_weight, 6: + arp_set_text_groups, arp_text_groups, 7: + arp_embedding_dim, arp_embed_host, arp_embed_file, arp_label_embeddings, 8: + arp_tower_dim, arp_embed_tower_host, arp_embed_tower_file, arp_label_tower */
+#define ARP_B200_ABI_VERSION 9   /* 3: + arp_encode_taps_chw, 4: + arp_operand_dtype, 5: + ARP_PREC_F32RESID, arp_ln_gemm, arp_resid_gemm_stats, arp_label_file, arp_wants_weight, 6: + arp_set_text_groups, arp_text_groups, 7: + arp_embedding_dim, arp_embed_host, arp_embed_file, arp_label_embeddings, 8: + arp_tower_dim, arp_embed_tower_host, arp_embed_tower_file, arp_label_tower, 9: + ArpInflateStatus, arp_inflate_rows, arp_label_zfile, arp_embed_zfile, arp_embed_tower_zfile */
 
 #define ARP_MAX_TEXT 16          /* texts of one instruction set (arp_set_text's n_text, one group's size) */
 #define ARP_MAX_TEXT_GROUPS 16   /* instruction sets of one arp_set_text_groups call */
@@ -61,6 +67,20 @@ typedef enum ArpStatus {
   ARP_ERR_NO_DEVICE = -4,   /* no CUDA device, or not compute capability 10.x */
   ARP_ERR_UNKNOWN_KEY = -5  /* arp_set_weight: name is not part of the model */
 } ArpStatus;
+
+/* Per-row result of the device zlib inflate (arp_inflate_rows' status_dev; named by arp_last_error after a failed
+ * arp_*_zfile call). The first violation stops the row. */
+typedef enum ArpInflateStatus {
+  ARP_INFLATE_OK = 0,
+  ARP_INFLATE_TRUNCATED = 1,          /* a read past the row's compressed bytes */
+  ARP_INFLATE_BAD_HEADER = 2,         /* zlib header: CM != 8, CINFO > 7, FCHECK wrong, or FDICT set */
+  ARP_INFLATE_BAD_BLOCK = 3,          /* block type 3, or a stored block whose LEN / NLEN disagree */
+  ARP_INFLATE_BAD_CODE = 4,           /* over-subscribed or invalid Huffman code, bad code-length repeat, symbol 286-287 / 30-31 */
+  ARP_INFLATE_DISTANCE_TOO_FAR = 5,   /* a back-reference before the start of the row */
+  ARP_INFLATE_TOO_LONG = 6,           /* more than row_bytes of output */
+  ARP_INFLATE_TOO_SHORT = 7,          /* the stream ended before row_bytes of output */
+  ARP_INFLATE_BAD_ADLER = 8           /* the Adler-32 trailer does not match the inflated row */
+} ArpInflateStatus;
 
 /* label_reward.py:109-121 vs clip_multiscale_adapter.py:121-133 */
 typedef enum ArpPreprocess { ARP_PRE_PIL_BICUBIC = 0, ARP_PRE_BILINEAR = 1 } ArpPreprocess;
@@ -234,6 +254,32 @@ ARP_API int arp_embed_tower_host(ArpHandle* h, const uint8_t* ob_host, int64_t T
                                  float* rec_host);
 ARP_API int arp_embed_tower_file(ArpHandle* h, int32_t fd, int64_t file_offset, int64_t T, int64_t row_stride_bytes,
                                  float* rec_host);
+
+/* Compressed rows. Row t of the call is one zlib stream (RFC 1950) of chunk_bytes_host[t] bytes at byte
+ * chunk_offset_host[t] of the open descriptor `fd`, and inflates to exactly row_bytes = F * in_h * in_w * 3 bytes, F in
+ * [1, 64] (the row's F stacked frames; the LAST one is scored). The gather threads pread() each row's compressed bytes
+ * into the pinned ring (slots sized from the call's largest chunk), each max_batch chunk crosses PCIe compressed, and
+ * inflate_rows_kernel writes the whole rows into a device scratch of max_batch * row_bytes bytes that the encoder reads
+ * with row stride row_bytes. Outputs as for arp_label_file / arp_embed_file / arp_embed_tower_file, bit for bit what
+ * those give on the same rows stored uncompressed. ARP_ERR_INVALID for fd < 0, T < 0, null tables, a negative offset or
+ * size, a bad row_bytes, and for a row that does not inflate: arp_last_error then names the first such row (its index
+ * in the call) and its ArpInflateStatus, no output is written, and the handle stays usable. Synchronises.
+ * replaces g[img_key][traj, -1] (label_reward.py:268) for gzip datasets chunked (1, F, H, W, 3). */
+ARP_API int arp_label_zfile(ArpHandle* h, int32_t fd, const int64_t* chunk_offset_host, const int64_t* chunk_bytes_host,
+                            int64_t T, int64_t row_bytes, const int64_t* ep_offsets_host, int32_t n_eps,
+                            int32_t num_frames, float* reward_host, float* rtg_host, float* reward_stacked_host,
+                            float* rtg_stacked_host);
+ARP_API int arp_embed_zfile(ArpHandle* h, int32_t fd, const int64_t* chunk_offset_host, const int64_t* chunk_bytes_host,
+                            int64_t T, int64_t row_bytes, float* emb_host);
+ARP_API int arp_embed_tower_zfile(ArpHandle* h, int32_t fd, const int64_t* chunk_offset_host,
+                                  const int64_t* chunk_bytes_host, int64_t T, int64_t row_bytes, float* rec_host);
+/* The inflate kernel alone, on DEVICE buffers: row r's zlib stream is src_dev[src_off_dev[r], + src_bytes_dev[r]) (the
+ * caller keeps those ranges inside src_dev), it is inflated to out_dev[r * row_bytes, (r + 1) * row_bytes) and
+ * status_dev[r] (int32) receives its ArpInflateStatus. Rows that fail leave the rest of their output unwritten.
+ * Stream-ordered, does not synchronise; ARP_ERR_INVALID only for bad arguments (row_bytes as for arp_label_zfile). */
+ARP_API int arp_inflate_rows(ArpHandle* h, const uint8_t* src_dev, const int64_t* src_off_dev,
+                             const int64_t* src_bytes_dev, int64_t n, int64_t row_bytes, uint8_t* out_dev,
+                             int32_t* status_dev, void* stream);
 /* arp_label's outputs ([G,T] / [G,T,F] with text groups, the goal-conditioned adapter head included) from tower records:
  * rec_dev [T, arp_tower_dim] fp32 DEVICE rows (16-byte aligned) from arp_embed_tower_* of a handle with the same CLIP
  * weights, arch, frame size, crop and precision; the other arguments and the four outputs are those of arp_label. Needs
