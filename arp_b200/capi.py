@@ -43,6 +43,7 @@ EXPORTS = (
     "arp_set_text_groups", "arp_text_groups", "arp_embedding_dim", "arp_embed_host", "arp_embed_file",
     "arp_label_embeddings", "arp_tower_dim", "arp_embed_tower_host", "arp_embed_tower_file", "arp_label_tower",
     "arp_label_zfile", "arp_embed_zfile", "arp_embed_tower_zfile", "arp_inflate_rows",
+    "arp_label_zchunks", "arp_embed_zchunks", "arp_embed_tower_zchunks", "arp_gather_frames",
 )
 PROFILE_CLASSES = ("gemm", "attention", "layernorm", "decode", "head", "scan", "other")
 
@@ -55,6 +56,24 @@ class ArpConfig(C.Structure):
     _fields_ = [(n, C.c_int32) for n in (
         "struct_size", "device", "patch", "width", "layers", "heads", "embed_dim", "in_h", "in_w", "use_crop",
         "preprocess", "head", "reduce", "max_batch", "precision")]
+
+
+class ArpChunkLayout(C.Structure):
+    _fields_ = [("struct_size", C.c_int32), ("ndim", C.c_int32), ("shape", C.c_int64 * 5), ("chunk", C.c_int64 * 5)]
+
+
+#: device scratch bound of one max_batch batch's inflated chunks (ARP_ZCHUNK_SCRATCH_BYTES)
+ZCHUNK_SCRATCH_BYTES = 4 << 30
+#: largest compressed chunk the compressed-chunk calls take (ARP_ZCHUNK_MAX_COMPRESSED_BYTES)
+ZCHUNK_MAX_COMPRESSED_BYTES = 64 << 20
+
+
+def chunk_layout(shape, chunks) -> ArpChunkLayout:
+    """ArpChunkLayout of a uint8 dataset `shape` ([T, F, H, W, 3] or [T, H, W, 3]) stored in chunks of shape `chunks`"""
+    assert len(shape) == len(chunks) and len(shape) in (4, 5), (shape, chunks)
+    pad = (0,) * (5 - len(shape))
+    return ArpChunkLayout(C.sizeof(ArpChunkLayout), len(shape), (C.c_int64 * 5)(*shape, *pad),
+                          (C.c_int64 * 5)(*chunks, *pad))
 
 
 class ArpError(RuntimeError):
@@ -116,6 +135,11 @@ def load_library() -> C.CDLL:
     lib.arp_embed_zfile.argtypes = [vp, i32, vp, vp, i64, i64, vp]
     lib.arp_embed_tower_zfile.argtypes = [vp, i32, vp, vp, i64, i64, vp]
     lib.arp_inflate_rows.argtypes = [vp, vp, vp, vp, i64, i64, vp, vp, vp]
+    lay = C.POINTER(ArpChunkLayout)
+    lib.arp_label_zchunks.argtypes = [vp, i32, lay, vp, vp, vp, i64, i64, i64, vp, i32, i32, vp, vp, vp, vp]
+    lib.arp_embed_zchunks.argtypes = [vp, i32, lay, vp, vp, vp, i64, i64, i64, vp]
+    lib.arp_embed_tower_zchunks.argtypes = [vp, i32, lay, vp, vp, vp, i64, i64, i64, vp]
+    lib.arp_gather_frames.argtypes = [vp, lay, i64, i64, vp, vp, vp]
     lib.arp_compute_reward.argtypes = [vp, vp, i64, i64, vp, vp, vp]
     lib.arp_online_reward.argtypes = [vp, vp, i32, vp, vp, vp]
     lib.arp_preprocess_rtgs.argtypes = [vp, vp, i64, vp, i32, i32, i32, vp, vp, vp, vp, vp]
@@ -501,6 +525,61 @@ class Engine:
         self._check(self._lib.arp_inflate_rows(self._h, _ptr(src), _ptr(so), _ptr(sb), n, int(row_bytes), _ptr(out),
                                                _ptr(status), _stream_ptr(self.device)))
         return out, status
+
+    # -- compressed chunks of any shape ------------------------------------------------------------
+    @staticmethod
+    def _zchunk_args(layout, origins, offsets, sizes):
+        """(ArpChunkLayout, arrays kept alive, ctypes pointers to origins / offsets / sizes, n_chunks); layout is the
+        dataset's (shape, chunks) and origins [n_chunks, ndim] the chunks' logical origins"""
+        lay = chunk_layout(*layout)
+        o = np.ascontiguousarray(origins, dtype=np.int64).reshape(-1, lay.ndim)
+        off, nb, p_off, p_nb = Engine._chunk_table(offsets, sizes)
+        assert o.shape[0] == off.size, (o.shape, off.shape)
+        return lay, (o, off, nb), C.c_void_p(o.ctypes.data), p_off, p_nb, off.size
+
+    def label_zchunks(self, fd: int, layout, origins: np.ndarray, offsets: np.ndarray, sizes: np.ndarray, row_lo: int,
+                      T: int, ep_offsets: np.ndarray, num_frames: int, out=None):
+        """arp_label_zchunks: label_file's outputs for dataset rows [row_lo, row_lo + T) (frame F-1 of each) of a gzip
+        dataset stored in chunks of any shape: layout = (shape, chunks), chunk i is the zlib stream of sizes[i] bytes at
+        file offset offsets[i] of `fd` with logical origin origins[i]. ep_offsets are relative to row_lo."""
+        lay, keep, p_o, p_off, p_nb, n = self._zchunk_args(layout, origins, offsets, sizes)
+        ep = np.ascontiguousarray(ep_offsets, dtype=np.int64)
+        if out is None:
+            out = self._host_outputs(int(T), num_frames)
+        hp = lambda a: C.c_void_p(a.ctypes.data)  # noqa: E731
+        self._check(self._lib.arp_label_zchunks(self._h, int(fd), C.byref(lay), p_o, p_off, p_nb, n, int(row_lo), int(T),
+                                                hp(ep), ep.size - 1, num_frames, hp(out[0]), hp(out[1]), hp(out[2]),
+                                                hp(out[3])))
+        return out
+
+    def embed_zchunks(self, fd: int, layout, origins: np.ndarray, offsets: np.ndarray, sizes: np.ndarray, row_lo: int,
+                      T: int, out: "np.ndarray | None" = None) -> np.ndarray:
+        """arp_embed_zchunks: embed_file's result for the rows label_zchunks reads."""
+        lay, keep, p_o, p_off, p_nb, n = self._zchunk_args(layout, origins, offsets, sizes)
+        out = self._emb_out(int(T), out)
+        self._check(self._lib.arp_embed_zchunks(self._h, int(fd), C.byref(lay), p_o, p_off, p_nb, n, int(row_lo), int(T),
+                                                C.c_void_p(out.ctypes.data)))
+        return out
+
+    def embed_tower_zchunks(self, fd: int, layout, origins: np.ndarray, offsets: np.ndarray, sizes: np.ndarray,
+                            row_lo: int, T: int, out: "np.ndarray | None" = None) -> np.ndarray:
+        """arp_embed_tower_zchunks: embed_tower_file's result for the rows label_zchunks reads."""
+        lay, keep, p_o, p_off, p_nb, n = self._zchunk_args(layout, origins, offsets, sizes)
+        out = self._emb_out(int(T), out, self.tower_dim)
+        self._check(self._lib.arp_embed_tower_zchunks(self._h, int(fd), C.byref(lay), p_o, p_off, p_nb, n, int(row_lo),
+                                                      int(T), C.c_void_p(out.ctypes.data)))
+        return out
+
+    def gather_frames(self, layout, row0: int, n: int, chunks: torch.Tensor) -> torch.Tensor:
+        """arp_gather_frames on device tensors: chunks (uint8, the batch's inflated chunks in (row-chunk, H-, W-,
+        channel-chunk) order) -> frame F-1 of dataset rows [row0, row0 + n) as uint8 [n, H, W, 3]."""
+        assert chunks.dtype == torch.uint8 and chunks.is_cuda and chunks.is_contiguous()
+        lay = chunk_layout(*layout)
+        shape = tuple(layout[0])
+        out = torch.empty((int(n),) + tuple(shape[-3:]), device=self.device, dtype=torch.uint8)
+        self._check(self._lib.arp_gather_frames(self._h, C.byref(lay), int(row0), int(n), _ptr(chunks), _ptr(out),
+                                                _stream_ptr(self.device)))
+        return out
 
     def compute_reward(self, ob: torch.Tensor, want_logits: bool = False):
         """reward [T] (or [G, T] after set_text_groups); logits [T, n_text] over the texts of all groups."""

@@ -178,8 +178,8 @@ struct ArpHandle {
   size_t scratch_bytes[2] = {0, 0};
   uint8_t* stage_dev[2] = {nullptr, nullptr};
   size_t stage_bytes = 0;
-  // compressed-row entry points (arp_*_zfile): two device buffers of one chunk's compressed rows, the inflated rows of one
-  // chunk [max_batch, row_bytes], and the call's per-row tables (packed offset, size, inflate status)
+  // compressed entry points (arp_*_zfile, arp_*_zchunks): two device buffers of one batch's compressed chunks, the
+  // inflated chunks of one batch (one chunk volume each), and the call's per-chunk tables (packed offset, size, status)
   uint8_t* zsrc_dev[2] = {nullptr, nullptr};
   size_t zsrc_bytes = 0;
   uint8_t* zrows_dev = nullptr;
@@ -1617,6 +1617,8 @@ static int ensure_stage(ArpHandle* h) {
 constexpr int STG_SLOTS = 8;       // pinned ring depth
 constexpr int STG_SUB = 64;        // frames per slot (12.6 MB at 256x256x3)
 constexpr int STG_WORKERS = 4;
+// compressed calls: at most this per slot unless one chunk is larger (zfile rows only; zchunks refuse such chunks)
+constexpr int64_t ZRING_SLOT_BYTES = ARP_ZCHUNK_MAX_COMPRESSED_BYTES;
 
 static bool host_ptr_is_pinned(const void* p) {
   cudaPointerAttributes a;
@@ -1624,9 +1626,9 @@ static bool host_ptr_is_pinned(const void* p) {
   return a.type == cudaMemoryTypeHost;   // pageable memory reports cudaMemoryTypeUnregistered
 }
 
-// row_bytes: the ring's row pitch (a frame, or the largest compressed chunk of a zfile call)
-static int ensure_pinned_ring(ArpHandle* h, size_t row_bytes) {
-  const size_t need = row_bytes * STG_SUB * STG_SLOTS;
+// slot_bytes: one ring slot (STG_SUB frames, or up to STG_SUB of the largest compressed chunk of a zfile / zchunks call)
+static int ensure_pinned_ring(ArpHandle* h, size_t slot_bytes) {
+  const size_t need = slot_bytes * STG_SLOTS;
   if (h->pin_bytes >= need) return ARP_OK;
   if (h->pin_ring) { cudaFreeHost(h->pin_ring); h->pin_ring = nullptr; h->pin_bytes = 0; }
   ARP_CUDA(h, cudaHostAlloc((void**)&h->pin_ring, need, cudaHostAllocDefault));
@@ -1636,7 +1638,8 @@ static int ensure_pinned_ring(ArpHandle* h, size_t row_bytes) {
   return ARP_OK;
 }
 
-struct SubChunk { int64_t t0; int n; };   // rows [t0, t0+n) of the call, never straddling a device chunk
+// rows [t0, t0+n) of the call (compressed calls: ZRows entries), never straddling a device chunk
+struct SubChunk { int64_t t0; int n; };
 
 // gathers sub-chunk after sub-chunk into the pinned ring; the main thread consumes them in order
 // pread() exactly n bytes at off; 0, errno, or -1 at end of file
@@ -1650,14 +1653,26 @@ static int pread_full(int fd, uint8_t* dst, size_t n, int64_t off) {
   return 0;
 }
 
-// compressed rows of a zfile call: row t is the zlib stream of bytes[t] bytes at file offset off[t]; pos[t] is its byte
-// offset in its device chunk's packed buffer
-struct ZRows { const int64_t* off; const int64_t* bytes; std::vector<int64_t> pos; int64_t row_bytes; int64_t max_chunk; };
+// The compressed chunks a zfile / zchunks call reads, planned per max_batch batch (plan_zchunks). Entry e is one needed
+// chunk: the zlib stream of bytes[e] bytes at file offset off[e], chunk[e] of the caller's table; pos[e] is its byte
+// offset in its batch's packed buffer, and it inflates to slot e - batch[b] of the batch's scratch. Batch b's entries
+// are [batch[b], batch[b + 1]), in the order (row-chunk, H-chunk, W-chunk, channel-chunk) that gather_frames_kernel
+// indexes. A row-chunk serving two batches has an entry in each.
+struct ZRows {
+  std::vector<int64_t> off, bytes, pos, chunk, batch;
+  const int64_t* origins = nullptr;   // the caller's table [n_chunks, ndim], for messages
+  int ndim = 5;
+  int64_t row_lo = 0;
+  int64_t max_chunk = 1;              // largest compressed chunk: the pinned ring's pitch
+  bool dense = false;                 // chunks (1, cF, H, W, 3): the encoder reads frame F-1 in place, stride grid.vol
+  arp_inflate::ChunkGrid grid{};      // row0 and rc0 are set per batch
+};
 
 struct HostStager {
-  const uint8_t* src; int64_t stride; size_t frame_bytes; uint8_t* ring; cudaEvent_t* ev_slot; int device;
+  const uint8_t* src; int64_t stride; size_t frame_bytes; size_t slot_bytes; uint8_t* ring; cudaEvent_t* ev_slot;
+  int device;
   int fd = -1; int64_t fd_base = 0;          // fd >= 0: rows are pread() from a file (no page-table traffic) instead of src
-  const ZRows* z = nullptr;                  // compressed rows: a slot holds its rows' chunks packed, pitch frame_bytes
+  const ZRows* z = nullptr;                  // compressed chunks: a slot holds its entries' chunks packed
   std::atomic<int> io_error{0};
   const std::vector<SubChunk>* subs;
   std::atomic<int64_t> next{0}, issued{0};   // next task to start | sub-chunks whose H2D has been enqueued
@@ -1681,7 +1696,7 @@ struct HostStager {
         cudaEventSynchronize(ev_slot[slot]);
       }
       const SubChunk& sc = (*subs)[j];
-      uint8_t* dst = ring + (size_t)slot * STG_SUB * frame_bytes;
+      uint8_t* dst = ring + (size_t)slot * slot_bytes;
       if (z) {
         for (int f = 0; f < sc.n && !io_error.load(); ++f) {
           const int64_t t = sc.t0 + f;
@@ -1716,8 +1731,8 @@ struct HostStager {
   void stop() { abort.store(true); for (auto& t : threads) t.join(); threads.clear(); }
 };
 
-// ---- compressed rows (arp_*_zfile) --------------------------------------------------------------------------------
-struct ZDev { int64_t* pos = nullptr; int64_t* bytes = nullptr; int* status = nullptr; };   // [T] each, device
+// ---- compressed chunks (arp_*_zfile, arp_*_zchunks) ----------------------------------------------------------------
+struct ZDev { int64_t* pos = nullptr; int64_t* bytes = nullptr; int* status = nullptr; };   // one per ZRows entry, device
 
 static int launch_inflate(ArpHandle* h, const uint8_t* src, const int64_t* off, const int64_t* bytes, int64_t n,
                           int64_t row_bytes, uint8_t* out, int* status, cudaStream_t st) {
@@ -1730,20 +1745,176 @@ static int launch_inflate(ArpHandle* h, const uint8_t* src, const int64_t* off, 
   return ARP_OK;
 }
 
-// packs each max_batch chunk's compressed rows back to back (z->pos), sizes the device buffers from the call's largest
-// chunk, and uploads the per-row tables
-static int prepare_zrows(ArpHandle* h, ZRows* z, int64_t T, int64_t B, ZDev* zd, cudaStream_t st) {
-  z->pos.assign((size_t)T, 0);
-  size_t zsrc = 1;
-  z->max_chunk = 1;
-  for (int64_t t0 = 0; t0 < T; t0 += B) {
-    int64_t p = 0;
-    for (int64_t t = t0; t < std::min(T, t0 + B); ++t) {
-      z->pos[t] = p;
-      p += z->bytes[t];
-      z->max_chunk = std::max(z->max_chunk, z->bytes[t]);
+// frame F-1 of dataset rows [row0, row0 + n) from a batch's inflated chunks into dense frames out [n, H, W, 3]
+static int launch_gather(ArpHandle* h, arp_inflate::ChunkGrid g, int64_t row0, int64_t n, const uint8_t* chunks,
+                         uint8_t* out, cudaStream_t st) {
+  if (n <= 0) return ARP_OK;
+  g.row0 = row0;
+  g.rc0 = row0 / g.cT;
+  const int64_t npix = n * g.H * g.W;
+  ProfScope prof(h, PC_DECODE, 0.0, (double)npix * 3 * 2, st);
+  const unsigned blocks = (unsigned)std::min<int64_t>((npix + 255) / 256, 148 * 16);
+  arp_inflate::gather_frames_kernel<<<blocks, 256, 0, st>>>(chunks, g, (int)n, out);
+  h->launches++;
+  ARP_CUDA(h, cudaGetLastError());
+  return ARP_OK;
+}
+
+constexpr int64_t ZCHUNK_MAX_NEEDED = 1ll << 26;   // needed chunks of one zchunks call
+
+// a chunk layout as 5-D [T, F, H, W, C] (a 4-D dataset has F = 1); n[d]: chunks along axis d
+struct ZLayout { int64_t s[5], c[5], n[5]; int64_t vol; int nd; };
+
+// origin (of `nd` entries) as "(a, b, ...)"
+static const char* origin_str(char (&buf)[160], const int64_t* o, int nd) {
+  int k = snprintf(buf, sizeof buf, "(");
+  for (int d = 0; d < nd; ++d) k += snprintf(buf + k, sizeof buf - k, d ? ", %lld" : "%lld", (long long)o[d]);
+  snprintf(buf + k, sizeof buf - k, ")");
+  return buf;
+}
+
+// the layout checks of the zchunks entry points: uint8 frames of this handle's H x W x 3, every chunk extent >= 1, and
+// one chunk's volume (the inflate output size) within the device-scratch bound
+static int check_chunk_layout(ArpHandle* h, const ArpChunkLayout* L, ZLayout* z) {
+  if (!L || L->struct_size < (int32_t)sizeof(ArpChunkLayout) || (L->ndim != 4 && L->ndim != 5))
+    return fail(h, ARP_ERR_INVALID, "bad chunk layout (null, struct_size or ndim not 4 / 5)");
+  z->nd = L->ndim;
+  for (int d = 0, k = 0; d < 5; ++d, ++k) {
+    const bool f_axis = z->nd == 4 && d == 1;
+    z->s[d] = f_axis ? 1 : L->shape[k];
+    z->c[d] = f_axis ? 1 : L->chunk[k];
+    if (f_axis) --k;
+  }
+  const int64_t* s = z->s;
+  if (s[0] < 0 || s[1] < 1 || s[2] != h->cfg.in_h || s[3] != h->cfg.in_w || s[4] != 3)
+    return fail(h, ARP_ERR_INVALID, "dataset shape [T=%lld, F=%lld, %lld, %lld, %lld] is not [T, F >= 1, %d, %d, 3]",
+                (long long)s[0], (long long)s[1], (long long)s[2], (long long)s[3], (long long)s[4], h->cfg.in_h,
+                h->cfg.in_w);
+  z->vol = 1;
+  for (int d = 0; d < 5; ++d) {
+    if (z->c[d] < 1 || z->c[d] > INT32_MAX) return fail(h, ARP_ERR_INVALID, "chunk extent %lld of axis %d is not in [1, 2^31)",
+                                                        (long long)z->c[d], d);
+    if (z->c[d] > ARP_ZCHUNK_SCRATCH_BYTES / z->vol)
+      return fail(h, ARP_ERR_INVALID, "one chunk inflates to more than the %lld-byte device scratch bound",
+                  (long long)ARP_ZCHUNK_SCRATCH_BYTES);
+    z->vol *= z->c[d];
+    z->n[d] = (s[d] + z->c[d] - 1) / z->c[d];
+  }
+  return ARP_OK;
+}
+
+static arp_inflate::ChunkGrid chunk_grid(const ZLayout& l) {
+  arp_inflate::ChunkGrid g{};
+  g.vol = l.vol;
+  g.row_pitch = l.c[1] * l.c[2] * l.c[3] * l.c[4];
+  g.frame_off = (l.s[1] - 1) % l.c[1] * l.c[2] * l.c[3] * l.c[4];
+  g.cT = (int)l.c[0]; g.cH = (int)l.c[2]; g.cW = (int)l.c[3]; g.cC = (int)l.c[4];
+  g.nH = (int)l.n[2]; g.nW = (int)l.n[3]; g.nC = (int)l.n[4];
+  g.H = (int)l.s[2]; g.W = (int)l.s[3];
+  return g;
+}
+
+// Checks a zchunks call's layout, rows and chunk table and plans its batches (host only, nothing is read): the needed
+// chunks are the row-chunks covering dataset rows [row_lo, row_lo + T) at the F-chunk of frame F-1, every H, W and
+// channel chunk; every other entry of the table is only checked.
+static int plan_zchunks(ArpHandle* h, const ArpChunkLayout* layout, const int64_t* origins, const int64_t* offs,
+                        const int64_t* sizes, int64_t n_chunks, int64_t row_lo, int64_t T, bool bounded, ZRows* z) {
+  // bounded (the zchunks calls): one batch's inflated chunks within ARP_ZCHUNK_SCRATCH_BYTES, at most ZCHUNK_MAX_NEEDED
+  // needed chunks, and no compressed chunk larger than a pinned-ring slot, so the ring stays within
+  // STG_SLOTS * ZRING_SLOT_BYTES. The zfile calls keep the limits they always had: none of these.
+  const int64_t scratch_bound = bounded ? ARP_ZCHUNK_SCRATCH_BYTES : INT64_MAX;
+  ZLayout l;
+  ARP_TRY(check_chunk_layout(h, layout, &l));
+  if (row_lo < 0 || T < 0 || row_lo > l.s[0] - T)
+    return fail(h, ARP_ERR_INVALID, "rows [%lld, %lld + %lld) are not inside the dataset's %lld rows", (long long)row_lo,
+                (long long)row_lo, (long long)T, (long long)l.s[0]);
+  if (n_chunks < 0 || (n_chunks > 0 && (!origins || !offs || !sizes)))
+    return fail(h, ARP_ERR_INVALID, "null chunk table or n_chunks < 0");
+  const int nd = l.nd;
+  const int64_t fc = (l.s[1] - 1) / l.c[1];                        // F-chunk of the scored frame
+  const int64_t nsp = l.n[2] * l.n[3] * l.n[4];                    // chunks of one (row-chunk, F-chunk) cell
+  const int64_t rc_lo = T ? row_lo / l.c[0] : 0, rc_hi = T ? (row_lo + T - 1) / l.c[0] : -1;
+  if (bounded && (rc_hi - rc_lo + 1) > ZCHUNK_MAX_NEEDED / nsp)   // tiny chunks: host tables and one warp per chunk would not scale
+    return fail(h, ARP_ERR_INVALID, "the call needs more than %lld chunks", (long long)ZCHUNK_MAX_NEEDED);
+  std::vector<int64_t> need((size_t)((rc_hi - rc_lo + 1) * nsp), -1);   // needed chunk -> table entry
+  std::vector<std::pair<int64_t, int64_t>> keys((size_t)n_chunks);     // (chunk grid index, table entry)
+  char buf[160];
+  for (int64_t i = 0; i < n_chunks; ++i) {
+    const int64_t* o = origins + i * nd;
+    int64_t gi[5];
+    for (int d = 0, k = 0; d < 5; ++d, ++k) {
+      const bool f_axis = nd == 4 && d == 1;
+      const int64_t od = f_axis ? 0 : o[k];
+      if (f_axis) --k;
+      if (od < 0 || od >= l.s[d] || od % l.c[d] != 0)
+        return fail(h, ARP_ERR_INVALID, "chunk %lld: logical origin %s is not a multiple of the chunk shape inside the "
+                    "dataset", (long long)i, origin_str(buf, o, nd));
+      gi[d] = od / l.c[d];
     }
-    zsrc = std::max(zsrc, (size_t)p);
+    if (offs[i] < 0 || sizes[i] < 0)
+      return fail(h, ARP_ERR_INVALID, "chunk %lld at logical origin %s: negative file offset or size", (long long)i,
+                  origin_str(buf, o, nd));
+    keys[(size_t)i] = {(((gi[0] * l.n[1] + gi[1]) * l.n[2] + gi[2]) * l.n[3] + gi[3]) * l.n[4] + gi[4], i};
+    if (gi[1] == fc && gi[0] >= rc_lo && gi[0] <= rc_hi)
+      need[(size_t)((gi[0] - rc_lo) * nsp + (gi[2] * l.n[3] + gi[3]) * l.n[4] + gi[4])] = i;
+  }
+  std::sort(keys.begin(), keys.end());
+  for (size_t k = 1; k < keys.size(); ++k)
+    if (keys[k].first == keys[k - 1].first)
+      return fail(h, ARP_ERR_INVALID, "chunks %lld and %lld share the logical origin %s", (long long)keys[k - 1].second,
+                  (long long)keys[k].second, origin_str(buf, origins + keys[k].second * nd, nd));
+  for (size_t j = 0; j < need.size(); ++j)
+    if (need[j] < 0) {
+      const int64_t sp = (int64_t)j % nsp;
+      const int64_t o5[5] = {(rc_lo + (int64_t)j / nsp) * l.c[0], fc * l.c[1], sp / (l.n[3] * l.n[4]) * l.c[2],
+                             sp / l.n[4] % l.n[3] * l.c[3], sp % l.n[4] * l.c[4]};
+      const int64_t o4[4] = {o5[0], o5[2], o5[3], o5[4]};
+      return fail(h, ARP_ERR_INVALID, "the chunk at logical origin %s holds scored frames but is not in the chunk table",
+                  origin_str(buf, nd == 4 ? o4 : o5, nd));
+    } else if (bounded && sizes[need[j]] > ZRING_SLOT_BYTES) {
+      return fail(h, ARP_ERR_INVALID, "chunk %lld at logical origin %s: %lld compressed bytes, more than the %lld-byte "
+                  "staging slot", (long long)need[j], origin_str(buf, origins + need[j] * nd, nd),
+                  (long long)sizes[need[j]], (long long)ZRING_SLOT_BYTES);
+    }
+  // batches: every needed chunk of the batch's row-chunks, packed back to back in table order
+  const int64_t B = h->cfg.max_batch;
+  *z = ZRows{};
+  z->batch.assign(1, 0);
+  for (int64_t t0 = 0; t0 < T; t0 += B) {
+    const int64_t n = std::min(B, T - t0);
+    const int64_t a = (row_lo + t0) / l.c[0] - rc_lo, b = (row_lo + t0 + n - 1) / l.c[0] - rc_lo;
+    if ((b - a + 1) * nsp > scratch_bound / l.vol)
+      return fail(h, ARP_ERR_INVALID, "the inflated chunks of one max_batch batch (%lld chunks of %lld bytes) exceed the "
+                  "%lld-byte device scratch bound", (long long)((b - a + 1) * nsp), (long long)l.vol,
+                  (long long)scratch_bound);
+    int64_t p = 0;
+    for (int64_t j = a * nsp; j < (b + 1) * nsp; ++j) {
+      const int64_t i = need[(size_t)j];
+      z->off.push_back(offs[i]);
+      z->bytes.push_back(sizes[i]);
+      z->pos.push_back(p);
+      z->chunk.push_back(i);
+      p += sizes[i];
+      z->max_chunk = std::max(z->max_chunk, sizes[i]);
+    }
+    z->batch.push_back((int64_t)z->off.size());
+  }
+  z->origins = origins;
+  z->ndim = nd;
+  z->row_lo = row_lo;
+  z->dense = l.c[0] == 1 && l.c[2] == l.s[2] && l.c[3] == l.s[3] && l.c[4] == 3;
+  z->grid = chunk_grid(l);
+  return ARP_OK;
+}
+
+// sizes the device buffers from the call's largest batch and uploads the per-entry tables
+static int prepare_zrows(ArpHandle* h, const ZRows& z, ZDev* zd, cudaStream_t st) {
+  const int64_t E = (int64_t)z.off.size();
+  size_t zsrc = 1, zrows = 1;
+  for (size_t b = 0; b + 1 < z.batch.size(); ++b) {
+    const int64_t e0 = z.batch[b], e1 = z.batch[b + 1];
+    if (e1 > e0) zsrc = std::max(zsrc, (size_t)(z.pos[e1 - 1] + z.bytes[e1 - 1]));
+    zrows = std::max(zrows, (size_t)((e1 - e0) * z.grid.vol));
   }
   if (h->zsrc_bytes < zsrc) {
     for (int i = 0; i < 2; ++i) {
@@ -1752,13 +1923,13 @@ static int prepare_zrows(ArpHandle* h, ZRows* z, int64_t T, int64_t B, ZDev* zd,
     }
     h->zsrc_bytes = zsrc;
   }
-  ARP_TRY(grow(h, reinterpret_cast<void**>(&h->zrows_dev), &h->zrows_bytes, (size_t)std::min(B, T) * z->row_bytes));
-  ARP_TRY(grow(h, &h->ztab_dev, &h->ztab_bytes, (size_t)T * 20));
+  ARP_TRY(grow(h, reinterpret_cast<void**>(&h->zrows_dev), &h->zrows_bytes, zrows));
+  ARP_TRY(grow(h, &h->ztab_dev, &h->ztab_bytes, (size_t)std::max<int64_t>(E, 1) * 20));
   zd->pos = reinterpret_cast<int64_t*>(h->ztab_dev);
-  zd->bytes = zd->pos + T;
-  zd->status = reinterpret_cast<int*>(zd->bytes + T);
-  ARP_CUDA(h, cudaMemcpyAsync(zd->pos, z->pos.data(), (size_t)T * 8, cudaMemcpyHostToDevice, st));
-  ARP_CUDA(h, cudaMemcpyAsync(zd->bytes, z->bytes, (size_t)T * 8, cudaMemcpyHostToDevice, st));
+  zd->bytes = zd->pos + E;
+  zd->status = reinterpret_cast<int*>(zd->bytes + E);
+  ARP_CUDA(h, cudaMemcpyAsync(zd->pos, z.pos.data(), (size_t)E * 8, cudaMemcpyHostToDevice, st));
+  ARP_CUDA(h, cudaMemcpyAsync(zd->bytes, z.bytes.data(), (size_t)E * 8, cudaMemcpyHostToDevice, st));
   return ARP_OK;
 }
 
@@ -1776,16 +1947,22 @@ static const char* inflate_status_name(int s) {
   }
 }
 
-// ARP_ERR_INVALID naming the first row that did not inflate
-static int check_zrows(ArpHandle* h, const ZRows& z, const ZDev& zd, int64_t T, cudaStream_t st) {
-  std::vector<int> status((size_t)T);
-  ARP_CUDA(h, cudaMemcpyAsync(status.data(), zd.status, (size_t)T * 4, cudaMemcpyDeviceToHost, st));
+// ARP_ERR_INVALID naming the first chunk that did not inflate: the first row of the call it holds, its logical origin
+static int check_zrows(ArpHandle* h, const ZRows& z, const ZDev& zd, cudaStream_t st) {
+  const size_t E = z.off.size();
+  std::vector<int> status(E);
+  ARP_CUDA(h, cudaMemcpyAsync(status.data(), zd.status, E * 4, cudaMemcpyDeviceToHost, st));
   ARP_CUDA(h, cudaStreamSynchronize(st));
-  for (int64_t t = 0; t < T; ++t)
-    if (status[t] != ARP_INFLATE_OK)
-      return fail(h, ARP_ERR_INVALID, "row %lld of the call (chunk at file offset %lld, %lld bytes) does not inflate to "
-                  "%lld bytes: %s (ArpInflateStatus %d)", (long long)t, (long long)z.off[t], (long long)z.bytes[t],
-                  (long long)z.row_bytes, inflate_status_name(status[t]), status[t]);
+  char buf[160];
+  for (size_t e = 0; e < E; ++e)
+    if (status[e] != ARP_INFLATE_OK) {
+      const int64_t* o = z.origins + z.chunk[e] * z.ndim;
+      return fail(h, ARP_ERR_INVALID, "row %lld of the call: chunk %lld at logical origin %s (file offset %lld, %lld "
+                  "bytes) does not inflate to %lld bytes: %s (ArpInflateStatus %d)",
+                  (long long)std::max<int64_t>(o[0] - z.row_lo, 0), (long long)z.chunk[e], origin_str(buf, o, z.ndim),
+                  (long long)z.off[e], (long long)z.bytes[e], (long long)z.grid.vol, inflate_status_name(status[e]),
+                  status[e]);
+    }
   return ARP_OK;
 }
 
@@ -1807,6 +1984,19 @@ static int check_zargs(ArpHandle* h, int32_t fd, const int64_t* off, const int64
     if (off[t] < 0 || bytes[t] < 0)
       return fail(h, ARP_ERR_INVALID, "row %lld: negative chunk offset or size", (long long)t);
   return ARP_OK;
+}
+
+// a zfile call is the zchunks call of a dataset [T, F, H, W, 3] chunked (1, F, H, W, 3) whose chunk t is row t, without
+// the zchunks limits (its rows are at most 64 frames); `origins` holds the table's origins for as long as z is used
+static int plan_zfile(ArpHandle* h, int32_t fd, const int64_t* off, const int64_t* bytes, int64_t T, int64_t row_bytes,
+                      std::vector<int64_t>* origins, ZRows* z) {
+  ARP_TRY(check_zargs(h, fd, off, bytes, T, row_bytes));
+  const int64_t F = row_bytes / ((int64_t)h->cfg.in_h * h->cfg.in_w * 3);
+  const ArpChunkLayout L{(int32_t)sizeof(ArpChunkLayout), 5, {T, F, h->cfg.in_h, h->cfg.in_w, 3},
+                         {1, F, h->cfg.in_h, h->cfg.in_w, 3}};
+  origins->assign((size_t)T * 5, 0);
+  for (int64_t t = 0; t < T; ++t) (*origins)[(size_t)t * 5] = t;
+  return plan_zchunks(h, &L, origins->data(), off, bytes, T, 0, T, false, z);
 }
 
 // arp_embed_tower_*: the adapter head stopped after the CLIP feature; the chunk's taps and feature become n tower records
@@ -1831,7 +2021,7 @@ static int tower_chunk(ArpHandle* h, int64_t n, float* rec, cudaStream_t st) {
 static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t fd_offset, int64_t T,
                            int64_t row_stride_bytes, const int64_t* ep_offsets_host, int32_t n_eps, int32_t num_frames,
                            float* reward_host, float* rtg_host, float* reward_stacked_host, float* rtg_stacked_host,
-                           float* emb_host = nullptr, bool tower = false, ZRows* z = nullptr) {
+                           float* emb_host = nullptr, bool tower = false, const ZRows* z = nullptr) {
   if (!h) return ARP_ERR_INVALID;
   cudaStream_t st = h->own_stream;
   const bool embed = emb_host != nullptr;
@@ -1847,7 +2037,7 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
   const int F = embed ? 1 : num_frames;
   ARP_TRY(ensure_stage(h));
   ZDev zd;
-  if (z) ARP_TRY(prepare_zrows(h, z, T, B, &zd, st));
+  if (z) ARP_TRY(prepare_zrows(h, *z, &zd, st));
   // device outputs (scratch slot 1), G = n_groups:
   // [ep_off (n_eps+1) i64][reward G*T][rtg G*T][reward_stacked G*T*F][rtg_stacked G*T*F]; embed mode: [emb T*ew]
   const size_t G = (size_t)h->n_groups;
@@ -1868,16 +2058,24 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
   // pinned (or registered) caller memory goes to the device directly, one strided 2-D copy per chunk; pageable memory is
   // gathered through the pinned ring by worker threads
   const bool staged = fd >= 0 || !host_ptr_is_pinned(ob_host);
-  const size_t pitch = z ? (size_t)z->max_chunk : frame_bytes;   // pinned ring: bytes per row of a slot
+  // pinned ring: items (frames, or compressed chunks) per slot and bytes per item; large chunks get fewer per slot so
+  // that a slot stays within ZRING_SLOT_BYTES
+  const size_t pitch = z ? (size_t)z->max_chunk : frame_bytes;
+  const int sub = z ? (int)std::max<int64_t>(1, std::min<int64_t>(STG_SUB, ZRING_SLOT_BYTES / (int64_t)pitch)) : STG_SUB;
+  // the items of batch ci: rows, or the batch's ZRows entries
+  auto items = [&](int64_t ci) {
+    return z ? std::make_pair(z->batch[ci], z->batch[ci + 1]) : std::make_pair(ci * B, std::min(T, ci * B + B));
+  };
   std::vector<SubChunk> subs;
   HostStager stager;
   if (staged) {
-    ARP_TRY(ensure_pinned_ring(h, pitch));
+    ARP_TRY(ensure_pinned_ring(h, pitch * sub));
     for (int64_t ci = 0; ci < nchunks; ++ci) {
-      const int64_t t0 = ci * B, n = std::min(B, T - t0);
-      for (int64_t s0 = 0; s0 < n; s0 += STG_SUB) subs.push_back(SubChunk{t0 + s0, (int)std::min<int64_t>(STG_SUB, n - s0)});
+      const auto [i0, i1] = items(ci);
+      for (int64_t s0 = i0; s0 < i1; s0 += sub) subs.push_back(SubChunk{s0, (int)std::min<int64_t>(sub, i1 - s0)});
     }
-    stager.src = ob_host; stager.stride = row_stride_bytes; stager.frame_bytes = pitch; stager.ring = h->pin_ring;
+    stager.src = ob_host; stager.stride = row_stride_bytes; stager.frame_bytes = pitch; stager.slot_bytes = pitch * sub;
+    stager.ring = h->pin_ring;
     stager.ev_slot = h->ev_slot; stager.device = c.device; stager.subs = &subs;
     stager.fd = fd; stager.fd_base = fd_offset; stager.z = z;
     stager.start();
@@ -1894,17 +2092,18 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
       e = cudaMemcpy2DAsync(h->stage_dev[buf], frame_bytes, ob_host + t0 * row_stride_bytes, (size_t)row_stride_bytes,
                             frame_bytes, (size_t)n, cudaMemcpyHostToDevice, h->copy_stream);
     } else {
-      for (int64_t s0 = 0; s0 < n && e == cudaSuccess; s0 += STG_SUB, ++sub_j) {
+      const auto [i0, i1] = items(ci);
+      for (int64_t s0 = i0; s0 < i1 && e == cudaSuccess; s0 += sub, ++sub_j) {
         stager.wait(sub_j);
         const int slot = (int)(sub_j % STG_SLOTS);
-        const uint8_t* ring_slot = h->pin_ring + (size_t)slot * STG_SUB * pitch;
-        if (z) {   // the sub-chunk's compressed rows, packed, to their place in the chunk's packed buffer
-          const int64_t a = t0 + s0, b = a + subs[sub_j].n - 1;
+        const uint8_t* ring_slot = h->pin_ring + (size_t)slot * sub * pitch;
+        if (z) {   // the sub-chunk's compressed chunks, packed, to their place in the batch's packed buffer
+          const int64_t a = s0, b = a + subs[sub_j].n - 1;
           e = cudaMemcpyAsync(h->zsrc_dev[buf] + z->pos[a], ring_slot, (size_t)(z->pos[b] + z->bytes[b] - z->pos[a]),
                               cudaMemcpyHostToDevice, h->copy_stream);
         } else {
-          e = cudaMemcpyAsync(h->stage_dev[buf] + (size_t)s0 * frame_bytes, ring_slot, (size_t)subs[sub_j].n * frame_bytes,
-                              cudaMemcpyHostToDevice, h->copy_stream);
+          e = cudaMemcpyAsync(h->stage_dev[buf] + (size_t)(s0 - t0) * frame_bytes, ring_slot,
+                              (size_t)subs[sub_j].n * frame_bytes, cudaMemcpyHostToDevice, h->copy_stream);
         }
         if (e == cudaSuccess) e = cudaEventRecord(h->ev_slot[slot], h->copy_stream);
         stager.issued.store(sub_j + 1, std::memory_order_release);
@@ -1913,11 +2112,15 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
     if (e != cudaSuccess) { rc = fail(h, ARP_ERR_CUDA, "H2D frames failed: %s", cudaGetErrorString(e)); break; }
     cudaEventRecord(h->ev_copied[buf], h->copy_stream);
     cudaStreamWaitEvent(st, h->ev_copied[buf], 0);
-    if (z) {   // whole rows inflated into zrows_dev; the encoder reads each row's last frame with stride row_bytes
-      if ((rc = launch_inflate(h, h->zsrc_dev[buf], zd.pos + t0, zd.bytes + t0, n, z->row_bytes, h->zrows_dev,
-                               zd.status + t0, st)) != ARP_OK)
+    if (z) {   // the batch's chunks inflated into zrows_dev, one slot each
+      const int64_t e0 = z->batch[ci];
+      if ((rc = launch_inflate(h, h->zsrc_dev[buf], zd.pos + e0, zd.bytes + e0, z->batch[ci + 1] - e0, z->grid.vol,
+                               h->zrows_dev, zd.status + e0, st)) != ARP_OK)
         break;
-      rc = encode_chunk(h, h->zrows_dev + (z->row_bytes - (int64_t)frame_bytes), n, z->row_bytes, st);
+      if (z->dense)   // chunk t holds row t: the encoder reads frame F-1 of each chunk in place, stride one chunk
+        rc = encode_chunk(h, h->zrows_dev + z->grid.frame_off, n, z->grid.vol, st);
+      else if ((rc = launch_gather(h, z->grid, z->row_lo + t0, n, h->zrows_dev, h->stage_dev[buf], st)) == ARP_OK)
+        rc = encode_chunk(h, h->stage_dev[buf], n, (int64_t)frame_bytes, st);
     } else {
       rc = encode_chunk(h, h->stage_dev[buf], n, (int64_t)frame_bytes, st);
     }
@@ -1937,7 +2140,7 @@ static int label_host_impl(ArpHandle* h, const uint8_t* ob_host, int fd, int64_t
       fprintf(stderr, "arp_label_host: %lld frames staged in %zu sub-chunks, consumer waited %.3f s for the gather threads\n",
               (long long)T, subs.size(), stager.waited_s);
   }
-  if (rc == ARP_OK && z) rc = check_zrows(h, *z, zd, T, st);
+  if (rc == ARP_OK && z) rc = check_zrows(h, *z, zd, st);
   if (rc == ARP_OK && embed) {
     cudaError_t e = cudaMemcpyAsync(emb_host, d_emb, (size_t)T * ew * 4, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
@@ -2078,8 +2281,9 @@ extern "C" int arp_label_zfile(ArpHandle* h, int32_t fd, const int64_t* chunk_of
                                int64_t T, int64_t row_bytes, const int64_t* ep_offsets_host, int32_t n_eps,
                                int32_t num_frames, float* reward_host, float* rtg_host, float* reward_stacked_host,
                                float* rtg_stacked_host) {
-  ARP_TRY(check_zargs(h, fd, chunk_offset_host, chunk_bytes_host, T, row_bytes));
-  ZRows z{chunk_offset_host, chunk_bytes_host, {}, row_bytes, 0};
+  std::vector<int64_t> origins;
+  ZRows z;
+  ARP_TRY(plan_zfile(h, fd, chunk_offset_host, chunk_bytes_host, T, row_bytes, &origins, &z));
   return label_host_impl(h, nullptr, fd, 0, T, row_bytes, ep_offsets_host, n_eps, num_frames, reward_host, rtg_host,
                          reward_stacked_host, rtg_stacked_host, nullptr, false, &z);
 }
@@ -2089,7 +2293,9 @@ extern "C" int arp_embed_zfile(ArpHandle* h, int32_t fd, const int64_t* chunk_of
   ARP_TRY(check_zargs(h, fd, chunk_offset_host, chunk_bytes_host, T, row_bytes));
   if (T > 0 && !emb_host) return fail(h, ARP_ERR_INVALID, "null argument");
   if (T == 0) return check_ready(h, reinterpret_cast<const uint8_t*>(h), T, row_bytes, h->own_stream);
-  ZRows z{chunk_offset_host, chunk_bytes_host, {}, row_bytes, 0};
+  std::vector<int64_t> origins;
+  ZRows z;
+  ARP_TRY(plan_zfile(h, fd, chunk_offset_host, chunk_bytes_host, T, row_bytes, &origins, &z));
   return label_host_impl(h, nullptr, fd, 0, T, row_bytes, nullptr, 0, 0, nullptr, nullptr, nullptr, nullptr, emb_host,
                          false, &z);
 }
@@ -2100,9 +2306,67 @@ extern "C" int arp_embed_tower_zfile(ArpHandle* h, int32_t fd, const int64_t* ch
   if (T > 0 && !rec_host) return fail(h, ARP_ERR_INVALID, "null argument");
   if (!h->adapter) return fail(h, ARP_ERR_INVALID, "tower records serve the adapter heads only");
   if (T == 0) return check_ready(h, reinterpret_cast<const uint8_t*>(h), T, row_bytes, h->own_stream);
-  ZRows z{chunk_offset_host, chunk_bytes_host, {}, row_bytes, 0};
+  std::vector<int64_t> origins;
+  ZRows z;
+  ARP_TRY(plan_zfile(h, fd, chunk_offset_host, chunk_bytes_host, T, row_bytes, &origins, &z));
   return label_host_impl(h, nullptr, fd, 0, T, row_bytes, nullptr, 0, 0, nullptr, nullptr, nullptr, nullptr, rec_host,
                          true, &z);
+}
+
+// the zchunks entry points: label_host_impl reads the planned chunks; its row stride argument is one frame (only
+// check_ready sees it)
+extern "C" int arp_label_zchunks(ArpHandle* h, int32_t fd, const ArpChunkLayout* layout, const int64_t* origins_host,
+                                 const int64_t* offsets_host, const int64_t* bytes_host, int64_t n_chunks,
+                                 int64_t row_lo, int64_t T, const int64_t* ep_offsets_host, int32_t n_eps,
+                                 int32_t num_frames, float* reward_host, float* rtg_host, float* reward_stacked_host,
+                                 float* rtg_stacked_host) {
+  if (!h) return ARP_ERR_INVALID;
+  if (fd < 0) return fail(h, ARP_ERR_INVALID, "bad file descriptor");
+  ZRows z;
+  ARP_TRY(plan_zchunks(h, layout, origins_host, offsets_host, bytes_host, n_chunks, row_lo, T, true, &z));
+  return label_host_impl(h, nullptr, fd, 0, T, (int64_t)h->cfg.in_h * h->cfg.in_w * 3, ep_offsets_host, n_eps,
+                         num_frames, reward_host, rtg_host, reward_stacked_host, rtg_stacked_host, nullptr, false, &z);
+}
+
+static int embed_zchunks(ArpHandle* h, int32_t fd, const ArpChunkLayout* layout, const int64_t* origins_host,
+                         const int64_t* offsets_host, const int64_t* bytes_host, int64_t n_chunks, int64_t row_lo,
+                         int64_t T, float* out_host, bool tower) {
+  if (!h) return ARP_ERR_INVALID;
+  if (fd < 0) return fail(h, ARP_ERR_INVALID, "bad file descriptor");
+  if (T > 0 && !out_host) return fail(h, ARP_ERR_INVALID, "null argument");
+  if (tower && !h->adapter) return fail(h, ARP_ERR_INVALID, "tower records serve the adapter heads only");
+  const int64_t frame = (int64_t)h->cfg.in_h * h->cfg.in_w * 3;
+  ZRows z;
+  ARP_TRY(plan_zchunks(h, layout, origins_host, offsets_host, bytes_host, n_chunks, row_lo, T, true, &z));
+  if (T == 0) return check_ready(h, reinterpret_cast<const uint8_t*>(h), T, frame, h->own_stream);
+  return label_host_impl(h, nullptr, fd, 0, T, frame, nullptr, 0, 0, nullptr, nullptr, nullptr, nullptr, out_host, tower,
+                         &z);
+}
+
+extern "C" int arp_embed_zchunks(ArpHandle* h, int32_t fd, const ArpChunkLayout* layout, const int64_t* origins_host,
+                                 const int64_t* offsets_host, const int64_t* bytes_host, int64_t n_chunks,
+                                 int64_t row_lo, int64_t T, float* emb_host) {
+  return embed_zchunks(h, fd, layout, origins_host, offsets_host, bytes_host, n_chunks, row_lo, T, emb_host, false);
+}
+
+extern "C" int arp_embed_tower_zchunks(ArpHandle* h, int32_t fd, const ArpChunkLayout* layout,
+                                       const int64_t* origins_host, const int64_t* offsets_host,
+                                       const int64_t* bytes_host, int64_t n_chunks, int64_t row_lo, int64_t T,
+                                       float* rec_host) {
+  return embed_zchunks(h, fd, layout, origins_host, offsets_host, bytes_host, n_chunks, row_lo, T, rec_host, true);
+}
+
+extern "C" int arp_gather_frames(ArpHandle* h, const ArpChunkLayout* layout, int64_t row0, int64_t n,
+                                 const uint8_t* chunks_dev, uint8_t* out_dev, void* stream) {
+  if (!h) return ARP_ERR_INVALID;
+  ZLayout l;
+  ARP_TRY(check_chunk_layout(h, layout, &l));
+  if (n < 0 || n > 0x7fffffffLL || row0 < 0 || row0 > l.s[0] - n)
+    return fail(h, ARP_ERR_INVALID, "rows [%lld, %lld + %lld) are not inside the dataset's %lld rows", (long long)row0,
+                (long long)row0, (long long)n, (long long)l.s[0]);
+  if (n > 0 && (!chunks_dev || !out_dev)) return fail(h, ARP_ERR_INVALID, "null argument");
+  ARP_CUDA(h, cudaSetDevice(h->cfg.device));
+  return launch_gather(h, chunk_grid(l), row0, n, chunks_dev, out_dev, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int arp_inflate_rows(ArpHandle* h, const uint8_t* src_dev, const int64_t* src_off_dev,

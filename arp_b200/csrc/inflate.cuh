@@ -12,6 +12,9 @@
 // memory (3.6 KB per warp): puff-style canonical count / symbol arrays plus a FAST_BITS-bit direct lookup; codes longer
 // than FAST_BITS take the canonical walk.
 //
+// Other chunk shapes (arp_*_zchunks): each stream is one HDF5 chunk inflated to the chunk volume, and
+// gather_frames_kernel copies the scored frame of each row out of its batch's chunks into dense [n, H, W, 3] frames.
+//
 // Malformed input never faults: every source read is checked against the row's src_bytes, every back-reference against
 // the output position and every write against row_bytes. The first violation stops the row and sets status[row] to an
 // ArpInflateStatus; no check traps.
@@ -273,6 +276,44 @@ inflate_rows_kernel(const uint8_t* __restrict__ src, const int64_t* __restrict__
                                    : inflate_stream(src + off, nb, out + static_cast<int64_t>(row) * row_bytes, row_bytes,
                                                     smem[w], lane);
   if (lane == 0) status[row] = st;
+}
+
+// Where the scored frame of each row lies in a batch's inflated chunks. A batch needs the row-chunks rc0 .. of its rows,
+// and of each every (H, W, channel) chunk at the F-chunk holding frame F-1; they are inflated in the order (row-chunk,
+// H-chunk, W-chunk, channel-chunk), so a chunk's scratch slot follows from its grid indices and no table is needed.
+struct ChunkGrid {
+  int64_t row0;        // dataset row of output frame 0
+  int64_t rc0;         // first row-chunk of the batch
+  int64_t vol;         // bytes of one inflated chunk
+  int64_t row_pitch;   // bytes of one row inside a chunk: cF * cH * cW * cC
+  int64_t frame_off;   // offset of frame F-1 inside a chunk row: ((F - 1) % cF) * cH * cW * cC
+  int cT, cH, cW, cC;  // chunk extents
+  int nH, nW, nC;      // chunks along H, W and the channels
+  int H, W;
+};
+
+// out[i, y, x, c] = frame F-1 of dataset row g.row0 + i: one thread per output pixel (consecutive threads read
+// consecutive pixels of one chunk row), grid-stride over n * H * W pixels
+__global__ void __launch_bounds__(256)
+gather_frames_kernel(const uint8_t* __restrict__ chunks, ChunkGrid g, int n, uint8_t* __restrict__ out) {
+  const int64_t npix = static_cast<int64_t>(n) * g.H * g.W;
+  for (int64_t p = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; p < npix;
+       p += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+    const int x = static_cast<int>(p % g.W);
+    const int64_t iy = p / g.W;
+    const int y = static_cast<int>(iy % g.H);
+    const int64_t row = g.row0 + iy / g.H;
+    const int64_t rc = row / g.cT - g.rc0;
+    const int hi = y / g.cH, wi = x / g.cW;
+    const int64_t base = row % g.cT * g.row_pitch + g.frame_off +
+                         (static_cast<int64_t>(y - hi * g.cH) * g.cW + (x - wi * g.cW)) * g.cC;
+    const int64_t slot0 = ((rc * g.nH + hi) * g.nW + wi) * g.nC;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      const int ci = c / g.cC;
+      out[p * 3 + c] = __ldg(chunks + (slot0 + ci) * g.vol + base + (c - ci * g.cC));
+    }
+  }
 }
 
 }  // namespace arp_inflate

@@ -46,6 +46,7 @@ from __future__ import annotations
 
 import argparse
 import hashlib
+import itertools
 import json
 import os
 
@@ -287,7 +288,7 @@ class RewardLabeler:
             assert model_ckpt_dir is not None, "specify model_ckpt_dir"  # label_reward.py:174
         if device is None:
             device = int(os.environ.get("LOCAL_RANK", "0"))
-        self.model_type, self.device_index = model_type, device
+        self.model_type, self.device_index, self.max_batch = model_type, device, int(max_batch)
         patch = 32 if arch.endswith("/32") else 16
         self.engine = _cached_engine(device=device, patch=patch, in_h=int(frame_hw[0]), in_w=int(frame_hw[1]),
                                      use_crop=bool(use_crop), preprocess=pre, head=head,
@@ -382,6 +383,22 @@ class RewardLabeler:
     def embed_tower_zfile(self, fd: int, chunk_offsets: np.ndarray, chunk_bytes: np.ndarray, row_bytes: int) -> np.ndarray:
         """The frozen-CLIP side of label_zfile."""
         return self.engine.embed_tower_zfile(fd, chunk_offsets, chunk_bytes, row_bytes)
+
+    def label_zchunks(self, fd: int, layout, origins: np.ndarray, offsets: np.ndarray, sizes: np.ndarray, row_lo: int,
+                      T: int, ep_offsets: np.ndarray, num_frames: int):
+        """label_file's outputs for dataset rows [row_lo, row_lo + T) of a gzip dataset in chunks of any shape
+        (_zchunk_table gives layout, origins, offsets and sizes); ep_offsets relative to row_lo."""
+        return self.engine.label_zchunks(fd, layout, origins, offsets, sizes, row_lo, T, ep_offsets, num_frames)
+
+    def embed_zchunks(self, fd: int, layout, origins: np.ndarray, offsets: np.ndarray, sizes: np.ndarray, row_lo: int,
+                      T: int) -> np.ndarray:
+        """The image side of label_zchunks."""
+        return self.engine.embed_zchunks(fd, layout, origins, offsets, sizes, row_lo, T)
+
+    def embed_tower_zchunks(self, fd: int, layout, origins: np.ndarray, offsets: np.ndarray, sizes: np.ndarray,
+                            row_lo: int, T: int) -> np.ndarray:
+        """The frozen-CLIP side of label_zchunks."""
+        return self.engine.embed_tower_zchunks(fd, layout, origins, offsets, sizes, row_lo, T)
 
     def label_tower(self, rec: np.ndarray, ep_offsets: np.ndarray, num_frames: int):
         """label_slab's outputs (host arrays) from the CLIP tower records [T, tower_dim] of the same rows, with this
@@ -692,6 +709,56 @@ def _zfile_rows(ds):
     return ds.file.filename, offsets, sizes, int(np.prod(shape[1:]))
 
 
+def _zchunk_table(ds, lo: int = 0, hi: "int | None" = None, max_batch: int = 1):
+    """(path, layout, origins [n, ndim], file offsets [n], sizes [n]) of the chunks holding the scored frames (frame F-1)
+    of rows [lo, hi) of the image dataset `ds`, layout = (shape, chunks), when the library can read them itself, else
+    None: an h5py dataset of uint8 [T, F, H, W, 3] or [T, H, W, 3] chunked in any shape, gzip and optionally shuffle
+    (on 1-byte elements shuffle regroups each element's bytes by position, and a 1-byte element has one position, so the
+    stored bytes are the deflate stream's) and no other filter, every needed chunk allocated, written with
+    filter_mask 0 and at most ZCHUNK_MAX_COMPRESSED_BYTES compressed, and the inflated chunks of one max_batch batch
+    within the library's device-scratch bound. Only the needed chunks are looked up."""
+    dsid = getattr(ds, "id", None)
+    if dsid is None or not hasattr(dsid, "get_chunk_info_by_coord") or getattr(getattr(ds, "file", None), "filename",
+                                                                                None) is None:
+        return None
+    shape, chunks = tuple(ds.shape), tuple(ds.chunks or ())
+    if len(shape) not in (4, 5) or np.dtype(ds.dtype) != np.uint8 or len(chunks) != len(shape) or shape[-1] != 3:
+        return None
+    if ds.compression != "gzip" or ds.fletcher32 or getattr(ds, "scaleoffset", None) is not None:
+        return None
+    plist = getattr(dsid, "get_create_plist", None)
+    if plist is not None and plist().get_nfilters() != 1 + bool(ds.shuffle):   # a filter h5py has no property for
+        return None
+    hi = shape[0] if hi is None else hi
+    if not 0 <= lo < hi <= shape[0]:
+        return None
+    c5 = chunks if len(shape) == 5 else (chunks[0], 1) + chunks[1:]
+    s5 = shape if len(shape) == 5 else (shape[0], 1) + shape[1:]
+    fc = (s5[1] - 1) // c5[1]                                      # F-chunk of the scored frame
+    rc_lo, rc_hi = lo // c5[0], (hi - 1) // c5[0]
+    nsp = int(np.prod([-(-s // c) for s, c in zip(s5[2:], c5[2:])]))
+    # a batch of max_batch rows touches at most ceil((max_batch - 1) / cT) + 1 row-chunks
+    batch_chunks = min(rc_hi - rc_lo + 1, -(-(max_batch - 1) // c5[0]) + 1) * nsp
+    if batch_chunks * int(np.prod(chunks)) > capi.ZCHUNK_SCRATCH_BYTES or (rc_hi - rc_lo + 1) * nsp > 1 << 26:
+        return None                                                # over the scratch bound, or tiny chunks
+    # only the needed chunks are looked up (DatasetID.get_chunk_info_by_coord), so the cost follows what is read, not
+    # the dataset's chunk count
+    f_origin = () if len(shape) == 4 else (fc * c5[1],)
+    spatial = list(itertools.product(*[range(0, s, c) for s, c in zip(s5[2:], c5[2:])]))
+    origins, offsets, sizes = [], [], []
+    for rc in range(rc_lo, rc_hi + 1):
+        for sp in spatial:
+            o = (rc * c5[0],) + f_origin + sp
+            info = dsid.get_chunk_info_by_coord(o)
+            if info.filter_mask != 0 or info.byte_offset is None or info.size > capi.ZCHUNK_MAX_COMPRESSED_BYTES:
+                return None                                        # filtered otherwise, unallocated, or too large
+            origins.append(o)
+            offsets.append(int(info.byte_offset))
+            sizes.append(int(info.size))
+    return (ds.file.filename, (shape, chunks), np.array(origins, np.int64).reshape(-1, len(shape)),
+            np.array(offsets, np.int64), np.array(sizes, np.int64))
+
+
 def _read_slabs(ds, side, off, e_lo: int, e_hi: int, slab_frames: int):
     """(a, b, rows) of every non-empty slab of whole episodes [a, b), read on a thread one slab ahead of the consumer"""
     import threading
@@ -724,8 +791,8 @@ def _label_rows(labeler, ds, side, off, e_lo: int, e_hi: int, num_frames: int, s
     """[reward_stacked, rtg_stacked] of each of the n_groups instruction sets in turn (2 * n_groups arrays [rows, F]) for
     episodes [e_lo, e_hi). A memory-mapped container is handed to the library in ONE call (a strided pointer into the file
     mapping; the native stager overlaps page-cache reads, PCIe and compute). An h5py gzip dataset chunked one row per
-    chunk (_zfile_rows) is handed over as its chunk table: the library reads the compressed rows and inflates them on the
-    device. Any other container that has to be read through its API is read slab by slab on a reader thread, one slab
+    chunk (_zfile_rows), or in chunks of another shape (_zchunk_table), is handed over as its chunk table: the library
+    reads the compressed chunks and inflates them on the device. Any other container that has to be read through its API is read slab by slab on a reader thread, one slab
     ahead of the GPU."""
     lo_all, hi_all = int(off[e_lo]), int(off[e_hi])
     if hi_all <= lo_all:
@@ -740,6 +807,18 @@ def _label_rows(labeler, ds, side, off, e_lo: int, e_hi: int, num_frames: int, s
         try:
             r, _, rs, gs = labeler.label_zfile(fd, offsets[lo_all:hi_all], sizes[lo_all:hi_all], row_bytes, rel,
                                                num_frames)
+        finally:
+            os.close(fd)
+        return _pairs(*_finish(labeler, r, rs, gs, rel, num_frames))
+    zch = (_zchunk_table(ds, lo_all, hi_all, getattr(labeler, "max_batch", 1))
+           if side is None and hasattr(labeler, "label_zchunks") else None)
+    if zch is not None:
+        # gzip chunks of another shape: the library preads the chunks holding this shard's scored frames and inflates them
+        path, layout, origins, offsets, sizes = zch
+        fd = os.open(path, os.O_RDONLY)
+        try:
+            r, _, rs, gs = labeler.label_zchunks(fd, layout, origins, offsets, sizes, lo_all, hi_all - lo_all, rel,
+                                                 num_frames)
         finally:
             os.close(fd)
         return _pairs(*_finish(labeler, r, rs, gs, rel, num_frames))
@@ -786,6 +865,16 @@ def _embed_rows(labeler, ds, side, off, e_lo: int, e_hi: int, slab_frames: int, 
         fd = os.open(path, os.O_RDONLY)
         try:
             return getattr(labeler, embed_zfile)(fd, offsets[lo_all:hi_all], sizes[lo_all:hi_all], row_bytes)
+        finally:
+            os.close(fd)
+    embed_zchunks = "embed_tower_zchunks" if tower else "embed_zchunks"
+    zch = (_zchunk_table(ds, lo_all, hi_all, getattr(labeler, "max_batch", 1))
+           if side is None and hasattr(labeler, embed_zchunks) else None)
+    if zch is not None:
+        path, layout, origins, offsets, sizes = zch
+        fd = os.open(path, os.O_RDONLY)
+        try:
+            return getattr(labeler, embed_zchunks)(fd, layout, origins, offsets, sizes, lo_all, hi_all - lo_all)
         finally:
             os.close(fd)
     frows = _file_rows(labeler, src, embed_file, lo_all)

@@ -37,6 +37,13 @@
  * take the file offset and size of every row's chunk (h5py: DatasetID.get_chunk_info), pread() the compressed bytes and
  * inflate them on the device (one warp per row, Adler-32 checked) before the unchanged encoder pass. No HDF5 parsing
  * happens here: the caller's chunk index says where the streams are.
+ *
+ * Compressed chunks of any shape: a gzip dataset that was re-chunked (h5py's own chunk guess, several rows per chunk,
+ * frames split along F, H, W or the channels) is one zlib stream per chunk, each inflating to the full chunk volume,
+ * edge chunks included. arp_label_zchunks / arp_embed_zchunks / arp_embed_tower_zchunks take the dataset's
+ * ArpChunkLayout and its chunk table (logical origin, file offset, size), read and inflate only the chunks that hold a
+ * scored frame, and gather the scored frames into dense [n, H, W, 3] frames on the device (gather_frames_kernel)
+ * before the unchanged encoder pass. The arp_*_zfile calls are the (1, F, H, W, 3) case of the same code.
  */
 #ifndef ARP_B200_H_
 #define ARP_B200_H_
@@ -47,7 +54,7 @@
 extern "C" {
 #endif
 
-#define ARP_B200_ABI_VERSION 9   /* 3: + arp_encode_taps_chw, 4: + arp_operand_dtype, 5: + ARP_PREC_F32RESID, arp_ln_gemm, arp_resid_gemm_stats, arp_label_file, arp_wants_weight, 6: + arp_set_text_groups, arp_text_groups, 7: + arp_embedding_dim, arp_embed_host, arp_embed_file, arp_label_embeddings, 8: + arp_tower_dim, arp_embed_tower_host, arp_embed_tower_file, arp_label_tower, 9: + ArpInflateStatus, arp_inflate_rows, arp_label_zfile, arp_embed_zfile, arp_embed_tower_zfile */
+#define ARP_B200_ABI_VERSION 10  /* 3: + arp_encode_taps_chw, 4: + arp_operand_dtype, 5: + ARP_PREC_F32RESID, arp_ln_gemm, arp_resid_gemm_stats, arp_label_file, arp_wants_weight, 6: + arp_set_text_groups, arp_text_groups, 7: + arp_embedding_dim, arp_embed_host, arp_embed_file, arp_label_embeddings, 8: + arp_tower_dim, arp_embed_tower_host, arp_embed_tower_file, arp_label_tower, 9: + ArpInflateStatus, arp_inflate_rows, arp_label_zfile, arp_embed_zfile, arp_embed_tower_zfile, 10: + ArpChunkLayout, arp_label_zchunks, arp_embed_zchunks, arp_embed_tower_zchunks, arp_gather_frames */
 
 #define ARP_MAX_TEXT 16          /* texts of one instruction set (arp_set_text's n_text, one group's size) */
 #define ARP_MAX_TEXT_GROUPS 16   /* instruction sets of one arp_set_text_groups call */
@@ -280,6 +287,57 @@ ARP_API int arp_embed_tower_zfile(ArpHandle* h, int32_t fd, const int64_t* chunk
 ARP_API int arp_inflate_rows(ArpHandle* h, const uint8_t* src_dev, const int64_t* src_off_dev,
                              const int64_t* src_bytes_dev, int64_t n, int64_t row_bytes, uint8_t* out_dev,
                              int32_t* status_dev, void* stream);
+
+/* Compressed chunks of any shape. A uint8 dataset [T, F, H, W, 3] (ndim 5) or [T, H, W, 3] (ndim 4, read as F = 1) with
+ * H, W = in_h, in_w is stored as chunks of shape `chunk` (every extent >= 1; HDF5 compresses an edge chunk at the full
+ * chunk size, including the part past the dataset's extent, so every chunk inflates to exactly
+ * prod(chunk) bytes). */
+typedef struct ArpChunkLayout {
+  int32_t struct_size;   /* sizeof(ArpChunkLayout) */
+  int32_t ndim;          /* 4 or 5 */
+  int64_t shape[5];      /* dataset shape (first ndim entries) */
+  int64_t chunk[5];      /* chunk shape (first ndim entries) */
+} ArpChunkLayout;
+
+/* Maximum device scratch for the inflated chunks of one max_batch batch (and so for one chunk). */
+#define ARP_ZCHUNK_SCRATCH_BYTES (4LL << 30)
+/* Maximum compressed size of one needed chunk: one pinned staging slot, so the pinned ring (8 slots) stays within
+ * 512 MiB. */
+#define ARP_ZCHUNK_MAX_COMPRESSED_BYTES (64LL << 20)
+
+/* Scores dataset rows [row_lo, row_lo + T), frame F-1 of each (the call's row t is dataset row row_lo + t). Chunk i of
+ * the table has logical origin origins_host[i * ndim .. + ndim) (h5py: StoreInfo.chunk_offset) and is one zlib stream of
+ * bytes_host[i] bytes at offsets_host[i] of `fd`. Only the chunks holding a scored frame are read: the row-chunks that
+ * cover the call's rows, at the F-chunk of frame F-1, all H, W and channel chunks. The table may hold more (the whole
+ * dataset's, or only a shard's part); the others are never read. Per max_batch batch the gather threads pread() the
+ * batch's needed chunks into the pinned ring, they cross PCIe compressed, inflate_rows_kernel inflates each to its chunk
+ * volume (one warp per chunk), and gather_frames_kernel copies each row's scored frame into a dense [n, H, W, 3] buffer
+ * for the encoder. When every chunk is (1, cF, H, W, 3) the scored frames already sit at a fixed stride and the gather
+ * is skipped. A row-chunk that straddles a batch boundary (or row_lo) is read and inflated once per batch it serves.
+ * ep_offsets_host are relative to row_lo (0 .. T) and the outputs are those of arp_label_zfile, bit for bit what
+ * arp_label_file gives on the same rows uncompressed. ARP_ERR_INVALID, with nothing written and the handle usable, for
+ * a bad layout (ndim, H, W, 3 channels, a chunk extent < 1), rows outside the dataset, null tables, a negative offset or
+ * size, an origin that is not a multiple of the chunk shape or lies outside the dataset, a duplicated origin, a needed
+ * chunk missing from the table, one batch's inflated chunks needing more than ARP_ZCHUNK_SCRATCH_BYTES, more than 2^26
+ * needed chunks, a needed chunk of more than ARP_ZCHUNK_MAX_COMPRESSED_BYTES compressed, and a needed
+ * chunk that does not inflate to its chunk volume: arp_last_error names the chunk's logical origin (and
+ * ArpInflateStatus). Synchronises. */
+ARP_API int arp_label_zchunks(ArpHandle* h, int32_t fd, const ArpChunkLayout* layout, const int64_t* origins_host,
+                              const int64_t* offsets_host, const int64_t* bytes_host, int64_t n_chunks, int64_t row_lo,
+                              int64_t T, const int64_t* ep_offsets_host, int32_t n_eps, int32_t num_frames,
+                              float* reward_host, float* rtg_host, float* reward_stacked_host, float* rtg_stacked_host);
+ARP_API int arp_embed_zchunks(ArpHandle* h, int32_t fd, const ArpChunkLayout* layout, const int64_t* origins_host,
+                              const int64_t* offsets_host, const int64_t* bytes_host, int64_t n_chunks, int64_t row_lo,
+                              int64_t T, float* emb_host);
+ARP_API int arp_embed_tower_zchunks(ArpHandle* h, int32_t fd, const ArpChunkLayout* layout,
+                                    const int64_t* origins_host, const int64_t* offsets_host, const int64_t* bytes_host,
+                                    int64_t n_chunks, int64_t row_lo, int64_t T, float* rec_host);
+/* The gather kernel alone, on DEVICE buffers: chunks_dev holds, for the row-chunks row0 / chunk[0] ..
+ * (row0 + n - 1) / chunk[0], every (H, W, channel) chunk at the F-chunk of frame F-1, in the order (row-chunk, H-chunk,
+ * W-chunk, channel-chunk), each inflated to prod(chunk) bytes. out_dev[n, H, W, 3] receives frame F-1 of dataset rows
+ * [row0, row0 + n). Stream-ordered, does not synchronise; ARP_ERR_INVALID for bad arguments or layout. */
+ARP_API int arp_gather_frames(ArpHandle* h, const ArpChunkLayout* layout, int64_t row0, int64_t n,
+                              const uint8_t* chunks_dev, uint8_t* out_dev, void* stream);
 /* arp_label's outputs ([G,T] / [G,T,F] with text groups, the goal-conditioned adapter head included) from tower records:
  * rec_dev [T, arp_tower_dim] fp32 DEVICE rows (16-byte aligned) from arp_embed_tower_* of a handle with the same CLIP
  * weights, arch, frame size, crop and precision; the other arguments and the four outputs are those of arp_label. Needs
