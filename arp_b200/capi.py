@@ -43,7 +43,7 @@ EXPORTS = (
     "arp_set_text_groups", "arp_text_groups", "arp_embedding_dim", "arp_embed_host", "arp_embed_file",
     "arp_label_embeddings", "arp_tower_dim", "arp_embed_tower_host", "arp_embed_tower_file", "arp_label_tower",
     "arp_label_zfile", "arp_embed_zfile", "arp_embed_tower_zfile", "arp_inflate_rows",
-    "arp_label_zchunks", "arp_embed_zchunks", "arp_embed_tower_zchunks", "arp_gather_frames",
+    "arp_label_zchunks", "arp_embed_zchunks", "arp_embed_tower_zchunks", "arp_gather_frames", "arp_cls_attention",
 )
 PROFILE_CLASSES = ("gemm", "attention", "layernorm", "decode", "head", "scan", "other")
 
@@ -153,6 +153,7 @@ def load_library() -> C.CDLL:
     lib.arp_resid_gemm_stats.argtypes = [vp, vp, vp, vp, vp, vp, i64, i32, i32, vp]
     lib.arp_layernorm_bf16.argtypes = [vp, vp, vp, vp, vp, i64, vp]
     lib.arp_attention.argtypes = [vp, vp, vp, i32, i32, vp]
+    lib.arp_cls_attention.argtypes = [vp, vp, vp, vp, i32, i32, vp]
     lib.arp_launch_count.argtypes = [vp]
     lib.arp_launch_count.restype = i64
     lib.arp_profile_begin.argtypes = [vp]
@@ -726,4 +727,14 @@ class Engine:
         qkv = qkv.to(operand_dtype()).contiguous()
         out = torch.empty(B * tokens, qkv.shape[-1] // 3, device=self.device, dtype=qkv.dtype)
         self._check(self._lib.arp_attention(self._h, _ptr(qkv), _ptr(out), B, tokens, _stream_ptr(self.device)))
+        return out
+
+    def cls_attention(self, q: torch.Tensor, qkv: torch.Tensor, B: int, tokens: int) -> torch.Tensor:
+        """Test hook: the last block's class-token attention. q [B, W] (one query row per frame), qkv [B*tokens, 3W]
+        (K and V of every token; the Q third is not read) -> [B, W], all in the operand format."""
+        assert q.dtype in (torch.bfloat16, torch.float16) and qkv.dtype in (torch.bfloat16, torch.float16)
+        q, qkv = q.to(operand_dtype()).contiguous(), qkv.to(operand_dtype()).contiguous()
+        out = torch.empty(B, qkv.shape[-1] // 3, device=self.device, dtype=qkv.dtype)
+        self._check(self._lib.arp_cls_attention(self._h, _ptr(q), _ptr(qkv), _ptr(out), B, tokens,
+                                                _stream_ptr(self.device)))
         return out

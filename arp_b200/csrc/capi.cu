@@ -1079,6 +1079,26 @@ static int launch_attention(ArpHandle* h, const bf16* qkv, bf16* out, int B, int
   return ARP_OK;
 }
 
+// Class-token attention of the pruned last block: q [B, W] (the class-token rows' Q), K / V of every token in qkv
+// [B*tokens, 3W] (the Q third is not read) -> out [B, W]
+static int launch_cls_attention(ArpHandle* h, const bf16* q, const bf16* qkv, bf16* out, int64_t B, int tokens,
+                                cudaStream_t st) {
+  if (B <= 0) return ARP_OK;
+  const int W = h->cfg.width;
+  ProfScope prof(h, PC_ATTENTION, 4.0 * (double)B * h->cfg.heads * tokens * 64,
+                 (double)B * tokens * W * 2 * 2 + (double)B * W * 2 * 2, st);
+  const unsigned blocks = (unsigned)((B * h->cfg.heads + 7) / 8);
+  if (tokens == 197)
+    cls_attention_kernel<197><<<blocks, 256, 0, st>>>(q, qkv, out, (int)B, h->cfg.heads, W, 0.125f);
+  else if (tokens == 50)
+    cls_attention_kernel<50><<<blocks, 256, 0, st>>>(q, qkv, out, (int)B, h->cfg.heads, W, 0.125f);
+  else
+    return fail(h, ARP_ERR_INVALID, "attention is built for 197 or 50 tokens, got %d", tokens);
+  h->launches++;
+  ARP_CUDA(h, cudaGetLastError());
+  return ARP_OK;
+}
+
 // ------------------------------------------------------------------------------------------------
 // the encoder: n frames (n <= max_batch) -> residual stream x after the last block (+ CLS taps)
 // ------------------------------------------------------------------------------------------------
@@ -1100,18 +1120,7 @@ static int last_block_cls(ArpHandle* h, const LayerW& L, const XT* x, int64_t n,
   h->launches++;
   ARP_TRY(launch_ln_bf16(h, ws.xcls, L.ln1_g, L.ln1_b, ws.xncls, n, st));
   ARP_TRY(launch_gemm(h, ws.xncls, B, L.w_qkv, ws.qcls, false, ACT_NONE, n, W, W, W, L.b_qkv, nullptr, 0, nullptr, 0, st));
-  {
-    ProfScope prof(h, PC_ATTENTION, 4.0 * (double)n * c.heads * h->tokens * 64,
-                   (double)n * h->tokens * W * 2 * 2 + (double)n * W * 2 * 2, st);
-    const unsigned blocks = (unsigned)((n * c.heads + 7) / 8);
-    if (h->tokens == 197)
-      cls_attention_kernel<197><<<blocks, 256, 0, st>>>(ws.qcls, ws.qkv, ws.acls, (int)n, c.heads, W, 0.125f);
-    else if (h->tokens == 50)
-      cls_attention_kernel<50><<<blocks, 256, 0, st>>>(ws.qcls, ws.qkv, ws.acls, (int)n, c.heads, W, 0.125f);
-    else
-      return fail(h, ARP_ERR_INVALID, "attention is built for 197 or 50 tokens, got %d", h->tokens);
-    h->launches++;
-  }
+  ARP_TRY(launch_cls_attention(h, ws.qcls, ws.qkv, ws.acls, n, h->tokens, st));
   ARP_TRY(launch_gemm(h, ws.acls, B, L.w_out, ws.xcls, true, ACT_NONE, n, W, W, W, L.b_out, ws.xcls, W, nullptr, 0, st));
   ARP_TRY(launch_ln_bf16(h, ws.xcls, L.ln2_g, L.ln2_b, ws.xncls, n, st));
   ARP_TRY(launch_gemm(h, ws.xncls, B, L.w_fc, ws.hcls, false, ACT_QUICKGELU, n, 4 * W, W, 4 * W, L.b_fc, nullptr, 0,
@@ -2670,6 +2679,15 @@ extern "C" int arp_attention(ArpHandle* h, const void* qkv_dev, void* out_dev, i
   ARP_CUDA(h, cudaSetDevice(h->cfg.device));
   return launch_attention(h, static_cast<const bf16*>(qkv_dev), static_cast<bf16*>(out_dev), B, tokens,
                           static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int arp_cls_attention(ArpHandle* h, const void* q_dev, const void* qkv_dev, void* out_dev, int32_t B,
+                                 int32_t tokens, void* stream) {
+  if (!h || !q_dev || !qkv_dev || !out_dev) return fail(h, ARP_ERR_INVALID, "null argument");
+  if (tokens != 197 && tokens != 50) return fail(h, ARP_ERR_INVALID, "attention is built for 197 or 50 tokens, got %d", tokens);
+  ARP_CUDA(h, cudaSetDevice(h->cfg.device));
+  return launch_cls_attention(h, static_cast<const bf16*>(q_dev), static_cast<const bf16*>(qkv_dev),
+                              static_cast<bf16*>(out_dev), B, tokens, static_cast<cudaStream_t>(stream));
 }
 
 #ifdef ARP_ATTN_TRACE

@@ -54,7 +54,7 @@
 extern "C" {
 #endif
 
-#define ARP_B200_ABI_VERSION 10  /* 3: + arp_encode_taps_chw, 4: + arp_operand_dtype, 5: + ARP_PREC_F32RESID, arp_ln_gemm, arp_resid_gemm_stats, arp_label_file, arp_wants_weight, 6: + arp_set_text_groups, arp_text_groups, 7: + arp_embedding_dim, arp_embed_host, arp_embed_file, arp_label_embeddings, 8: + arp_tower_dim, arp_embed_tower_host, arp_embed_tower_file, arp_label_tower, 9: + ArpInflateStatus, arp_inflate_rows, arp_label_zfile, arp_embed_zfile, arp_embed_tower_zfile, 10: + ArpChunkLayout, arp_label_zchunks, arp_embed_zchunks, arp_embed_tower_zchunks, arp_gather_frames */
+#define ARP_B200_ABI_VERSION 11  /* 3: + arp_encode_taps_chw, 4: + arp_operand_dtype, 5: + ARP_PREC_F32RESID, arp_ln_gemm, arp_resid_gemm_stats, arp_label_file, arp_wants_weight, 6: + arp_set_text_groups, arp_text_groups, 7: + arp_embedding_dim, arp_embed_host, arp_embed_file, arp_label_embeddings, 8: + arp_tower_dim, arp_embed_tower_host, arp_embed_tower_file, arp_label_tower, 9: + ArpInflateStatus, arp_inflate_rows, arp_label_zfile, arp_embed_zfile, arp_embed_tower_zfile, 10: + ArpChunkLayout, arp_label_zchunks, arp_embed_zchunks, arp_embed_tower_zchunks, arp_gather_frames, 11: + arp_cls_attention */
 
 #define ARP_MAX_TEXT 16          /* texts of one instruction set (arp_set_text's n_text, one group's size) */
 #define ARP_MAX_TEXT_GROUPS 16   /* instruction sets of one arp_set_text_groups call */
@@ -433,6 +433,11 @@ ARP_API int arp_layernorm_bf16(ArpHandle* h, const float* x_dev, const float* ga
                        int64_t M, void* stream);
 /* softmax(QK^T/8)V for qkv bf16 [B*tokens, 3*width] -> bf16 [B*tokens, width]; tokens = 197 or 50 */
 ARP_API int arp_attention(ArpHandle* h, const void* qkv_dev, void* out_dev, int32_t B, int32_t tokens, void* stream);
+/* the pruned last block's class-token attention: softmax(q K^T/8) V of ONE query row per (frame, head), q [B, width]
+ * (head h at columns 64h), K and V of the frame's tokens in qkv [B*tokens, 3*width] as arp_attention takes it (the Q
+ * third is not read) -> out [B, width]; operand format throughout, tokens = 197 or 50. Test seam. */
+ARP_API int arp_cls_attention(ArpHandle* h, const void* q_dev, const void* qkv_dev, void* out_dev, int32_t B,
+                              int32_t tokens, void* stream);
 
 /* counters: kernels launched by this handle since creation (bench.py's gpu_launches) */
 ARP_API int64_t arp_launch_count(const ArpHandle* h);
